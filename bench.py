@@ -9,6 +9,7 @@ Workload = BASELINE.json configs[1]: ResNet-50 VOC, 8 images x 2000 mask proposa
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          one JSON line on rank 0
     python bench.py --impl reference ...                          the CPU restatement, host cores
+    python bench.py --dump-outputs DIR ...                        + the last timed step's results as DIR/<name>.npy
 
 Weak scaling: every rank owns its own 8 images (the path shards per image, no data-path
 collective; SURVEY.md section 8e).  Timing: CUDA events on the launching stream, barrier +
@@ -374,6 +375,32 @@ def timed(fn, steps, warmup, dev, cdist=None, finish=None):
     return cdist.max_over_ranks(e0.elapsed_time(e1) / steps, dev)
 
 
+#: the results CIMHeadStep.run leaves for its caller (see its docstring); the second group with head_grads=True
+STEP_OUTPUTS = ("roi_out", "grad_feat", "iou", "asy", "scores", "pseudo_labels", "pseudo_iou", "loss_weights", "valid")
+STEP_OUTPUTS_HEAD_GRADS = ("losses", "pcl_loss", "grad_scores", "grad_seg_x", "grad_weight", "grad_bias")
+DUMP_ELEMS = 1 << 19
+
+
+def dump_outputs(step, out_dir):
+    """Write the results of the last step run on `step` to out_dir/<name>.npy as float32 (the float16 and uint8 ones
+    convert exactly).  An array of more than DUMP_ELEMS elements is written as the DUMP_ELEMS elements at flat indices
+    drawn from a fixed seed and sorted: the same indices in every run, so that two builds can be compared output for
+    output.  At most 15 x 2 MiB in all."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name in STEP_OUTPUTS + (STEP_OUTPUTS_HEAD_GRADS if step.head_grads else ()):
+        t = getattr(step, name).reshape(-1)
+        if t.numel() > DUMP_ELEMS:
+            t = t[torch.from_numpy(dump_indices(t.numel())).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
+def dump_indices(n):
+    """The sorted flat indices dump_outputs writes of an array of n > DUMP_ELEMS elements."""
+    # a generator of its own: numpy's global one drives the step's anti-noise sampling
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_ELEMS, replace=False))
+
+
 SAMPLING_NOTE = {
     "stream": "anti-noise sampling without a host hop: the device reads numpy's random stream from a ring the host "
               "fills ahead of time (cim_anti_noise_stream), pseudo-GT counts are read back with a lag, np.random is "
@@ -424,6 +451,8 @@ def measure_training(name, cfg, args, dev, rank, world, peaks, cdist, headline):
         sampler.start()
     ms_graph = timed(lambda: run("graph"), steps, warmup, dev, cdist, finish=step.sync_rng)
     clocks = sampler.stop() if headline and rank == 0 else None
+    if headline and rank == 0 and args.dump_outputs:
+        dump_outputs(step, args.dump_outputs)          # before the runs below overwrite the step's buffers
     ms_hop = None
     if args.sampling == "stream" and not args.no_anti_noise:
         step.rng = "hop"                       # same step, same buffers, the host hop instead of the device ring
@@ -635,7 +664,9 @@ def measure_inference(name, cfg, args, dev, rank, world, peaks, cdist):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline workload; the --also workloads time between 3 and 10 of "
+                         "them, --impl reference at most 3")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="cfg2_r50_voc_8x2000", choices=sorted(WORKLOADS))
@@ -653,7 +684,15 @@ def main():
     ap.add_argument("--no-anti-noise", action="store_true")
     ap.add_argument("--no-head-grads", action="store_true",
                     help="leave the loss block, the scoring backward and the allreduce of the head gradients out of the step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps of the headline workload, write what its last timed step computed (rank "
+                         f"0) as DIR/<name>.npy in float32; arrays of more than {DUMP_ELEMS} elements as a fixed, seeded "
+                         "sample of that many")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the GPU path")
     # stdout carries exactly ONE line, the JSON result: everything else a library may write to fd 1 (NCCL prints its
     # version banner there on the first collective) goes to stderr
     sys.stdout.flush()

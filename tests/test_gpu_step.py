@@ -300,3 +300,26 @@ def test_run_host_with_crops_and_changing_inputs(depth):
         np.testing.assert_array_equal(got["valid"], w_valid)
         np.testing.assert_array_equal(np.nan_to_num(got["losses"], nan=-7.0), np.nan_to_num(w_loss, nan=-7.0))
         assert torch.equal(step.iou.view(torch.int16), w_iou.view(torch.int16)) and torch.equal(step.roi_out, w_roi)
+
+
+def test_bench_dump_outputs_of_one_step(tmp_path):
+    """bench.py --dump-outputs on a real step of its tiny workload: every result it names exists on CIMHeadStep, and
+    each file holds that result whole or at bench.dump_indices, in float32."""
+    import bench
+    cfg = bench.WORKLOADS["tiny"]
+    inp = bench.build_inputs(cfg, torch.device(DEV), 1234)
+    Cf, H, W, scale = inp["shape"]
+    step = CIMHeadStep(cfg["n_img"], cfg["R"], cfg["C"], Cf, H, W, scale, inp["packed"].shape[-1], device=DEV,
+                       mask_kb_per_row=inp["kb_per_row"], head_grads=True)
+    np.random.seed(3)
+    step.run(inp["feat"], inp["rois"], inp["grad_out"], inp["packed"], inp["seg_x"], inp["weight"], inp["bias"],
+             inp["labels"], mat=inp["mat"], mask_meta=inp["mask_meta"])
+    torch.cuda.synchronize()
+    bench.dump_outputs(step, str(tmp_path))
+    names = bench.STEP_OUTPUTS + bench.STEP_OUTPUTS_HEAD_GRADS
+    assert sorted(p.name for p in tmp_path.iterdir()) == sorted(f"{n}.npy" for n in names)
+    for name in names:
+        got = np.load(tmp_path / f"{name}.npy")
+        full = getattr(step, name).float().reshape(-1).cpu().numpy()
+        assert got.dtype == np.float32
+        np.testing.assert_array_equal(got, full[bench.dump_indices(full.size)] if full.size > bench.DUMP_ELEMS else full)

@@ -216,3 +216,31 @@ def test_rank_core_plan_follows_the_gpus_numa_node():
     # unknown nodes, fewer cores than ranks
     assert cdist.plan_rank_cores(2, 4, range(8), [-1] * 4, {}) == [4, 5]
     assert cdist.plan_rank_cores(0, 8, range(4), [-1] * 8, {}) is None
+
+
+def test_bench_dump_outputs_writes_whole_or_fixed_sample(tmp_path):
+    """bench.py --dump-outputs: small results whole, larger ones as the same seeded sample every run, all float32,
+    numpy's global generator (the step's anti-noise sampling) untouched."""
+    import types
+    import bench
+    n = bench.DUMP_ELEMS
+    g = torch.Generator().manual_seed(0)
+    step = types.SimpleNamespace(head_grads=False, **{name: torch.randn(3, 7, generator=g)
+                                                      for name in bench.STEP_OUTPUTS})
+    step.roi_out = torch.arange(2 * n + 6, dtype=torch.float32).view(-1, 2)     # value = flat index
+    step.iou = torch.rand(4, 5, generator=g).half()
+    step.valid = torch.tensor([[1, 0]], dtype=torch.uint8)
+    np.random.seed(5)
+    state = np.random.get_state()[1].copy()
+    bench.dump_outputs(step, str(tmp_path / "a"))
+    bench.dump_outputs(step, str(tmp_path / "b"))
+    assert np.array_equal(np.random.get_state()[1], state)
+    assert sorted(p.name for p in (tmp_path / "a").iterdir()) == sorted(f"{s}.npy" for s in bench.STEP_OUTPUTS)
+    for name in bench.STEP_OUTPUTS:
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, b)
+        full = getattr(step, name).float().reshape(-1).numpy()
+        if name == "roi_out":
+            np.testing.assert_array_equal(a, bench.dump_indices(full.size))
+        else:
+            np.testing.assert_array_equal(a, full)
