@@ -419,14 +419,21 @@ cim_anti_noise_kernel(cim_mine_params p, const float *__restrict__ labels, const
         if (n == 0) continue;
         if (lane == 0) {
             const float s = np_pairwise_sum_f32(prob, n);
-            double acc = 0.0;
-            for (int i = 0; i < n; ++i) {                              // np.cumsum: sequential, float64
-                const double v = (double)__fdiv_rn(prob[i], s);
-                acc = i == 0 ? v : __dadd_rn(acc, v);
-                cdf[i] = acc;
+            if (s == 0.f) {
+                // every weight of the class is 0: np.random.choice raises there (p = 0/0).  Deliberate divergence,
+                // shared with heads._anti_noise_keep: all n draws pick the class's first pseudo GT (cdf = 1 > u),
+                // and the class still consumes its n uniforms, so the stream stays in step for the classes after it
+                for (int i = 0; i < n; ++i) cdf[i] = 1.0;
+            } else {
+                double acc = 0.0;
+                for (int i = 0; i < n; ++i) {                          // np.cumsum: sequential, float64
+                    const double v = (double)__fdiv_rn(prob[i], s);
+                    acc = i == 0 ? v : __dadd_rn(acc, v);
+                    cdf[i] = acc;
+                }
+                const double last = cdf[n - 1];
+                for (int i = 0; i < n; ++i) cdf[i] = __ddiv_rn(cdf[i], last);
             }
-            const double last = cdf[n - 1];
-            for (int i = 0; i < n; ++i) cdf[i] = __ddiv_rn(cdf[i], last);
         }
         __syncwarp();
         for (int i = lane; i < n; i += 32) gt_keep[base + idx[i]] = 0;

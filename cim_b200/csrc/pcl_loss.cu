@@ -13,7 +13,7 @@
 //     return 12 * loss / (1e-6 + sum_k n_k)                                                                (:40-41)
 //   The reference loops over `mat.unique()` on the host with ~10 launches and two syncs per cluster; here one CTA
 //   per image makes three passes over its [R, C+1] slices (8 rows in flight per thread: the work is latency bound):
-//   ids -> per-row id lists and cluster tables in shared memory; cluster sums in 2^40 fixed point, so the
+//   ids -> per-row id lists and cluster tables in shared memory; cluster sums in 2^-44 fixed point, so the
 //   shared-memory atomics commute exactly (deterministic); gradients.
 // Cluster ids must be integers in [1, max_id] (they are small counters); anything else, or two different ids in
 // column 0 (the reference asserts there), yields a NaN loss and zero gradient.
@@ -43,8 +43,11 @@ __device__ float block_sum_p(float v, float *red) {
 }
 
 constexpr int UN = 8;                                   // rows in flight per thread: the passes are latency bound
-constexpr float FIX = 1099511627776.f;                  // 2^40: cluster sums are accumulated in fixed point, so the
-                                                        // shared-memory atomics commute exactly (deterministic)
+// Cluster sums are accumulated in fixed point (units of 2^-44), so the shared-memory atomics commute exactly
+// (deterministic).  Every float32 at or above 2^-21 is a whole number of units, so a cluster of one row has exactly
+// that row's scores as its mean and the clamp at float32(1e-6) decides as the reference does (with 2^-40 units a score
+// one ulp below the bound was rounded up onto the other side of it).  16384 rows of scores <= 1 stay below 2^58.
+constexpr float FIX = 17592186044416.f;                 // 2^44
 
 // insert `id` into the row's list of distinct ids (4 x 8 bit in one word); true if this call added it
 __device__ __forceinline__ bool row_add_id(uint32_t *slot, int id, int *err) {

@@ -121,13 +121,24 @@ def _anti_noise_keep(gt_cls, gt_w, present):
     (numpy/random/mtrand.pyx: cdf = p.cumsum(); cdf /= cdf[-1]; uniform = random_sample(n);
     idx = cdf.searchsorted(uniform, side='right')): it consumes the same n doubles of the global stream and
     returns the same indices, without choice()'s argument validation, which is 2/3 of its cost at these sizes
-    (this hop sits on the step's critical path).  tests/test_host_logic.py checks the equivalence."""
+    (this hop sits on the step's critical path).  tests/test_host_logic.py checks the equivalence.
+
+    A class whose pseudo GTs ALL have weight 0 (cls * det underflowed to 0 for every one of them, which a confident
+    head produces) is a deliberate divergence: np.random.choice raises ValueError on p = 0/0 and stops the reference's
+    training; here the class keeps its first pseudo GT and still consumes its n doubles, so the classes and steps
+    after it draw the doubles they would draw had the class been sampled.  cim_anti_noise does the same on the
+    device."""
     keep = np.ones(gt_cls.shape[0], dtype=np.uint8)
     for c in present:
         class_idx = np.nonzero(gt_cls == c)[0]
         if len(class_idx) == 0:
             continue
         prob = gt_w[class_idx]
+        if prob.sum() == 0:
+            np.random.random_sample(len(class_idx))
+            keep[class_idx] = 0
+            keep[class_idx[0]] = 1
+            continue
         cdf = (prob / prob.sum()).astype(np.float64).cumsum()
         cdf /= cdf[-1]
         drawn = class_idx[cdf.searchsorted(np.random.random_sample(len(class_idx)), side="right")]

@@ -59,27 +59,30 @@ def score_heads(x, weights, biases):
     return f(predict_cls), f(predict_det), [f(a) for a in ref_cls], [f(a) for a in ref_iou]
 
 
-def score_heads_bwd(x, weights, biases, grads):
+def score_heads_bwd(x, weights, biases, grads, outputs=None):
     """Backward of cls_iou_model.forward (autograd of heads.py:194-219) in float64.
 
     grads: 2+2K arrays [R,C1] = dL/d(output) in the order of `weights`.  Returns
     (grad_x [R,D], [grad_W_h [C1,D]], [grad_b_h [C1]]) as float32.  Pinned by oracle/make_golden.py
-    against torch autograd through the reference's own cls_iou_model."""
+    against torch autograd through the reference's own cls_iou_model.
+    outputs: optionally the forward's float32 outputs (2+2K arrays [R,C1]) to differentiate through, as torch's
+    softmax / sigmoid backward does with its saved outputs; by default they are recomputed in float64.  On saturated
+    scores the difference matters: near y = 1 the float32 rounding of y changes 1 - y by percents."""
     x = np.asarray(x, dtype=np.float64)
     k = (len(weights) - 2) // 2
     gx = np.zeros_like(x)
     gws, gbs = [], []
     for h, (w, b, g) in enumerate(zip(weights, biases, grads)):
         w, g = np.asarray(w, np.float64), np.asarray(g, np.float64)
-        z = x @ w.T + np.asarray(b, np.float64)
+        z = x @ w.T + np.asarray(b, np.float64) if outputs is None else None
         if h == 1:                                    # softmax over proposals (:203)
-            y = _softmax(z, axis=0)
+            y = _softmax(z, axis=0) if z is not None else np.asarray(outputs[h], np.float64)
             dz = y * (g - (g * y).sum(0, keepdims=True))
         elif h < 2 + k:                               # softmax over classes (:200, :212)
-            y = _softmax(z, axis=-1)
+            y = _softmax(z, axis=-1) if z is not None else np.asarray(outputs[h], np.float64)
             dz = y * (g - (g * y).sum(-1, keepdims=True))
         else:                                         # sigmoid (:216)
-            y = 1.0 / (1.0 + np.exp(-z))
+            y = 1.0 / (1.0 + np.exp(-z)) if z is not None else np.asarray(outputs[h], np.float64)
             dz = g * y * (1.0 - y)
         gx += dz @ w
         gws.append((dz.T @ x).astype(np.float32))

@@ -15,7 +15,10 @@ restatement reproduces them within 1e-6 relative (make_golden asserts it, tests/
 import numpy as np
 import torch
 
-LO, HI = 1e-6, 1 - 1e-6
+# The reference clamps float32 tensors, so torch rounds the bounds 1e-6 and 1 - 1e-6 to float32 first (both roundings
+# go down).  At float64 the unrounded bound 1e-6 would lie above float32(1e-6) and zero the gradient of a score that
+# sits exactly on it, where the reference passes the gradient (torch.clamp is inclusive).
+LO, HI = float(np.float32(1e-6)), float(np.float32(1 - 1e-6))
 
 
 def weighted_bag_loss(pred, pseudo, label_tmp, w):

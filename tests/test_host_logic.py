@@ -5,6 +5,7 @@ import inspect
 import sys
 
 import numpy as np
+import pytest
 import torch
 
 from cim_b200 import heads, integration, ops, synth
@@ -83,6 +84,83 @@ def test_anti_noise_draw_equals_numpy_choice_on_many_cases():
         state_b = np.random.get_state()[1].copy(), np.random.get_state()[2]
         assert a.astype(bool).tolist() == b.tolist(), case
         assert state_a[1] == state_b[1] and np.array_equal(state_a[0], state_b[0]), case
+
+
+def _zero_weight_groups(rng, n_cases):
+    """Pseudo-GT lists whose class groups hold exact zeros (det underflowed), all-equal weights and a single non-zero
+    weight among zeros; no group is all zero."""
+    cases = []
+    for _ in range(n_cases):
+        g = int(rng.choice([2, 3, 9, 40, 130, 600]))
+        gt_cls = rng.randint(0, 3, g)
+        kind = int(rng.randint(3))
+        if kind == 0:                                              # some zeros, anywhere (first and last included)
+            gt_w = rng.rand(g).astype(np.float32) * (rng.rand(g) < 0.5)
+        elif kind == 1:                                            # all equal
+            gt_w = np.full(g, np.float32(rng.choice([1.0, 0.0625, 1e-30])), np.float32)
+        else:                                                      # one non-zero weight per class
+            gt_w = np.zeros(g, np.float32)
+        for c in range(3):
+            idx = np.nonzero(gt_cls == c)[0]
+            if len(idx) and gt_w[idx].sum() == 0:
+                gt_w[idx[rng.randint(len(idx))]] = np.float32(rng.rand() + 1e-3)
+        cases.append((gt_cls, gt_w.astype(np.float32)))
+    return cases
+
+
+def test_anti_noise_draw_equals_numpy_choice_with_zero_weights():
+    """Zero weights are legal input for np.random.choice (heads.py:459) as long as a class's weights do not all
+    vanish: the host draw must pick what choice picks and consume what it consumes."""
+    rng = np.random.RandomState(31)
+    cases = _zero_weight_groups(rng, 200)
+    assert sum(int((w == 0).sum()) for _, w in cases) > 1000
+    assert any(len(np.unique(w)) == 1 and len(w) > 1 for _, w in cases)
+    assert any(np.count_nonzero(w[c == 0]) == 1 and (c == 0).sum() > 3 for c, w in cases)
+    labels = np.zeros(20, np.float32)
+    labels[:3] = 1
+    for case, (gt_cls, gt_w) in enumerate(cases):
+        np.random.seed(case)
+        a = heads._anti_noise_keep(gt_cls, gt_w, np.nonzero(labels)[0])
+        state_a = np.random.get_state()
+        np.random.seed(case)
+        b = heads_oracle.anti_noise_keep(gt_cls, gt_w, labels)
+        state_b = np.random.get_state()
+        assert a.astype(bool).tolist() == b.tolist(), case
+        assert state_a[2] == state_b[2] and np.array_equal(state_a[1], state_b[1]), case
+        assert not a[gt_w == 0].any(), case                          # a zero-weight pseudo GT is never drawn
+
+
+def test_anti_noise_all_zero_group_keeps_first_gt_and_consumes_the_stream():
+    """A class whose pseudo GTs all have weight 0: np.random.choice raises (the reference stops), the host keeps the
+    class's first pseudo GT, consumes the class's n doubles, and draws the other classes as choice does."""
+    gt_cls = np.array([0, 1, 1, 2, 1, 0, 1, 2, 2], np.int64)
+    gt_w = np.array([0.5, 0, 0, 0.25, 0, 0.125, 0, 0, 0.75], np.float32)
+    present = np.array([0, 1, 2])
+    with np.errstate(invalid="ignore"):
+        with pytest.raises(ValueError):
+            np.random.choice(np.nonzero(gt_cls == 1)[0], 4, replace=True, p=gt_w[gt_cls == 1] / gt_w[gt_cls == 1].sum())
+        np.random.seed(7)
+        keep = heads._anti_noise_keep(gt_cls, gt_w, present)
+    state = np.random.get_state()
+    assert keep[gt_cls == 1].tolist() == [1, 0, 0, 0] and keep[1] == 1
+    np.random.seed(7)
+    want = np.ones(len(gt_cls), np.uint8)
+    for c in present:
+        idx = np.nonzero(gt_cls == c)[0]
+        if c == 1:
+            np.random.random_sample(len(idx))
+            want[idx] = 0
+            want[idx[0]] = 1
+            continue
+        drawn = np.random.choice(idx, len(idx), replace=True, p=gt_w[idx] / gt_w[idx].sum())
+        want[idx] = 0
+        want[drawn] = 1
+    assert keep.tolist() == want.tolist()
+    want_state = np.random.get_state()
+    assert state[2] == want_state[2] and np.array_equal(state[1], want_state[1])
+    np.random.seed(7)
+    np.random.random_sample(len(gt_cls))
+    assert np.array_equal(np.random.get_state()[1], state[1])      # exactly n doubles per class, n summed
 
 
 def test_one_random_sample_call_is_the_stream_of_the_per_class_choice_calls():
