@@ -75,6 +75,8 @@ _SIGNATURES = {
     "cim_test_scores": (_I, [_P, _P, _I64, _I, _I, _P]),
     "cim_box_nms": (_I, [_P, _P, _I, _I, _I, _F, _F, _P, _P]),
     "cim_box_nms_batched": (_I, [_P, _P, _I, _I, _I, _I, _F, _F, _P, _P]),
+    "cim_test_scores_tta": (_I, [_P, _P, _I64, _I, _I, _I, _I, _P]),
+    "cim_box_detections": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P]),
     "cim_sizeof_mine_params": (_SZ, []),
     "cim_mine_workspace_bytes": (_SZ, [C.POINTER(MineParams)]),
     "cim_mine": (_I, [C.POINTER(MineParams), C.POINTER(_P), C.POINTER(_P), _P, _P, _P, _P, _P, _P, _P, _P,

@@ -392,6 +392,24 @@ int cim_box_nms(const float *boxes, const float *scores, int n, int n_classes, i
  * keep [n_img, n_classes, n] (one CTA per (class, image): 80 CTAs of one image leave half a B200 idle). */
 int cim_box_nms_batched(const float *boxes, const float *scores, int n_img, int n, int n_classes, int score_stride,
                         float score_thresh, float nms_thresh, uint8_t *keep, cim_stream_t stream);
+/* cim_test_scores_tta: pass t of T of the test-time-augmentation score mean of lib/core/test.py:149-226
+ *   (TEST.BBOX_AUG, SCORE_HEUR 'AVG': np.mean(scores_ts, axis=0)).  s = the cim_test_scores result of this pass's
+ *   scores [2+2K, M, C1]; acc [M, C1-1] = s when t == 0, fl(acc + s) otherwise, and on the last pass (t == T-1,
+ *   T > 1) fl(acc / T).  The passes are summed in call order.  cim_test_scores is the t = 0, T = 1 case. */
+int cim_test_scores_tta(const float *scores, float *acc, int64_t M, int C1, int K, int t, int T, cim_stream_t stream);
+/* cim_box_detections: the DETECTIONS_PER_IM limit and the per-class detection lists of
+ *   lib/utils/mask_eval_utils.py:80-110 for the keep mask of cim_box_nms_batched (same boxes, scores, n_img, n,
+ *   n_classes, score_stride).  Per image: total = kept entries over all classes; when detections_per_im > 0 and
+ *   total > detections_per_im, thresh = the detections_per_im-th largest kept score (with multiplicity) and an entry
+ *   survives iff it is kept and score >= thresh (float32; ties at thresh all survive), otherwise every kept entry
+ *   survives.  count [n_img] int32 = survivors (also when > cap); the first min(count, cap) survivors, ordered by
+ *   class then proposal index, are written to det_cls / det_idx [n_img, cap] int32, det_score [n_img, cap] fp32
+ *   (= scores[i][c]) and det_box [n_img, cap, 4] fp32 (= boxes[i]; may be NULL); the rest of a row is not written.
+ *   keep_out [n_img, n_classes, n] uint8 (may be NULL) = the keep mask after the limit.  det_* may be NULL when
+ *   cap == 0.  No workspace.  n <= 8192. */
+int cim_box_detections(const float *boxes, const float *scores, const uint8_t *keep, int n_img, int n, int n_classes,
+                       int score_stride, int detections_per_im, int cap, uint8_t *keep_out, int32_t *count,
+                       int32_t *det_cls, int32_t *det_idx, float *det_score, float *det_box, cim_stream_t stream);
 
 #ifdef __cplusplus
 }
