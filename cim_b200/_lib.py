@@ -8,11 +8,12 @@ import ctypes as C
 import os
 import threading
 
+import numpy as np
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libcimhead.so")
-ABI_VERSION = 3
+ABI_VERSION = 4
 MAX_LAYERS = 4
 OVERLAP_ALGOS = {"auto": 0, "popc": 1, "tensor": 2}
 #: cim_set_debug_flags bits (include/cimhead.h): diagnostic kernel selection for A/B timing and bit-identity tests
@@ -70,8 +71,11 @@ _SIGNATURES = {
     "cim_score_heads": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _SZ, _P]),
     "cim_score_heads_bwd_workspace_bytes": (_SZ, [_I, _I, _I, _I, _I]),
     "cim_score_heads_bwd": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _SZ, _P]),
+    "cim_score_heads_ex": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _SZ, _P]),
+    "cim_score_heads_bwd_ex": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _SZ, _P]),
     "cim_head_losses": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _F, _F, _F, _P]),
     "cim_pcl_loss": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _F, _I, _P]),
+    "cim_pcl_loss_ex": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _I, _P]),
     "cim_test_scores": (_I, [_P, _P, _I64, _I, _I, _P]),
     "cim_box_nms": (_I, [_P, _P, _I, _I, _I, _F, _F, _P, _P]),
     "cim_box_nms_batched": (_I, [_P, _P, _I, _I, _I, _I, _F, _F, _P, _P]),
@@ -85,6 +89,10 @@ _SIGNATURES = {
     "cim_anti_noise": (_I, [C.POINTER(MineParams), _P, _P, _P, _P, _P, _P, _P]),
     "cim_anti_noise_stream": (_I, [C.POINTER(MineParams), _P, _P, _P, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "cim_assign": (_I, [C.POINTER(MineParams), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "cim_mine_ex": (_I, [C.POINTER(MineParams), _P, C.c_double, C.POINTER(_P), C.POINTER(_P), _P, _P, _P, _P, _P, _P,
+                         _P, _P, _P, _SZ, _P]),
+    "cim_mine_image_constants": (_I, [C.c_double, _I, C.POINTER(_I), C.POINTER(_F)]),
+    "cim_assign_ex": (_I, [C.POINTER(MineParams), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 
@@ -140,6 +148,31 @@ def stream_ptr(device):
 
 def ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
+
+
+def n_props_arg(n_props, n_img, R, device):
+    """The n_props argument of the ragged entry points -> None (every image has R proposals) or a CUDA int32 [n_img]
+    tensor on `device`.  A host sequence, numpy array or CPU tensor is validated (length n_img, integers in [1, R]) and
+    copied to the device once; a CUDA tensor must be int32 [n_img] on `device` and is used as is (its values cannot be
+    checked without a synchronisation: the kernels clamp them to [1, R])."""
+    if n_props is None:
+        return None
+    if isinstance(n_props, torch.Tensor) and n_props.device.type != "cpu":
+        if not n_props.is_cuda or n_props.device != torch.device(device):
+            raise ValueError(f"n_props must be on {device} or on the host, got {n_props.device}")
+        if n_props.dtype != torch.int32:
+            raise TypeError(f"n_props must be int32 on the device, got {n_props.dtype}")
+        if n_props.numel() != n_img or n_props.dim() != 1:
+            raise ValueError(f"n_props must have shape [{n_img}], got {tuple(n_props.shape)}")
+        return n_props.contiguous()
+    a = n_props.numpy() if isinstance(n_props, torch.Tensor) else np.asarray(n_props)
+    if a.dtype.kind not in "iu":
+        raise TypeError(f"n_props must hold integers, got {a.dtype}")
+    if a.shape != (n_img,):
+        raise ValueError(f"n_props must have shape [{n_img}], got {a.shape}")
+    if a.size and (a.min() < 1 or a.max() > R):
+        raise ValueError(f"n_props must lie in [1, {R}], got [{a.min()}, {a.max()}]")
+    return torch.from_numpy(a.astype(np.int32)).to(device, non_blocking=True)
 
 
 def require_cuda(t, name, dtype=None):

@@ -23,7 +23,24 @@
 //                       labels (:477-501; :493-498 is a swallowed exception in the reference and
 //                       is deliberately not applied).
 // Every comparison on a map value is made in fp16 against fp16(threshold).
+//
+// Ragged batches (cim_mine_ex / cim_assign_ex): image b owns rows [0, n_b) of its R rows.  Its seeds are sorted from
+// rows < n_b only, its containment counts run over columns < n_b, and keep_count / big_thr are evaluated for n_b on
+// the device by cim_image_constants(); rows >= n_b get asy_flag 0 and the ignore row of the assignment.
 #include "common.cuh"
+
+// heads.py:332 and :338 for an image of n proposals, in the reference's arithmetic: int(np.ceil(p_seed * n)) and
+// np.float32(0.9 * n), a float64 product rounded once.  Shared by the kernels and cim_mine_image_constants().
+__host__ __device__ inline void cim_image_constants(double p_seed, int n, int *keep_count, float *big_thr) {
+#ifdef __CUDA_ARCH__
+    *keep_count = (int)ceil(__dmul_rn(p_seed, (double)n));
+    *big_thr = __double2float_rn(__dmul_rn(0.9, (double)n));
+#else
+    volatile double kp = p_seed * (double)n, bp = 0.9 * (double)n;      // volatile: no contraction, no x87 excess
+    *keep_count = (int)ceil(kp);
+    *big_thr = (float)bp;
+#endif
+}
 
 namespace {
 
@@ -41,6 +58,24 @@ struct MineWs {
 };
 
 __host__ __device__ inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// rows, seed count and big-proposal threshold of image img: n_props[img] clamped to [1, R] and the constants for it,
+// or R and the host-evaluated p.keep_count / p.big_thr when n_props is NULL.  keep_count never exceeds p.keep_count,
+// the capacity the workspace was sized for.
+struct ImageRows {
+    int n, keep_count;
+    float big_thr;
+};
+__device__ __forceinline__ ImageRows image_rows(const cim_mine_params &p, const int32_t *n_props, double p_seed,
+                                                int img) {
+    ImageRows r{p.R, p.keep_count, p.big_thr};
+    if (n_props) {
+        r.n = min(max(n_props[img], 1), p.R);
+        cim_image_constants(p_seed, r.n, &r.keep_count, &r.big_thr);
+        r.keep_count = min(max(r.keep_count, 1), p.keep_count);
+    }
+    return r;
+}
 
 __host__ inline MineWs carve_ws(void *ws, const cim_mine_params &p) {
     const size_t slots = (size_t)p.n_layers * p.n_img * p.C;
@@ -60,14 +95,17 @@ __device__ __forceinline__ bool before(float ka, int ia, float kb, int ib) {
 }
 
 // ------------------------------------------------------------------------------ seeds + NMS
-__global__ void __launch_bounds__(512)
+__global__ void __launch_bounds__(512, 4)
 cim_seed_kernel(LayerPtrs ptrs, const float *__restrict__ labels, const __half *__restrict__ iou_all,
-                cim_mine_params p, int npad, MineWs ws) {
+                cim_mine_params p, int npad, MineWs ws, const int32_t *__restrict__ n_props, double p_seed) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int c = blockIdx.x, l = blockIdx.y, img = blockIdx.z;
     if (labels[(size_t)img * p.C + c] == 0.f) return;
     const int R = p.R, kc = p.keep_count, tid = threadIdx.x, nthr = blockDim.x;
     const int slot = (l * p.n_img + img) * p.C + c;
+    const ImageRows ir = image_rows(p, n_props, p_seed, img);
+    const int n = ir.n;
+    while ((npad >> 1) >= n) npad >>= 1;                              // the image's own power of two
 
     int *seeds = reinterpret_cast<int *>(smem_raw);                   // [kc]
     unsigned char *big = smem_raw + align_up((size_t)kc * 4, 16);
@@ -80,12 +118,12 @@ cim_seed_kernel(LayerPtrs ptrs, const float *__restrict__ labels, const __half *
     const int dcol = p.det_cols == 1 ? 0 : c + (p.det_cols == p.C + 1 ? 1 : 0);
     for (int i = tid; i < npad; i += nthr) {
         float v = -INFINITY;
-        if (i < R) {
+        if (i < n) {
             v = cls[(size_t)i * p.C1 + c + bg];
             if (p.mode == 1 && det) v = __fmul_rn(v, det[(size_t)i * p.det_cols + dcol]);   // MIST ranks cls*det
         }
         key[i] = v;
-        idx[i] = i < R ? i : 0x7fffffff;
+        idx[i] = i < n ? i : 0x7fffffff;
     }
     __syncthreads();
     for (int size = 2; size <= npad; size <<= 1)
@@ -100,7 +138,7 @@ cim_seed_kernel(LayerPtrs ptrs, const float *__restrict__ labels, const __half *
             }
             __syncthreads();
         }
-    const int k = min(kc, R);
+    const int k = min(ir.keep_count, n);
     for (int i = tid; i < k; i += nthr) seeds[i] = idx[i];
     __syncthreads();
 
@@ -149,26 +187,34 @@ cim_seed_kernel(LayerPtrs ptrs, const float *__restrict__ labels, const __half *
 // ------------------------------------------------------------------------- containment pass
 __global__ void __launch_bounds__(256)
 cim_contain_kernel(LayerPtrs ptrs, const float *__restrict__ labels, const __half *__restrict__ asy_all,
-                   cim_mine_params p, MineWs ws, uint8_t *__restrict__ asy_flag) {
+                   cim_mine_params p, MineWs ws, uint8_t *__restrict__ asy_flag, const int32_t *__restrict__ n_props,
+                   double p_seed) {
     const int img = blockIdx.y, lane = threadIdx.x & 31;
     const int i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const int R = p.R;
     if (i >= R) return;
+    const int n = n_props ? min(max(n_props[img], 1), R) : R;
+    if (i >= n) {                                                   // padding row: never big, never a container
+        if (lane == 0 && asy_flag) asy_flag[(size_t)img * R + i] = 0;
+        return;
+    }
     const __half *row = asy_all + ((size_t)img * R + i) * R;
     const __half con = __float2half_rn(p.con_thr);
     int cnt = 0;
     if ((R & 1) == 0 && (((uintptr_t)row) & 3) == 0) {
         const __half2 *row2 = reinterpret_cast<const __half2 *>(row);
-        for (int j = lane; j < (R >> 1); j += 32) {
+        for (int j = lane; j < (n >> 1); j += 32) {
             const __half2 v = row2[j];
             cnt += (int)__hgt(__low2half(v), con) + (int)__hgt(__high2half(v), con);
         }
+        if ((n & 1) && lane == 0) cnt += (int)__hgt(row[n - 1], con);
     } else {
-        for (int j = lane; j < R; j += 32) cnt += (int)__hgt(row[j], con);
+        for (int j = lane; j < n; j += 32) cnt += (int)__hgt(row[j], con);
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-    const bool flag = (float)cnt < p.big_thr;                       // heads.py:338
+    const float big_thr = n_props ? image_rows(p, n_props, p_seed, img).big_thr : p.big_thr;
+    const bool flag = (float)cnt < big_thr;                         // heads.py:338
     if (lane == 0 && asy_flag) asy_flag[(size_t)img * R + i] = flag ? 1 : 0;
     if (!flag || p.mode != 0) return;
 
@@ -268,11 +314,21 @@ cim_assign_kernel(cim_mine_params p, const __half *__restrict__ iou_all, const i
                   const int32_t *__restrict__ gt_rows, const int32_t *__restrict__ gt_class,
                   const float *__restrict__ gt_weight, const uint8_t *__restrict__ gt_keep,
                   float *__restrict__ pseudo_labels, __half *__restrict__ pseudo_iou,
-                  float *__restrict__ loss_weights, uint8_t *__restrict__ valid) {
+                  float *__restrict__ loss_weights, uint8_t *__restrict__ valid, const int32_t *__restrict__ n_props) {
     const int l = blockIdx.y, img = blockIdx.z, lane = threadIdx.x & 31, R = p.R;
     const int i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (i >= R) return;
     const int li = l * p.n_img + img;
+    const int C1o = p.C + 1;
+    if (n_props && i >= min(max(n_props[img], 1), R)) {             // padding row: the ignore row (heads.py:484-486)
+        float *pl = pseudo_labels + ((size_t)li * R + i) * C1o;
+        for (int c = lane; c < C1o; c += 32) pl[c] = 0.f;
+        if (lane == 0) {
+            pseudo_iou[(size_t)li * R + i] = __float2half_rn(0.f);
+            loss_weights[(size_t)li * R + i] = 0.f;
+        }
+        return;
+    }
     const int G = gt_count[li];
     const size_t gbase = (size_t)li * p.gt_cap;
     const __half *row = iou_all + ((size_t)img * R + i) * R;
@@ -301,7 +357,6 @@ cim_assign_kernel(cim_mine_params p, const __half *__restrict__ iou_all, const i
             bv = ov; bg_ = og; bh = __ushort_as_half(oh);
         }
     }
-    const int C1o = p.C + 1;
     float *pl = pseudo_labels + ((size_t)li * R + i) * C1o;
     if (!seen) {                                  // nothing mined for this (layer, image)
         for (int c = lane; c < C1o; c += 32) pl[c] = 0.f;
@@ -472,12 +527,26 @@ CIM_API size_t cim_mine_workspace_bytes(const cim_mine_params *p) {
            align_up(slots * 4, 256);
 }
 
-CIM_API int cim_mine(const cim_mine_params *p, const float *const *cls, const float *const *det,
-                     const float *labels, const void *iou_f16, const void *asy_f16, int32_t *gt_count,
-                     int32_t *gt_rows, int32_t *gt_class, float *gt_weight, uint8_t *asy_flag, void *workspace,
-                     size_t ws_bytes, cim_stream_t stream) {
+CIM_API int cim_mine_image_constants(double p_seed, int n, int *keep_count, float *big_thr) {
+    if (!keep_count || !big_thr || n < 1 || !(p_seed > 0.0 && p_seed <= 1.0)) return CIM_ERR_ARG;
+    cim_image_constants(p_seed, n, keep_count, big_thr);
+    return CIM_OK;
+}
+
+CIM_API int cim_mine_ex(const cim_mine_params *p, const int32_t *n_props, double p_seed, const float *const *cls,
+                        const float *const *det, const float *labels, const void *iou_f16, const void *asy_f16,
+                        int32_t *gt_count, int32_t *gt_rows, int32_t *gt_class, float *gt_weight, uint8_t *asy_flag,
+                        void *workspace, size_t ws_bytes, cim_stream_t stream) {
     int rc = check_params(p);
     if (rc) return rc;
+    if (n_props) {
+        if (!(p_seed > 0.0 && p_seed <= 1.0)) return CIM_ERR_ARG;
+        int kc_full;
+        float bt;
+        cim_image_constants(p_seed, p->R, &kc_full, &bt);
+        if (p->keep_count < kc_full) return CIM_ERR_ARG;          // the capacity must hold a full image's seeds
+        if (!cim_aligned(n_props, 4)) return CIM_ERR_ALIGN;
+    }
     if (!cls || !labels || !iou_f16 || !gt_count || !gt_rows || !gt_class || !gt_weight) return CIM_ERR_ARG;
     if (p->mode == 0 && (!det || !asy_f16)) return CIM_ERR_ARG;
     if (!workspace || ws_bytes < cim_mine_workspace_bytes(p) || !cim_aligned(workspace, 256)) return CIM_ERR_WORKSPACE;
@@ -500,13 +569,13 @@ CIM_API int cim_mine(const cim_mine_params *p, const float *const *cls, const fl
     if (smem_seed > (size_t)cim_max_smem_optin()) return CIM_ERR_SHAPE;
     cudaFuncSetAttribute(cim_seed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_seed);
     cim_seed_kernel<<<dim3(p->C, p->n_layers, p->n_img), 512, smem_seed, st>>>(
-        ptrs, labels, reinterpret_cast<const __half *>(iou_f16), *p, npad, ws);
+        ptrs, labels, reinterpret_cast<const __half *>(iou_f16), *p, npad, ws, n_props, p_seed);
     if ((rc = cim_launch_status())) return rc;
 
     if (p->mode == 0 || asy_flag) {
         if (asy_f16) {
             cim_contain_kernel<<<dim3((p->R + 7) / 8, p->n_img), 256, 0, st>>>(
-                ptrs, labels, reinterpret_cast<const __half *>(asy_f16), *p, ws, asy_flag);
+                ptrs, labels, reinterpret_cast<const __half *>(asy_f16), *p, ws, asy_flag, n_props, p_seed);
             if ((rc = cim_launch_status())) return rc;
         }
     }
@@ -517,19 +586,36 @@ CIM_API int cim_mine(const cim_mine_params *p, const float *const *cls, const fl
     return cim_launch_status();
 }
 
-CIM_API int cim_assign(const cim_mine_params *p, const void *iou_f16, const int32_t *gt_count,
-                       const int32_t *gt_rows, const int32_t *gt_class, const float *gt_weight,
-                       const uint8_t *gt_keep, float *pseudo_labels, void *pseudo_iou_f16, float *loss_weights,
-                       uint8_t *valid, cim_stream_t stream) {
+CIM_API int cim_mine(const cim_mine_params *p, const float *const *cls, const float *const *det,
+                     const float *labels, const void *iou_f16, const void *asy_f16, int32_t *gt_count,
+                     int32_t *gt_rows, int32_t *gt_class, float *gt_weight, uint8_t *asy_flag, void *workspace,
+                     size_t ws_bytes, cim_stream_t stream) {
+    return cim_mine_ex(p, nullptr, 0.0, cls, det, labels, iou_f16, asy_f16, gt_count, gt_rows, gt_class, gt_weight,
+                       asy_flag, workspace, ws_bytes, stream);
+}
+
+CIM_API int cim_assign_ex(const cim_mine_params *p, const int32_t *n_props, const void *iou_f16,
+                          const int32_t *gt_count, const int32_t *gt_rows, const int32_t *gt_class,
+                          const float *gt_weight, const uint8_t *gt_keep, float *pseudo_labels, void *pseudo_iou_f16,
+                          float *loss_weights, uint8_t *valid, cim_stream_t stream) {
     int rc = check_params(p);
     if (rc) return rc;
     if (!iou_f16 || !gt_count || !gt_rows || !gt_class || !gt_weight || !pseudo_labels || !pseudo_iou_f16 ||
         !loss_weights || !valid)
         return CIM_ERR_ARG;
+    if (!cim_aligned(n_props, 4)) return CIM_ERR_ALIGN;
     cim_assign_kernel<<<dim3((p->R + 7) / 8, p->n_layers, p->n_img), 256, 0, (cudaStream_t)stream>>>(
         *p, reinterpret_cast<const __half *>(iou_f16), gt_count, gt_rows, gt_class, gt_weight, gt_keep,
-        pseudo_labels, reinterpret_cast<__half *>(pseudo_iou_f16), loss_weights, valid);
+        pseudo_labels, reinterpret_cast<__half *>(pseudo_iou_f16), loss_weights, valid, n_props);
     return cim_launch_status();
+}
+
+CIM_API int cim_assign(const cim_mine_params *p, const void *iou_f16, const int32_t *gt_count,
+                       const int32_t *gt_rows, const int32_t *gt_class, const float *gt_weight,
+                       const uint8_t *gt_keep, float *pseudo_labels, void *pseudo_iou_f16, float *loss_weights,
+                       uint8_t *valid, cim_stream_t stream) {
+    return cim_assign_ex(p, nullptr, iou_f16, gt_count, gt_rows, gt_class, gt_weight, gt_keep, pseudo_labels,
+                         pseudo_iou_f16, loss_weights, valid, stream);
 }
 
 CIM_API size_t cim_anti_noise_uniform_count_max(const cim_mine_params *p) {

@@ -17,6 +17,8 @@
 //   shared-memory atomics commute exactly (deterministic); gradients.
 // Cluster ids must be integers in [1, max_id] (they are small counters); anything else, or two different ids in
 // column 0 (the reference asserts there), yields a NaN loss and zero gradient.
+// Ragged batches (cim_pcl_loss_ex): mat is read as 0 for rows r >= n_props[b], so those rows join no cluster and get
+// a zero gradient (or keep what grad_cls held, with accumulate).
 #include "common.cuh"
 
 namespace {
@@ -68,7 +70,8 @@ __device__ __forceinline__ bool row_add_id(uint32_t *slot, int id, int *err) {
 
 __global__ void __launch_bounds__(PT)
 cim_pcl_loss_kernel(const float *__restrict__ pcls, const float *__restrict__ mat, float *__restrict__ loss_out,
-                    float *__restrict__ grad, int R, int C1, int max_id, float grad_scale, int accumulate) {
+                    float *__restrict__ grad, const int32_t *__restrict__ n_props, int R, int C1, int max_id,
+                    float grad_scale, int accumulate) {
     extern __shared__ __align__(16) unsigned char dyn[];
     // layout: sum64 [max_id+1][C1] i64 (later re-used as vgrad f32) | cnt [max_id+1] i32 | colmask [max_id+1][4] u32 |
     //         lk [max_id+1] f32 | rowids [R] u32 (4 x 8-bit distinct ids of the row)
@@ -87,6 +90,7 @@ cim_pcl_loss_kernel(const float *__restrict__ pcls, const float *__restrict__ ma
     float *g = grad ? grad + (size_t)b * R * C1 : nullptr;
     const int G = PT / C1, rg = tid / C1, c = tid - rg * C1;
     const bool elem = tid < G * C1;
+    const int n = n_props ? min(max(n_props[b], 1), R) : R;          // rows of this image; the rest read as mat = 0
 
     for (int i = tid; i < NI * C1; i += PT) sum64[i] = 0ull;
     for (int i = tid; i < NI; i += PT) { cnt[i] = 0; lk[i] = 0.f; }
@@ -102,7 +106,7 @@ cim_pcl_loss_kernel(const float *__restrict__ pcls, const float *__restrict__ ma
 #pragma unroll
             for (int i = 0; i < UN; ++i) {
                 const int r = r0 + i * G;
-                v[i] = r < R ? __ldg(m + (size_t)r * C1 + c) : 0.f;
+                v[i] = r < n ? __ldg(m + (size_t)r * C1 + c) : 0.f;
             }
 #pragma unroll
             for (int i = 0; i < UN; ++i) {
@@ -210,17 +214,25 @@ cim_pcl_loss_kernel(const float *__restrict__ pcls, const float *__restrict__ ma
 
 }  // namespace
 
-CIM_API int cim_pcl_loss(const float *predict_cls, const float *mat, float *loss, float *grad_cls, int n_img, int R,
-                         int C1, int max_id, float grad_scale, int accumulate, cim_stream_t stream) {
+CIM_API int cim_pcl_loss_ex(const float *predict_cls, const float *mat, const int32_t *n_props, float *loss,
+                            float *grad_cls, int n_img, int R, int C1, int max_id, float grad_scale, int accumulate,
+                            cim_stream_t stream) {
     if (!predict_cls || !mat || !loss) return CIM_ERR_ARG;
     if (n_img < 0 || R <= 0 || C1 < 2 || max_id < 1) return CIM_ERR_ARG;
     if (n_img == 0) return CIM_OK;
     if (C1 > 128 || max_id > 255 || R > 16384) return CIM_ERR_SHAPE;
+    if (!cim_aligned(n_props, 4)) return CIM_ERR_ALIGN;
     const size_t NI = (size_t)max_id + 1;
     const size_t smem = NI * C1 * 8 + NI * 4 + NI * 16 + NI * 4 + (size_t)R * 4 + 16;
     if ((int)smem + 8192 > cim_max_smem_optin()) return CIM_ERR_SHAPE;
     cudaFuncSetAttribute(cim_pcl_loss_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    cim_pcl_loss_kernel<<<(unsigned)n_img, PT, smem, (cudaStream_t)stream>>>(predict_cls, mat, loss, grad_cls, R, C1,
-                                                                            max_id, grad_scale, accumulate);
+    cim_pcl_loss_kernel<<<(unsigned)n_img, PT, smem, (cudaStream_t)stream>>>(predict_cls, mat, loss, grad_cls, n_props, R,
+                                                                            C1, max_id, grad_scale, accumulate);
     return cim_launch_status();
+}
+
+CIM_API int cim_pcl_loss(const float *predict_cls, const float *mat, float *loss, float *grad_cls, int n_img, int R,
+                         int C1, int max_id, float grad_scale, int accumulate, cim_stream_t stream) {
+    return cim_pcl_loss_ex(predict_cls, mat, nullptr, loss, grad_cls, n_img, R, C1, max_id, grad_scale, accumulate,
+                           stream);
 }

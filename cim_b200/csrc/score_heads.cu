@@ -118,15 +118,19 @@ __global__ void score_row_act_kernel(float *__restrict__ s, int M, int C1, int K
     }
 }
 
-// detector head: softmax over the R proposals of one image for one class; block = (class, image)
+// detector head: softmax over the n proposals of one image for one class; block = (class, image).  n = n_props[img]
+// clamped to [1, R] (R when n_props is NULL): the partial sums run over r < n in the order of a launch with R = n, and
+// the block writes 0 into column c of every head for the padding rows r >= n.
 __global__ void __launch_bounds__(256)
-score_col_softmax_kernel(float *__restrict__ det, int R, int C1) {
+score_col_softmax_kernel(float *__restrict__ scores, const int32_t *__restrict__ n_props, long long M, int nheads,
+                         int R, int C1) {
     __shared__ float red[8];
     __shared__ float bcast;
     const int c = blockIdx.x, img = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    float *col = det + (size_t)img * R * C1 + c;
+    const int n = n_props ? min(max(n_props[img], 1), R) : R;
+    float *col = scores + ((size_t)M + (size_t)img * R) * C1 + c;
     float mx = -INFINITY;
-    for (int r = tid; r < R; r += 256) mx = fmaxf(mx, col[(size_t)r * C1]);
+    for (int r = tid; r < n; r += 256) mx = fmaxf(mx, col[(size_t)r * C1]);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
     if (lane == 0) red[warp] = mx;
@@ -139,7 +143,7 @@ score_col_softmax_kernel(float *__restrict__ det, int R, int C1) {
     __syncthreads();
     mx = bcast;
     float sum = 0.f;
-    for (int r = tid; r < R; r += 256) sum += expf(col[(size_t)r * C1] - mx);
+    for (int r = tid; r < n; r += 256) sum += expf(col[(size_t)r * C1] - mx);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
     __syncthreads();
@@ -152,7 +156,11 @@ score_col_softmax_kernel(float *__restrict__ det, int R, int C1) {
     }
     __syncthreads();
     sum = bcast;
-    for (int r = tid; r < R; r += 256) col[(size_t)r * C1] = expf(col[(size_t)r * C1] - mx) / sum;
+    for (int r = tid; r < n; r += 256) col[(size_t)r * C1] = expf(col[(size_t)r * C1] - mx) / sum;
+    for (int h = 0; h < nheads; ++h) {
+        float *hc = scores + ((size_t)h * M + (size_t)img * R) * C1 + c;
+        for (int r = n + tid; r < R; r += 256) hc[(size_t)r * C1] = 0.f;
+    }
 }
 
 }  // namespace
@@ -163,24 +171,26 @@ CIM_API size_t cim_score_heads_workspace_bytes(int n_img, int R, int D, int C1, 
     return cim_score_tc_workspace_bytes(D, C1, K);          // W_hi / W_lo of the tensor-core path
 }
 
-CIM_API int cim_score_heads(const float *x, const float *weight, const float *bias, float *scores, int n_img,
-                            int R, int D, int C1, int K, void *workspace, size_t ws_bytes, cim_stream_t stream) {
+CIM_API int cim_score_heads_ex(const float *x, const float *weight, const float *bias, float *scores,
+                               const int32_t *n_props, int n_img, int R, int D, int C1, int K, void *workspace,
+                               size_t ws_bytes, cim_stream_t stream) {
     if (!x || !weight || !bias || !scores) return CIM_ERR_ARG;
     if (n_img < 0 || R < 0 || D <= 0 || C1 <= 0 || K < 0 || K > 8) return CIM_ERR_ARG;
     if (n_img == 0 || R == 0) return CIM_OK;
-    if (!cim_aligned(x, 16) || !cim_aligned(weight, 16)) return CIM_ERR_ALIGN;
+    if (!cim_aligned(x, 16) || !cim_aligned(weight, 16) || !cim_aligned(n_props, 4)) return CIM_ERR_ALIGN;
     if (n_img > 65535 || C1 > 65535) return CIM_ERR_SHAPE;
     cudaStream_t st = (cudaStream_t)stream;
     const long long M = (long long)n_img * R;
     if (M > (1LL << 30)) return CIM_ERR_SHAPE;
     const int nheads = 2 + 2 * K, N = nheads * C1;
+    const dim3 col_grid((unsigned)C1, (unsigned)n_img);
     // tensor cores (3xTF32, fp32-accurate) when the shape allows and the caller gave the workspace;
     // CIM_DBG_SCORE_FFMA forces the FFMA kernel (tuning / A-B aid)
     if (!(cim_get_debug_flags() & CIM_DBG_SCORE_FFMA) && cim_score_tc_eligible(M, D, C1, K) && workspace &&
         ws_bytes >= cim_score_tc_workspace_bytes(D, C1, K)) {
         int rc2 = cim_score_tc_launch(x, weight, bias, scores, M, D, C1, K, workspace, st);
         if (rc2) return rc2;
-        score_col_softmax_kernel<<<dim3((unsigned)C1, (unsigned)n_img), 256, 0, st>>>(scores + (size_t)M * C1, R, C1);
+        score_col_softmax_kernel<<<col_grid, 256, 0, st>>>(scores, n_props, M, nheads, R, C1);
         return cim_launch_status();
     }
     dim3 grid((unsigned)((M + BM - 1) / BM), (unsigned)((N + BN - 1) / BN));
@@ -190,6 +200,11 @@ CIM_API int cim_score_heads(const float *x, const float *weight, const float *bi
     const long long rows = (long long)nheads * M;
     score_row_act_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(scores, (int)M, C1, K);
     if ((rc = cim_launch_status())) return rc;
-    score_col_softmax_kernel<<<dim3((unsigned)C1, (unsigned)n_img), 256, 0, st>>>(scores + (size_t)M * C1, R, C1);
+    score_col_softmax_kernel<<<col_grid, 256, 0, st>>>(scores, n_props, M, nheads, R, C1);
     return cim_launch_status();
+}
+
+CIM_API int cim_score_heads(const float *x, const float *weight, const float *bias, float *scores, int n_img,
+                            int R, int D, int C1, int K, void *workspace, size_t ws_bytes, cim_stream_t stream) {
+    return cim_score_heads_ex(x, weight, bias, scores, nullptr, n_img, R, D, C1, K, workspace, ws_bytes, stream);
 }

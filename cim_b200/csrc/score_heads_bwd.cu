@@ -49,14 +49,21 @@ __device__ __forceinline__ uint32_t tf32_idesc(int n) {       // F32 accumulate,
 }
 
 // ------------------------------------------------------------------------------- activations
-// detector head: dot[img][c] = sum_r g[r][c] * y[r][c] over the proposals of one image (fixed order)
+// image row count n_props[img] clamped to [1, R]; R when n_props is NULL
+__device__ __forceinline__ int image_rows(const int32_t *n_props, int img, int R) {
+    return n_props ? min(max(n_props[img], 1), R) : R;
+}
+
+// detector head: dot[img][c] = sum_r g[r][c] * y[r][c] over the n proposals of one image (fixed order)
 __global__ void __launch_bounds__(256)
-score_det_dot_kernel(const float *__restrict__ g, const float *__restrict__ y, float *__restrict__ dot, int R, int C1) {
+score_det_dot_kernel(const float *__restrict__ g, const float *__restrict__ y, const int32_t *__restrict__ n_props,
+                     float *__restrict__ dot, int R, int C1) {
     __shared__ float red[256];
     const int c = blockIdx.x, img = blockIdx.y, tid = threadIdx.x;
     const size_t base = (size_t)img * R * C1 + c;
+    const int n = image_rows(n_props, img, R);
     float s = 0.f;
-    for (int r = tid; r < R; r += 256) s = fmaf(g[base + (size_t)r * C1], y[base + (size_t)r * C1], s);
+    for (int r = tid; r < n; r += 256) s = fmaf(g[base + (size_t)r * C1], y[base + (size_t)r * C1], s);
     red[tid] = s;
     __syncthreads();
     for (int o = 128; o > 0; o >>= 1) {
@@ -69,10 +76,11 @@ score_det_dot_kernel(const float *__restrict__ g, const float *__restrict__ y, f
 // dz for 32 proposals x one head per warp (lane = proposal), written hi/lo-split as dz [M][NP] (row = proposal) and
 // dz^T [N][MP].  The warp parks its 32 x C1 values in a private smem tile so that both layouts leave in contiguous
 // runs: dz rows in C1-float runs, dz^T rows as 128 B (32 proposals) per class -- one thread per (head, row) writing
-// its row with a 768-byte stride took 57 us at cfg2 for 43 MB.
+// its row with a 768-byte stride took 57 us at cfg2 for 43 MB.  Padding rows (r >= n of their image) get dz = 0
+// whatever grad_scores holds there, so their grad_x rows and their share of grad_W / grad_b are 0.
 __global__ void __launch_bounds__(256)
 score_act_bwd_kernel(const float *__restrict__ y_all, const float *__restrict__ g_all,
-                     const float *__restrict__ det_dot, float *__restrict__ dz_hi, float *__restrict__ dz_lo,
+                     const float *__restrict__ det_dot, const int32_t *__restrict__ n_props, float *__restrict__ dz_hi, float *__restrict__ dz_lo,
                      float *__restrict__ dzT_hi, float *__restrict__ dzT_lo, int M, int R, int C1, int K, int NP,
                      long long MP) {
     extern __shared__ float act_smem[];
@@ -90,11 +98,14 @@ score_act_bwd_kernel(const float *__restrict__ y_all, const float *__restrict__ 
             const bool row_softmax = (h == 0) || (h >= 2 && h < 2 + K);
             if (row_softmax)
                 for (int c = 0; c < C1; ++c) dot = fmaf(g[c], y[c], dot);
-            const float *ddot = det_dot + (size_t)(m / R) * C1;
+            const int img = m / R;
+            const float *ddot = det_dot + (size_t)img * C1;
+            const bool pad = m - img * R >= image_rows(n_props, img, R);
             for (int c = 0; c < C1; ++c) {
                 const float yy = y[c], gg = g[c];
                 float v;
-                if (row_softmax) v = yy * (gg - dot);
+                if (pad) v = 0.f;
+                else if (row_softmax) v = yy * (gg - dot);
                 else if (h == 1) v = yy * (gg - ddot[c]);
                 else v = gg * yy * (1.f - yy);
                 tile[lane * pitch + c] = v;
@@ -520,9 +531,10 @@ CIM_API size_t cim_score_heads_bwd_workspace_bytes(int n_img, int R, int D, int 
     return bwd_layout(n_img, R, D, C1, K).total;
 }
 
-CIM_API int cim_score_heads_bwd(const float *x, const float *weight, const float *scores, const float *grad_scores,
-                                float *grad_x, float *grad_weight, float *grad_bias, int n_img, int R, int D, int C1,
-                                int K, void *workspace, size_t ws_bytes, cim_stream_t stream) {
+CIM_API int cim_score_heads_bwd_ex(const float *x, const float *weight, const float *scores, const float *grad_scores,
+                                   const int32_t *n_props, float *grad_x, float *grad_weight, float *grad_bias,
+                                   int n_img, int R, int D, int C1, int K, void *workspace, size_t ws_bytes,
+                                   cim_stream_t stream) {
     if (!x || !weight || !scores || !grad_scores || !workspace) return CIM_ERR_ARG;
     if (n_img < 0 || R < 0 || D <= 0 || C1 <= 0 || K < 0 || K > 8) return CIM_ERR_ARG;
     if (!grad_x && !grad_weight && !grad_bias) return CIM_OK;
@@ -537,7 +549,9 @@ CIM_API int cim_score_heads_bwd(const float *x, const float *weight, const float
     const BwdLayout L = bwd_layout(n_img, R, D, C1, K);
     if (L.M > (1LL << 30)) return CIM_ERR_SHAPE;
     if (ws_bytes < L.total) return CIM_ERR_WORKSPACE;
-    if (!cim_aligned(x, 16) || !cim_aligned(weight, 16) || (grad_x && !cim_aligned(grad_x, 16))) return CIM_ERR_ALIGN;
+    if (!cim_aligned(x, 16) || !cim_aligned(weight, 16) || (grad_x && !cim_aligned(grad_x, 16)) ||
+        !cim_aligned(n_props, 4))
+        return CIM_ERR_ALIGN;
     unsigned char *ws = reinterpret_cast<unsigned char *>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
     auto F = [&](size_t off) { return reinterpret_cast<float *>(ws + off - 256); };
     float *dot = F(L.off_dot), *dzh = F(L.off_dzh), *dzl = F(L.off_dzl), *dth = F(L.off_dth), *dtl = F(L.off_dtl);
@@ -546,7 +560,7 @@ CIM_API int cim_score_heads_bwd(const float *x, const float *weight, const float
     const bool want_t = grad_weight || grad_bias;
 
     score_det_dot_kernel<<<dim3((unsigned)C1, (unsigned)n_img), 256, 0, st>>>(grad_scores + (size_t)M * C1,
-                                                                             scores + (size_t)M * C1, dot, R, C1);
+                                                                             scores + (size_t)M * C1, n_props, dot, R, C1);
     int rc = cim_launch_status();
     if (rc) return rc;
     const long long rows = (long long)nheads * M;
@@ -556,7 +570,7 @@ CIM_API int cim_score_heads_bwd(const float *x, const float *weight, const float
     if (act_smem > (size_t)cim_max_smem_optin()) return CIM_ERR_SHAPE;         // C1 > ~1700
     if (act_smem > 48 * 1024)
         cudaFuncSetAttribute(score_act_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)act_smem);
-    score_act_bwd_kernel<<<(unsigned)((M + 31) / 32), act_warps * 32, act_smem, st>>>(scores, grad_scores, dot, grad_x ? dzh : nullptr,
+    score_act_bwd_kernel<<<(unsigned)((M + 31) / 32), act_warps * 32, act_smem, st>>>(scores, grad_scores, dot, n_props, grad_x ? dzh : nullptr,
                                                                         dzl, want_t ? dth : nullptr, dtl, M, R, C1, K,
                                                                         L.NP, L.MP);
     if ((rc = cim_launch_status())) return rc;
@@ -607,4 +621,11 @@ CIM_API int cim_score_heads_bwd(const float *x, const float *weight, const float
         if ((rc = cim_launch_status())) return rc;
     }
     return CIM_OK;
+}
+
+CIM_API int cim_score_heads_bwd(const float *x, const float *weight, const float *scores, const float *grad_scores,
+                                float *grad_x, float *grad_weight, float *grad_bias, int n_img, int R, int D, int C1,
+                                int K, void *workspace, size_t ws_bytes, cim_stream_t stream) {
+    return cim_score_heads_bwd_ex(x, weight, scores, grad_scores, nullptr, grad_x, grad_weight, grad_bias, n_img, R, D,
+                                  C1, K, workspace, ws_bytes, stream);
 }

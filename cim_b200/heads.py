@@ -32,10 +32,12 @@ from . import _lib
 
 # ------------------------------------------------------------------------------- scoring
 class ScoreHeadsFunction(Function):
-    """scores[h] = act_h(x @ W_h^T + b_h) for the 2+2K heads; see cim_score_heads in cimhead.h."""
+    """scores[h] = act_h(x @ W_h^T + b_h) for the 2+2K heads; see cim_score_heads in cimhead.h.
+    n_props (optional): proposals per image of a ragged batch (_lib.n_props_arg); image b owns rows [0, n_b) of its R
+    rows, the detector softmax runs over those and every head is 0 on the others (cim_score_heads_ex)."""
 
     @staticmethod
-    def forward(ctx, x, weight, bias, n_img, k):
+    def forward(ctx, x, weight, bias, n_img, k, n_props=None):
         _lib.require_cuda(x, "seg_feature", torch.float32)
         _lib.require_cuda(weight, "weight", torch.float32)
         _lib.require_cuda(bias, "bias", torch.float32)
@@ -46,14 +48,16 @@ class ScoreHeadsFunction(Function):
             raise ValueError("rows of seg_feature must be n_img * R")
         L = _lib.lib()
         with torch.cuda.device(x.device):
+            n_props = _lib.n_props_arg(n_props, n_img, m // n_img, x.device)
             scores = torch.empty((nh, m, c1), dtype=torch.float32, device=x.device)
             ws = torch.empty(L.cim_score_heads_workspace_bytes(n_img, m // n_img, d, c1, k), dtype=torch.uint8,
                              device=x.device)
-            rc = L.cim_score_heads(_lib.ptr(x), _lib.ptr(weight), _lib.ptr(bias), _lib.ptr(scores), n_img,
-                                   m // n_img, d, c1, k, _lib.ptr(ws), ws.numel(), _lib.stream_ptr(x.device))
+            rc = L.cim_score_heads_ex(_lib.ptr(x), _lib.ptr(weight), _lib.ptr(bias), _lib.ptr(scores),
+                                      _lib.ptr(n_props), n_img, m // n_img, d, c1, k, _lib.ptr(ws), ws.numel(),
+                                      _lib.stream_ptr(x.device))
         _lib.check(rc, "cim_score_heads")
         ctx.save_for_backward(x, weight, scores)
-        ctx.cfg = (n_img, k)
+        ctx.cfg = (n_img, k, n_props)
         return scores
 
     @staticmethod
@@ -62,7 +66,7 @@ class ScoreHeadsFunction(Function):
         """cim_score_heads_bwd: activation backward + grad_x / grad_weight / grad_bias in one call
         (autograd of heads.py:194-219)."""
         x, weight, s = ctx.saved_tensors
-        n_img, k = ctx.cfg
+        n_img, k, n_props = ctx.cfg
         nh, m, c1 = s.shape
         d = x.shape[1]
         grad = _lib.require_cuda(grad, "grad_scores", torch.float32).contiguous()
@@ -74,11 +78,11 @@ class ScoreHeadsFunction(Function):
             gb = torch.empty((nh, c1), dtype=torch.float32, device=x.device) if need_b else None
             ws = torch.empty(L.cim_score_heads_bwd_workspace_bytes(n_img, m // n_img, d, c1, k), dtype=torch.uint8,
                              device=x.device)
-            rc = L.cim_score_heads_bwd(_lib.ptr(x), _lib.ptr(weight), _lib.ptr(s), _lib.ptr(grad), _lib.ptr(gx),
-                                       _lib.ptr(gw), _lib.ptr(gb), n_img, m // n_img, d, c1, k, _lib.ptr(ws),
-                                       ws.numel(), _lib.stream_ptr(x.device))
+            rc = L.cim_score_heads_bwd_ex(_lib.ptr(x), _lib.ptr(weight), _lib.ptr(s), _lib.ptr(grad),
+                                          _lib.ptr(n_props), _lib.ptr(gx), _lib.ptr(gw), _lib.ptr(gb), n_img, m // n_img,
+                                          d, c1, k, _lib.ptr(ws), ws.numel(), _lib.stream_ptr(x.device))
         _lib.check(rc, "cim_score_heads_bwd")
-        return gx, gw, gb, None, None
+        return gx, gw, gb, None, None, None
 
 
 class cls_iou_model(nn.Module):
@@ -98,12 +102,13 @@ class cls_iou_model(nn.Module):
         layers = [self.classifier, self.detector, *self.refine_cls, *self.refine_iou]
         return torch.stack([l.weight for l in layers]), torch.stack([l.bias for l in layers])
 
-    def forward_batched(self, seg_feature, n_img=1):
-        """seg_feature [n_img*R, D] -> scores [2+2K, n_img*R, C1] (detector softmax per image)."""
+    def forward_batched(self, seg_feature, n_img=1, n_props=None):
+        """seg_feature [n_img*R, D] -> scores [2+2K, n_img*R, C1] (detector softmax per image).  n_props: proposals
+        per image of a ragged batch (R is then a capacity; see ScoreHeadsFunction)."""
         if seg_feature.dim() == 4:
             seg_feature = seg_feature.squeeze(3).squeeze(2)
         weight, bias = self._stacked()
-        return ScoreHeadsFunction.apply(seg_feature, weight, bias, n_img, len(self.refine_cls))
+        return ScoreHeadsFunction.apply(seg_feature, weight, bias, n_img, len(self.refine_cls), n_props)
 
     def forward(self, seg_feature):
         k = len(self.refine_cls)
@@ -248,7 +253,7 @@ def anti_noise_device(p, labels, gt_count, gt_class, gt_weight, gt_keep, stream=
 
 
 def mine_and_assign(cls_scores, det_scores, labels, iou_map, asy_iou_map, cls_thr, iou_thr, p_seed=0.1,
-                    con_thr=0.85, anti_noise_sampling=True, using_cim=True):
+                    con_thr=0.85, anti_noise_sampling=True, using_cim=True, n_props=None):
     """All images x all refinement layers of CIM_layer.forward in two device phases.
 
     cls_scores / det_scores: lists (one per layer) of [n_img, R, C1] float32 CUDA tensors -- layer 0
@@ -257,7 +262,10 @@ def mine_and_assign(cls_scores, det_scores, labels, iou_map, asy_iou_map, cls_th
     cls_thr / iou_thr: per-layer thresholds (model_builder.py:90-93).
     Returns dict(pseudo_labels [L,n_img,R,C+1] f32, pseudo_iou_labels [L,n_img,R] f16,
     loss_weights [L,n_img,R] f32, valid [L,n_img] uint8 (0 where the reference returns None),
-    asy_iou_flag [n_img,R] uint8, gt_count [L,n_img] int32)."""
+    asy_iou_flag [n_img,R] uint8, gt_count [L,n_img] int32).
+    n_props: proposals per image of a ragged batch (_lib.n_props_arg).  Image b is then mined from rows [0, n_b) as
+    if it were alone at R = n_b (keep_count and the big-proposal threshold from n_b, the same numpy stream); its rows
+    >= n_b get the ignore row and asy_iou_flag 0, and the maps' rows and columns >= n_b are never read."""
     n_layers = len(cls_scores)
     if n_layers < 1 or n_layers > _lib.MAX_LAYERS:
         raise ValueError(f"1..{_lib.MAX_LAYERS} layers supported")
@@ -287,13 +295,14 @@ def mine_and_assign(cls_scores, det_scores, labels, iou_map, asy_iou_map, cls_th
     p.det_cols = det_scores[0].shape[-1] if det_scores is not None else c1
     p.gt_cap = R
     p.mode = 0 if using_cim else 1
-    p.keep_count = int(np.ceil(p_seed * R))                      # heads.py:332
+    p.keep_count = int(np.ceil(p_seed * R))                      # heads.py:332 (with n_props: the capacity)
     p.big_thr = float(np.float32(0.9 * R))                       # heads.py:338
     p.con_thr = con_thr
     for l in range(n_layers):
         p.cls_thr[l], p.iou_thr[l] = cls_thr[l], iou_thr[l]
 
     L = _lib.lib()
+    n_props = _lib.n_props_arg(n_props, n_img, R, dev)
     PtrArr = C.c_void_p * n_layers
     cls_ptrs = PtrArr(*[t.data_ptr() for t in cls_scores])
     det_ptrs = PtrArr(*[t.data_ptr() for t in det_scores]) if det_scores is not None else None
@@ -305,9 +314,11 @@ def mine_and_assign(cls_scores, det_scores, labels, iou_map, asy_iou_map, cls_th
         gt_class = torch.empty((n_layers, n_img, R), dtype=torch.int32, device=dev)
         gt_weight = torch.empty((n_layers, n_img, R), dtype=torch.float32, device=dev)
         asy_flag = torch.ones((n_img, R), dtype=torch.uint8, device=dev)
-        rc = L.cim_mine(C.byref(p), cls_ptrs, det_ptrs, _lib.ptr(labels), _lib.ptr(iou_map),
-                        _lib.ptr(asy_iou_map), _lib.ptr(gt_count), _lib.ptr(gt_rows), _lib.ptr(gt_class),
-                        _lib.ptr(gt_weight), _lib.ptr(asy_flag), _lib.ptr(ws), ws.numel(), st)
+        if n_props is not None and asy_iou_map is None:
+            asy_flag[:, :] = (torch.arange(R, device=dev) < n_props[:, None]).to(torch.uint8)
+        rc = L.cim_mine_ex(C.byref(p), _lib.ptr(n_props), float(p_seed), cls_ptrs, det_ptrs, _lib.ptr(labels),
+                           _lib.ptr(iou_map), _lib.ptr(asy_iou_map), _lib.ptr(gt_count), _lib.ptr(gt_rows),
+                           _lib.ptr(gt_class), _lib.ptr(gt_weight), _lib.ptr(asy_flag), _lib.ptr(ws), ws.numel(), st)
         _lib.check(rc, "cim_mine")
 
         gt_keep = None
@@ -319,9 +330,9 @@ def mine_and_assign(cls_scores, det_scores, labels, iou_map, asy_iou_map, cls_th
         pseudo_iou = torch.empty((n_layers, n_img, R), dtype=torch.float16, device=dev)
         loss_weights = torch.empty((n_layers, n_img, R), dtype=torch.float32, device=dev)
         valid = torch.empty((n_layers, n_img), dtype=torch.uint8, device=dev)
-        rc = L.cim_assign(C.byref(p), _lib.ptr(iou_map), _lib.ptr(gt_count), _lib.ptr(gt_rows),
-                          _lib.ptr(gt_class), _lib.ptr(gt_weight), _lib.ptr(gt_keep), _lib.ptr(pseudo_labels),
-                          _lib.ptr(pseudo_iou), _lib.ptr(loss_weights), _lib.ptr(valid), st)
+        rc = L.cim_assign_ex(C.byref(p), _lib.ptr(n_props), _lib.ptr(iou_map), _lib.ptr(gt_count), _lib.ptr(gt_rows),
+                             _lib.ptr(gt_class), _lib.ptr(gt_weight), _lib.ptr(gt_keep), _lib.ptr(pseudo_labels),
+                             _lib.ptr(pseudo_iou), _lib.ptr(loss_weights), _lib.ptr(valid), st)
         _lib.check(rc, "cim_assign")
     return dict(pseudo_labels=pseudo_labels, pseudo_iou_labels=pseudo_iou, loss_weights=loss_weights,
                 valid=valid, asy_iou_flag=asy_flag, gt_count=gt_count, gt_rows=gt_rows, gt_class=gt_class,
@@ -413,7 +424,7 @@ class PCLLossFunction(Function):
     """cim_pcl_loss: heads.PCL_loss (heads.py:10-41) forward + backward in one launch, n_img images at once."""
 
     @staticmethod
-    def forward(ctx, predict_cls, mat, n_img, max_id):
+    def forward(ctx, predict_cls, mat, n_img, max_id, n_props=None):
         _lib.require_cuda(predict_cls, "predict_cls", torch.float32)
         _lib.require_cuda(mat, "mat", torch.float32)
         predict_cls, mat = predict_cls.contiguous(), mat.contiguous()
@@ -422,10 +433,12 @@ class PCLLossFunction(Function):
         if mat.numel() != m * c1 or m % n_img:
             raise ValueError("mat must be [n_img, R, C+1] matching predict_cls [n_img*R, C+1]")
         with torch.cuda.device(predict_cls.device):
+            n_props = _lib.n_props_arg(n_props, n_img, R, predict_cls.device)
             loss = torch.empty((n_img,), dtype=torch.float32, device=predict_cls.device)
             grad = torch.empty_like(predict_cls)
-            rc = _lib.lib().cim_pcl_loss(_lib.ptr(predict_cls), _lib.ptr(mat), _lib.ptr(loss), _lib.ptr(grad), n_img, R,
-                                         c1, int(max_id), 1.0, 0, _lib.stream_ptr(predict_cls.device))
+            rc = _lib.lib().cim_pcl_loss_ex(_lib.ptr(predict_cls), _lib.ptr(mat), _lib.ptr(n_props), _lib.ptr(loss),
+                                            _lib.ptr(grad), n_img, R, c1, int(max_id), 1.0, 0,
+                                            _lib.stream_ptr(predict_cls.device))
         _lib.check(rc, "cim_pcl_loss")
         ctx.save_for_backward(grad)
         ctx.shape = (n_img, R)
@@ -436,20 +449,21 @@ class PCLLossFunction(Function):
     def backward(ctx, g):
         (grad,) = ctx.saved_tensors
         n_img, R = ctx.shape
-        return (grad.view(n_img, R, -1) * g.view(n_img, 1, 1)).view_as(grad), None, None, None
+        return (grad.view(n_img, R, -1) * g.view(n_img, 1, 1)).view_as(grad), None, None, None, None
 
 
 #: cluster ids cim_pcl_loss accepts (its per-row id lists hold 8-bit ids); CIMHeadStep passes the same constant
 PCL_MAX_ID = 255
 
 
-def PCL_loss(predict_cls, mat, labels=None, n_img=1, max_id=PCL_MAX_ID, strict=False):
+def PCL_loss(predict_cls, mat, labels=None, n_img=1, max_id=PCL_MAX_ID, strict=False, n_props=None):
     """heads.PCL_loss(predict_cls, mat, labels) (heads.py:10-41; `labels` only supplied the device there).
     n_img = 1 returns a 0-d loss like the reference; n_img > 1 (predict_cls [n_img*R, C+1], mat [n_img, R, C+1])
     returns one loss per image.  A cluster matrix the kernel cannot take (an id above max_id, a non-integer id, more
     than four distinct ids in a row, two background ids -- the reference asserts on the last) gives a NaN loss and a
-    zero gradient for that image; strict=True turns that into a RuntimeError (one host sync)."""
-    loss = PCLLossFunction.apply(predict_cls, mat, n_img, max_id)
+    zero gradient for that image; strict=True turns that into a RuntimeError (one host sync).  n_props: proposals per
+    image of a ragged batch (_lib.n_props_arg); rows r >= n_b of an image join no cluster whatever mat holds there."""
+    loss = PCLLossFunction.apply(predict_cls, mat, n_img, max_id, n_props)
     if strict and bool(torch.isnan(loss.detach()).any()):
         raise RuntimeError("cim_pcl_loss: cluster matrix outside what the kernel supports (ids must be integers in "
                            f"[0, {max_id}], at most 4 distinct ids per row, one background id), or NaN scores")

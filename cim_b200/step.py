@@ -70,6 +70,8 @@ class CIMHeadStep:
         self.kb_per_row = int(mask_kb_per_row)
         self.sr, self.aligned = int(sampling_ratio), int(bool(aligned))
         self.anti = anti_noise_sampling
+        self.p_seed = float(p_seed)
+        self.n_props = None             # the device counts of the last run(): kept alive while its kernels may run
         self.order = order
         if rng not in ("hop", "stream"):
             raise ValueError("rng must be 'hop' or 'stream'")
@@ -105,7 +107,7 @@ class CIMHeadStep:
             p = _lib.MineParams()
             p.n_img, p.R, p.C, p.C1, p.n_layers = n_img, R, n_classes, C1, k
             p.det_cols, p.mode = C1, 0
-            p.keep_count = int(np.ceil(p_seed * R))                 # heads.py:332
+            p.keep_count = int(np.ceil(p_seed * R))                 # heads.py:332; the capacity for ragged batches
             # the pseudo-GT lists stay on the device (the sampling runs there, cim_anti_noise), so they get the full
             # capacity R: no overflow whatever the number of present classes (max_present is accepted and ignored)
             gcap = R
@@ -165,7 +167,7 @@ class CIMHeadStep:
 
     # -------------------------------------------------------------------------------------
     def run(self, feat, rois, grad_out, packed_masks, seg_x, weight, bias, labels, labels_host=None, grad_scores=None,
-            mat=None, mid_hook=None, order=None, mask_meta=None):
+            mat=None, mid_hook=None, order=None, mask_meta=None, n_props=None):
         """feat [n_img,Cf,H,W] f32, rois [n_img*R,5] f32 grouped by image, grad_out [n_img*R,Cf,7,7]
         f32, packed_masks [n_img,R,words] i32, seg_x [n_img*R,D] f32, weight [2+2K,C+1,D],
         bias [2+2K,C+1], labels [n_img,C] f32 (labels_host is no longer needed: the sampling runs on the device).
@@ -177,6 +179,12 @@ class CIMHeadStep:
         matrix, model_builder.py:125,203) adds PCL_loss: pcl_loss [n_img] and its gradient on the classifier head.
         mask_meta: mask_ops.mask_meta(packed_masks), produced with the masks (data-set packing / input prefetch): the
         overlap stage then skips its own pass over the 524 MB of packed masks.
+        n_props: proposals per image of a ragged batch (a host sequence / CPU tensor, validated and copied, or a CUDA
+        int32 [n_img] tensor used as is; it may change from step to step).  R is then a capacity: image b owns rows
+        [0, n_b) of its R rows, and every result of image b equals that of the image run alone at R = n_b (scores,
+        pseudo labels, losses, PCL_loss, gradients; padding rows of all of them are 0).  Padding rows must hold finite
+        seg_x, rois with the image's own index and finite coordinates, and grad_out rows of 0; the maps are computed
+        for them but never read.  None: every image has R proposals.
 
         order (default: the constructor's):
           "graph"      the model's dependency order (model_builder.py:136-204): RoIAlign forward -> scoring heads ->
@@ -201,18 +209,20 @@ class CIMHeadStep:
         ck = _lib.check
         cur = torch.cuda.current_stream(dev)
         pcl_early = self.head_grads and grad_scores is None and mat is not None
+        self.n_props = np_dev = _lib.n_props_arg(n_props, n_img, R, dev)
 
         def pcl(stream):
             # PCL_loss (model_builder.py:203) needs predict_cls and the cluster matrix only: 8 CTAs of pure latency;
             # its gradient is added to head 0's after the loss block
             with _nvtx("cim/pcl_loss"):
-                ck(L.cim_pcl_loss(P(self.scores), P(mat), P(self.pcl_loss), P(self.pcl_grad), n_img, R,
-                                  self.C + 1, PCL_MAX_ID, 1.0 / n_img, 0, stream), "cim_pcl_loss")
+                ck(L.cim_pcl_loss_ex(P(self.scores), P(mat), P(np_dev), P(self.pcl_loss), P(self.pcl_grad), n_img, R,
+                                     self.C + 1, PCL_MAX_ID, 1.0 / n_img, 0, stream), "cim_pcl_loss")
 
         def score_fwd(stream, with_pcl):
             with _nvtx("cim/score_heads"):
-                ck(L.cim_score_heads(P(seg_x), P(weight), P(bias), P(self.scores), n_img, R, self.D, self.C + 1, k,
-                                     P(self.score_ws), self.score_ws.numel(), stream), "cim_score_heads")
+                ck(L.cim_score_heads_ex(P(seg_x), P(weight), P(bias), P(self.scores), P(np_dev), n_img, R, self.D,
+                                        self.C + 1, k, P(self.score_ws), self.score_ws.numel(), stream),
+                   "cim_score_heads")
             if with_pcl and pcl_early:
                 pcl(stream)
 
@@ -231,9 +241,10 @@ class CIMHeadStep:
         def mine():
             self.ev_premine.record(cur)        # from here on the GPU is mostly idle until the hop is over
             with _nvtx("cim/mine"):
-                ck(L.cim_mine(C.byref(p), self.cls_ptrs, self.det_ptrs, P(labels), P(self.iou), P(self.asy),
-                              P(self.gt_count), P(self.gt_rows), P(self.gt_class), P(self.gt_weight),
-                              P(self.asy_flag), P(self.mine_ws), self.mine_ws.numel(), st), "cim_mine")
+                ck(L.cim_mine_ex(C.byref(p), P(np_dev), self.p_seed, self.cls_ptrs, self.det_ptrs, P(labels),
+                                 P(self.iou), P(self.asy), P(self.gt_count), P(self.gt_rows), P(self.gt_class),
+                                 P(self.gt_weight), P(self.asy_flag), P(self.mine_ws), self.mine_ws.numel(), st),
+                   "cim_mine")
                 if self.anti and self.rng == "stream":
                     hbuf, hev = self._cnt_slots[self._cnt_next]
                     self._cnt_next = (self._cnt_next + 1) % len(self._cnt_slots)
@@ -314,9 +325,9 @@ class CIMHeadStep:
             cur.wait_event(self.res_ev)                         # run_host: the previous step's results have been read
             self._res_guard = False
         with _nvtx("cim/assign"):
-            ck(L.cim_assign(C.byref(p), P(self.iou), P(self.gt_count), P(self.gt_rows), P(self.gt_class),
-                            P(self.gt_weight), P(keep), P(self.pseudo_labels), P(self.pseudo_iou),
-                            P(self.loss_weights), P(self.valid), st), "cim_assign")
+            ck(L.cim_assign_ex(C.byref(p), P(np_dev), P(self.iou), P(self.gt_count), P(self.gt_rows),
+                               P(self.gt_class), P(self.gt_weight), P(keep), P(self.pseudo_labels), P(self.pseudo_iou),
+                               P(self.loss_weights), P(self.valid), st), "cim_assign")
         reduce_work = None
         if self.head_grads:
             if grad_scores is None:
@@ -333,9 +344,10 @@ class CIMHeadStep:
                         self.grad_scores[0].add_(self.pcl_grad)
                 grad_scores = self.grad_scores
             with _nvtx("cim/score_heads_bwd"):
-                ck(L.cim_score_heads_bwd(P(seg_x), P(weight), P(self.scores), P(grad_scores), P(self.grad_seg_x),
-                                         P(self.grad_weight), P(self.grad_bias), n_img, R, self.D, self.C + 1, k,
-                                         P(self.score_bwd_ws), self.score_bwd_ws.numel(), st), "cim_score_heads_bwd")
+                ck(L.cim_score_heads_bwd_ex(P(seg_x), P(weight), P(self.scores), P(grad_scores), P(np_dev),
+                                            P(self.grad_seg_x), P(self.grad_weight), P(self.grad_bias), n_img, R,
+                                            self.D, self.C + 1, k, P(self.score_bwd_ws), self.score_bwd_ws.numel(),
+                                            st), "cim_score_heads_bwd")
                 reduce_work = cdist.allreduce_mean_async_(self.head_bucket)     # overlaps the RoIAlign backward
         with _nvtx("cim/roi_align_bwd"):
             ck(L.cim_roi_align_bwd_prepared(P(grad_out), P(rois), None, P(self.grad_feat), n_img, self.Cf, self.H,
@@ -612,7 +624,8 @@ class CIMHeadStep:
     def run_host(self, feat, grad_out, seg_x, weight, bias, prefetch_next=True, grad_scores=None, mat=None,
                  lag_results=False):
         """End-to-end step: host rois / labels / bit-packed masks -> device, the step, results ->
-        host.  feat / seg_x / grad_out are produced on the device by the backbone, MaskFuse and
+        host.  Every image has R proposals here (run() takes ragged batches; a ragged crop wire format, with empty
+        crops for the padding rows, is not implemented).  feat / seg_x / grad_out are produced on the device by the backbone, MaskFuse and
         autograd in the real pipeline and therefore stay device tensors.
         With prefetch_next the copy of the NEXT step's inputs (whatever is in the pinned input
         buffers now) is enqueued on the copy stream first, so it overlaps this step's kernels;

@@ -14,6 +14,25 @@
  *   - there is no CPU path.
  *
  * Each declaration cites the reference interface it replaces.
+ *
+ * Ragged batches (the _ex entry points of the scoring heads, mining, assignment and PCL_loss).  The images of a batch
+ * may have different proposal counts.  Tensors keep their shapes: R is a capacity, and image b owns rows [0, n_b) of
+ * its R rows, 0 < n_b <= R.  n_props is a device int32 [n_img] array of the n_b; NULL means n_b = R for every image,
+ * and each entry point without _ex is its NULL case.  The library cannot validate device-side counts: the kernels
+ * clamp every n_b to [1, R], so a count outside that range is well defined but not meaningful.  Contract:
+ *   - no result of image b depends on its padding rows r >= n_b: not on x there (which must still be finite: the
+ *     grad_weight product multiplies it by a zero dz, and 0 * NaN = NaN), not on the iou / asy map rows and columns
+ *     >= n_b (anything, NaN included), not on mat there, not on scores or grad_scores there;
+ *   - padding rows of the outputs are defined: every one of the 2+2K score heads is 0 (so cim_test_scores gives 0 and
+ *     the test-time NMS, score > 1e-5, never takes a padding row), pseudo labels / pseudo IoU / loss weights are 0
+ *     (the ignore row), asy_flag is 0, grad_x and the PCL gradient are exactly 0; cim_head_losses, fed those zeros,
+ *     writes exactly 0 into grad_scores there;
+ *   - every per-image quantity is computed for n_b, as running that image alone at R = n_b would: the detector
+ *     softmax over its n_b proposals, keep_count = int(ceil(p_seed * n_b)) and big_thr = float32(0.9 * n_b)
+ *     (cim_mine_image_constants), the containment counts over its n_b columns.
+ * RoIAlign and the mask overlap maps have no _ex form: their padding rows are computed and nobody reads them.  Give
+ * padding rois their own image index and finite coordinates, and grad_out rows of 0 at padding (what the scoring
+ * backward's zero grad_x rows produce through a per-ROI head).  Zero padding masks let the overlap kernel skip them.
  */
 #ifndef CIMHEAD_H
 #define CIMHEAD_H
@@ -27,7 +46,7 @@ extern "C" {
 
 typedef struct CUstream_st *cim_stream_t;   /* == cudaStream_t */
 
-#define CIM_ABI_VERSION 3
+#define CIM_ABI_VERSION 4
 
 enum {
     CIM_OK = 0,
@@ -253,6 +272,11 @@ size_t cim_score_heads_workspace_bytes(int n_img, int R, int D, int C1, int K);
 int cim_score_heads(const float *x, const float *weight, const float *bias, float *scores,
                     int n_img, int R, int D, int C1, int K,
                     void *workspace, size_t workspace_bytes, cim_stream_t stream);
+/* Ragged form (see the top of this file): the detector softmax runs over the n_b rows of each image and every head is
+ * 0 on its padding rows.  n_props 4-byte aligned. */
+int cim_score_heads_ex(const float *x, const float *weight, const float *bias, float *scores, const int32_t *n_props,
+                       int n_img, int R, int D, int C1, int K,
+                       void *workspace, size_t workspace_bytes, cim_stream_t stream);
 
 /* Backward of cim_score_heads = autograd of heads.cls_iou_model.forward (lib/modeling/heads.py:194-219; the
  * reference gets it from eight nn.Linear backward calls + softmax / sigmoid backward, run by loss.backward(),
@@ -273,6 +297,12 @@ int cim_score_heads_bwd(const float *x, const float *weight, const float *scores
                         float *grad_x, float *grad_weight, float *grad_bias,
                         int n_img, int R, int D, int C1, int K,
                         void *workspace, size_t workspace_bytes, cim_stream_t stream);
+/* Ragged form: the detector's sum runs over the n_b rows of each image, and dz = 0 on padding rows whatever
+ * grad_scores holds there, so grad_x rows there are 0 and padding adds nothing to grad_weight / grad_bias. */
+int cim_score_heads_bwd_ex(const float *x, const float *weight, const float *scores, const float *grad_scores,
+                           const int32_t *n_props, float *grad_x, float *grad_weight, float *grad_bias,
+                           int n_img, int R, int D, int C1, int K,
+                           void *workspace, size_t workspace_bytes, cim_stream_t stream);
 
 /* ------------------------------------------------------------------ CIM mining + assignment
  * Replace heads.CIM_layer (lib/modeling/heads.py:222-503) for n_img images x n_layers
@@ -311,6 +341,18 @@ int cim_mine(const cim_mine_params *p, const float *const *cls, const float *con
              const float *labels /* [n_img, C] */, const void *iou_f16, const void *asy_f16,
              int32_t *gt_count, int32_t *gt_rows, int32_t *gt_class, float *gt_weight,
              uint8_t *asy_flag, void *workspace, size_t workspace_bytes, cim_stream_t stream);
+/* Ragged form: n_props == NULL is cim_mine (p->keep_count and p->big_thr are used, p_seed is ignored).  Otherwise
+ * every image gets keep_count and big_thr from its n_b and p_seed (0 < p_seed <= 1) as cim_mine_image_constants()
+ * computes them, p->big_thr is ignored, and p->keep_count is the capacity the workspace is sized for: it must be at
+ * least the keep_count of n_b = R (CIM_ERR_ARG otherwise). */
+int cim_mine_ex(const cim_mine_params *p, const int32_t *n_props, double p_seed, const float *const *cls,
+                const float *const *det, const float *labels, const void *iou_f16, const void *asy_f16,
+                int32_t *gt_count, int32_t *gt_rows, int32_t *gt_class, float *gt_weight, uint8_t *asy_flag,
+                void *workspace, size_t workspace_bytes, cim_stream_t stream);
+/* Host memory only, no GPU needed: the per-image constants of cim_mine_ex for an image of n proposals, computed by the
+ * same code the kernels run.  keep_count = int(ceil(p_seed * n)) (heads.py:332), big_thr = float32(0.9 * n)
+ * (heads.py:338), both from one float64 product rounded to nearest.  n >= 1, 0 < p_seed <= 1, else CIM_ERR_ARG. */
+int cim_mine_image_constants(double p_seed, int n, int *keep_count, float *big_thr);
 /* Anti-noise sampling between the phases ON THE DEVICE (heads.py:440-473): per (layer, image) list and present class,
  * np.random.choice(class_idx, size=n, replace=True, p=w / w.sum()) with numpy's arithmetic restated bit for bit
  * (float32 pairwise sum, float32 p, float64 cumsum normalised by its last element, searchsorted side='right'); the
@@ -341,6 +383,11 @@ int cim_assign(const cim_mine_params *p, const void *iou_f16,
                const float *gt_weight, const uint8_t *gt_keep /* may be NULL = keep all */,
                float *pseudo_labels, void *pseudo_iou_f16, float *loss_weights, uint8_t *valid,
                cim_stream_t stream);
+/* Ragged form: padding rows get the ignore row (pseudo labels, pseudo IoU and loss weight 0). */
+int cim_assign_ex(const cim_mine_params *p, const int32_t *n_props, const void *iou_f16,
+                  const int32_t *gt_count, const int32_t *gt_rows, const int32_t *gt_class,
+                  const float *gt_weight, const uint8_t *gt_keep, float *pseudo_labels, void *pseudo_iou_f16,
+                  float *loss_weights, uint8_t *valid, cim_stream_t stream);
 
 /* ------------------------------------------------------------------ loss block (forward + backward)
  * cim_head_losses: per image b and refinement layer l < n_layers with valid[l][b] != 0 (the reference skips a
@@ -374,6 +421,9 @@ int cim_head_losses(const float *scores, const float *pseudo_labels, const void 
  *   C1 <= 128, max_id <= 255, R <= 16384. */
 int cim_pcl_loss(const float *predict_cls, const float *mat, float *loss, float *grad_cls, int n_img, int R, int C1,
                  int max_id, float grad_scale, int accumulate, cim_stream_t stream);
+/* Ragged form: mat reads as 0 on padding rows, which join no cluster and get gradient 0 (added 0 with accumulate). */
+int cim_pcl_loss_ex(const float *predict_cls, const float *mat, const int32_t *n_props, float *loss, float *grad_cls,
+                    int n_img, int R, int C1, int max_id, float grad_scale, int accumulate, cim_stream_t stream);
 
 /* ------------------------------------------------------------------ test-time post-processing
  * cim_test_scores: lib/core/test.py:130-133 over lib/modeling/model_builder.py:60-68 -- the K refinement
