@@ -39,12 +39,14 @@ def overlap_counts(masks):
     return inter, area
 
 
-def maps_from_counts(inter, area):
+def maps_from_counts(inter, area, row_area=None):
     """(iou_fp16, asy_fp16) from integer counts with the reference's rounding chain:
-    python/numpy int / int -> float64, assignment into a float32 array, `.astype(float16)`."""
+    python/numpy int / int -> float64, assignment into a float32 array, `.astype(float16)`.
+    row_area: areas of the rows when inter holds only some rows of the map (default: area, a square map)."""
     inter = np.asarray(inter, dtype=np.int64)
     area = np.asarray(area, dtype=np.int64)
-    union = area[:, None] + area[None, :] - inter
+    row_area = area if row_area is None else np.asarray(row_area, dtype=np.int64)
+    union = row_area[:, None] + area[None, :] - inter
     with np.errstate(divide="ignore", invalid="ignore"):
         iou32 = (inter.astype(np.float64) / union.astype(np.float64)).astype(np.float32)
         asy32 = (inter.astype(np.float64) / area[None, :].astype(np.float64)).astype(np.float32)
