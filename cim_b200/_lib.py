@@ -13,7 +13,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libcimhead.so")
-ABI_VERSION = 4
+ABI_VERSION = 5
 MAX_LAYERS = 4
 OVERLAP_ALGOS = {"auto": 0, "popc": 1, "tensor": 2}
 #: cim_set_debug_flags bits (include/cimhead.h): diagnostic kernel selection for A/B timing and bit-identity tests
@@ -41,6 +41,7 @@ _SIGNATURES = {
     "cim_set_debug_flags": (None, [C.c_uint]),
     "cim_get_debug_flags": (C.c_uint, []),
     "cim_debug_roi_window_plan": (_I, [_P, _I, _I, _I, _I, _F, _I, _I, _P, _P, _I, _P, _P]),
+    "cim_debug_roi_window_plan_ex": (_I, [_P, _P, _I, _I, _I, _I, _F, _I, _I, _P, _P, _I, _P, _P]),
     "cim_roi_align_workspace_bytes": (_SZ, [_I]),
     "cim_roi_align_workspace_bytes_ex": (_SZ, [_I, _I, _I, _I, _I, _I, _I]),
     "cim_roi_align_fwd": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _F, _I, _I, _P, _SZ, _P]),
@@ -48,6 +49,9 @@ _SIGNATURES = {
     "cim_roi_align_prepare": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _F, _I, _I, _P, _SZ, _P]),
     "cim_roi_align_fwd_prepared": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _F, _I, _I, _P, _SZ, _P]),
     "cim_roi_align_bwd_prepared": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _F, _I, _I, _P, _SZ, _P]),
+    "cim_roi_align_prepare_ex": (_I, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _F, _I, _I, _P, _SZ, _P]),
+    "cim_roi_align_fwd_prepared_ex": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _F, _I, _I, _P, _SZ, _P]),
+    "cim_roi_align_bwd_prepared_ex": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _F, _I, _I, _P, _SZ, _P]),
     "cim_roi_align_maskfuse_fwd": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _F, _I, _I, _P, _SZ, _P]),
     "cim_roi_align_maskfuse_bwd": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _F, _I, _I, _P, _SZ, _P]),
     "cim_roi_pool_fwd": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _F, _P]),
@@ -172,6 +176,32 @@ def n_props_arg(n_props, n_img, R, device):
         raise ValueError(f"n_props must have shape [{n_img}], got {a.shape}")
     if a.size and (a.min() < 1 or a.max() > R):
         raise ValueError(f"n_props must lie in [1, {R}], got [{a.min()}, {a.max()}]")
+    return torch.from_numpy(a.astype(np.int32)).to(device, non_blocking=True)
+
+
+def feat_hw_arg(feat_hw, B, H, W, device):
+    """The feat_hw argument of the RoIAlign _ex entry points -> None (every image fills the [H, W] canvas) or a CUDA
+    int32 [B, 2] tensor of the per-image extents (H_b, W_b) on `device`.  A host sequence, numpy array or CPU tensor is
+    validated (shape [B, 2], integers, 1 <= H_b <= H, 1 <= W_b <= W) and copied to the device once; a CUDA tensor must be
+    int32 [B, 2] on `device` and is used as is (the kernels clamp its values to [1, H] x [1, W])."""
+    if feat_hw is None:
+        return None
+    if isinstance(feat_hw, torch.Tensor) and feat_hw.device.type != "cpu":
+        if not feat_hw.is_cuda or feat_hw.device != torch.device(device):
+            raise ValueError(f"feat_hw must be on {device} or on the host, got {feat_hw.device}")
+        if feat_hw.dtype != torch.int32:
+            raise TypeError(f"feat_hw must be int32 on the device, got {feat_hw.dtype}")
+        if tuple(feat_hw.shape) != (B, 2):
+            raise ValueError(f"feat_hw must have shape [{B}, 2], got {tuple(feat_hw.shape)}")
+        return feat_hw.contiguous()
+    a = feat_hw.numpy() if isinstance(feat_hw, torch.Tensor) else np.asarray(feat_hw)
+    if a.dtype.kind not in "iu":
+        raise TypeError(f"feat_hw must hold integers, got {a.dtype}")
+    if a.shape != (B, 2):
+        raise ValueError(f"feat_hw must have shape [{B}, 2], got {a.shape}")
+    if a.size and (a[:, 0].min() < 1 or a[:, 0].max() > H or a[:, 1].min() < 1 or a[:, 1].max() > W):
+        raise ValueError(f"feat_hw must lie in [1, {H}] x [1, {W}], got heights [{a[:, 0].min()}, {a[:, 0].max()}] "
+                         f"and widths [{a[:, 1].min()}, {a[:, 1].max()}]")
     return torch.from_numpy(a.astype(np.int32)).to(device, non_blocking=True)
 
 

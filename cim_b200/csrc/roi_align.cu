@@ -90,8 +90,8 @@ __device__ __forceinline__ float sample_coord(float start, float bin, int p, int
 }
 
 template <bool WIDE>
-__global__ void roi_prep_kernel(const float *__restrict__ rois, int K, int B, int H, int W,
-                                int oh, int ow, float scale, int sampling_ratio, int aligned,
+__global__ void roi_prep_kernel(const float *__restrict__ rois, const int *__restrict__ feat_hw, int K, int B, int H,
+                                int W, int oh, int ow, float scale, int sampling_ratio, int aligned,
                                 int *__restrict__ hdr, int *__restrict__ img_start,
                                 int *__restrict__ desc) {
     int gid = blockIdx.x * blockDim.x + threadIdx.x;
@@ -115,7 +115,8 @@ __global__ void roi_prep_kernel(const float *__restrict__ rois, int K, int B, in
     }
 
     const int nb = axis == 0 ? oh : ow;       // bins along this axis (7 on the tile path)
-    const int L = axis == 0 ? H : W;
+    // border rule on the image's own extent; the x-window shift below stays on the canvas width W
+    const int L = (b >= 0 && b < B) ? img_extent(feat_hw, b, axis, axis == 0 ? H : W) : (axis == 0 ? H : W);
     const float off = aligned ? .5f : 0.f;
     float c1 = __fsub_rn(__fmul_rn(r[1 + (axis == 0 ? 1 : 0)], scale), off);
     float c2 = __fsub_rn(__fmul_rn(r[3 + (axis == 0 ? 1 : 0)], scale), off);
@@ -1658,9 +1659,10 @@ __device__ __forceinline__ bool corners(int H, int W, float y, float x, int &y0,
 template <bool BWD>
 __global__ void roi_align_generic_kernel(const float *__restrict__ in, const float *__restrict__ rois,
                                          float *__restrict__ outp, const int *__restrict__ hdr,
-                                         const int *__restrict__ descs, const float *__restrict__ mask7, int mode,
-                                         int B, int C, int H, int W, int K, int oh, int ow, float scale, int sr,
-                                         int aligned, int desc_words = DESC_WORDS) {
+                                         const int *__restrict__ descs, const float *__restrict__ mask7,
+                                         const int *__restrict__ feat_hw, int mode, int B, int C, int H, int W, int K,
+                                         int oh, int ow, float scale, int sr, int aligned,
+                                         int desc_words = DESC_WORDS) {
     // mode 0: one CTA column per ROI.  mode 1 (leftover pass): 8 ROIs per CTA -- warp w checks ROI 8 blockIdx.x + w
     // (almost every one was done by the tile kernel: 8x fewer CTAs scheduled for nothing), then the WHOLE CTA works
     // through the ROIs that are left, one after the other (a VGG-size ROI with bins wider than 8 taps is 25 000
@@ -1688,6 +1690,8 @@ __global__ void roi_align_generic_kernel(const float *__restrict__ in, const flo
     const Geom g = roi_geom(rois + 5 * (size_t)k, scale, oh, ow, sr, aligned);
     const int per_roi = C * oh * ow;
     const bool valid_b = g.b >= 0 && g.b < B;
+    // the border rule sees the image's extent (H_b, W_b); planes and rows are addressed on the canvas (H, W)
+    const int Hb = valid_b ? img_extent(feat_hw, g.b, 0, H) : H, Wb = valid_b ? img_extent(feat_hw, g.b, 1, W) : W;
     const int e0 = mode == 1 ? threadIdx.x : blockIdx.y * blockDim.x + threadIdx.x;
     const int estep = mode == 1 ? blockDim.x : gridDim.y * blockDim.x;
     for (int e = e0; e < per_roi; e += estep) {
@@ -1707,7 +1711,7 @@ __global__ void roi_align_generic_kernel(const float *__restrict__ in, const flo
             for (int ix = 0; ix < g.gw; ++ix) {
                 const float x = sample_coord(g.xs, g.bw, pw, ix, g.gw);
                 int y0, y1, x0, x1; float a, b2, c2, d2;
-                if (!corners(H, W, y, x, y0, y1, x0, x1, a, b2, c2, d2)) continue;
+                if (!corners(Hb, Wb, y, x, y0, y1, x0, x1, a, b2, c2, d2)) continue;
                 if (BWD) {
                     float *p = outp + plane;
                     atomicAdd(p + y0 * W + x0, top * a / g.count);
@@ -1821,17 +1825,17 @@ static RoiWs carve(void *ws, int B, int K) {
     return w;
 }
 
-static int run_prep(const float *rois, int B, int H, int W, int K, int oh, int ow, float scale, int sr,
-                    int aligned, const RoiWs &w, bool wide, cudaStream_t st) {
+static int run_prep(const float *rois, const int *feat_hw, int B, int H, int W, int K, int oh, int ow, float scale,
+                    int sr, int aligned, const RoiWs &w, bool wide, cudaStream_t st) {
     cudaMemsetAsync(w.hdr, 0, WS_HDR_BYTES + sizeof(int) * (size_t)(B + 1), st);
     if (K > 0) {
         int threads = 128, blocks = (2 * K + threads - 1) / threads;
         if (wide)
-            roi_prep_kernel<true><<<blocks, threads, 0, st>>>(rois, K, B, H, W, oh, ow, scale, sr, aligned, w.hdr,
-                                                              w.img_start, w.desc);
+            roi_prep_kernel<true><<<blocks, threads, 0, st>>>(rois, feat_hw, K, B, H, W, oh, ow, scale, sr, aligned,
+                                                              w.hdr, w.img_start, w.desc);
         else
-            roi_prep_kernel<false><<<blocks, threads, 0, st>>>(rois, K, B, H, W, oh, ow, scale, sr, aligned, w.hdr,
-                                                               w.img_start, w.desc);
+            roi_prep_kernel<false><<<blocks, threads, 0, st>>>(rois, feat_hw, K, B, H, W, oh, ow, scale, sr, aligned,
+                                                               w.hdr, w.img_start, w.desc);
     }
     return cim_launch_status();
 }
@@ -1866,17 +1870,17 @@ static bool use_win(const Plan &p, int B, int K, size_t ws_bytes) {
     return p.win && K > 0 && !(cim_get_debug_flags() & CIM_DBG_ROI_NO_WINDOWS) &&
            ws_bytes >= ws_glob_off(K) + win_ws_bytes(p, B, K);
 }
-static int run_prep_win(const float *rois, int B, int H, int W, int K, float scale, int sr, int aligned, const RoiWs &w,
-                        const WinWs &ww, const Plan &p, cudaStream_t st) {
+static int run_prep_win(const float *rois, const int *feat_hw, int B, int H, int W, int K, float scale, int sr,
+                        int aligned, const RoiWs &w, const WinWs &ww, const Plan &p, cudaStream_t st) {
     const int nb = B * p.wg.nwy * p.wg.nwx;
     cudaMemsetAsync(w.hdr, 0, WS_HDR_BYTES, st);
     cudaMemsetAsync(ww.bucket, 0, sizeof(int) * ((size_t)nb + 2), st);
-    roi_win_plan_kernel<<<(2 * K + 127) / 128, 128, 0, st>>>(rois, K, B, H, W, scale, sr, aligned, ww);
+    roi_win_plan_kernel<<<(2 * K + 127) / 128, 128, 0, st>>>(rois, feat_hw, K, B, H, W, scale, sr, aligned, ww);
     roi_win_scan_kernel<<<1, 1024, 0, st>>>(K, ww);
     roi_win_keys_kernel<<<(K + 127) / 128, 128, 0, st>>>(rois, K, p.wg.nwy * p.wg.nwx, p.wg.nwx, ww);
     roi_win_bucket_kernel<<<1, 1024, 0, st>>>(nb, ww);
     roi_win_place_kernel<<<nb, 256, 0, st>>>(K, ww);
-    roi_win_emit_kernel<<<(2 * K + 127) / 128, 128, 0, st>>>(rois, K, H, W, scale, sr, aligned, ww);
+    roi_win_emit_kernel<<<(2 * K + 127) / 128, 128, 0, st>>>(rois, feat_hw, K, H, W, scale, sr, aligned, ww);
     return cim_launch_status();
 }
 
@@ -1894,10 +1898,11 @@ CIM_API size_t cim_roi_align_workspace_bytes(int K) {
     return WS_HDR_BYTES + 4097 * sizeof(int) + 64 + (size_t)(K > 0 ? K : 0) * (DESC_WORDS_MAX + MASK_PAD) * 4;
 }
 
-static int roi_fwd_impl(const float *feat, const float *rois, const float *mask7, float *out, int B, int C, int H,
-                        int W, int K, int oh, int ow, float scale, int sr, int aligned, void *ws, size_t ws_bytes,
-                        cim_stream_t stream, bool prepared = false) {
+static int roi_fwd_impl(const float *feat, const float *rois, const int *feat_hw, const float *mask7, float *out, int B,
+                        int C, int H, int W, int K, int oh, int ow, float scale, int sr, int aligned, void *ws,
+                        size_t ws_bytes, cim_stream_t stream, bool prepared = false) {
     if (B > 4096) return CIM_ERR_SHAPE;
+    if (!cim_aligned(feat_hw, 4)) return CIM_ERR_ALIGN;
     if (K == 0 && feat && B > 0 && C > 0 && H > 0 && W > 0 && oh > 0 && ow > 0) return CIM_OK;   // empty output
     int rc = check_args(feat, rois, out, B, C, H, W, K, oh, ow, ws, ws_bytes);
     if (rc) return rc;
@@ -1908,23 +1913,23 @@ static int roi_fwd_impl(const float *feat, const float *rois, const float *mask7
     dim3 ggrid((unsigned)K, (unsigned)min(64, (per_roi + 255) / 256));
     if (!p.tile && use_win(p, B, K, ws_bytes)) {
         const WinWs ww = carve_win(ws, p, B, K);
-        if (!prepared && (rc = run_prep_win(rois, B, H, W, K, scale, sr, aligned, w, ww, p, st))) return rc;
+        if (!prepared && (rc = run_prep_win(rois, feat_hw, B, H, W, K, scale, sr, aligned, w, ww, p, st))) return rc;
         cudaFuncSetAttribute(roi_align_fwd_win_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem_fwd_win);
         roi_align_fwd_win_kernel<<<cim_num_sms(), p.win_fwd_warps * 32, p.smem_fwd_win, st>>>(
             feat, ww.bucket, ww.desc, mask7, out, B, C, H, W, p.wg, p.win_pitch, p.win_wyd_floats);
         if ((rc = cim_launch_status())) return rc;
         // leftover pass: ROIs the window plan could not take (bins wider than WIN_MTB taps, batch index out of range)
         roi_align_generic_kernel<false><<<dim3((unsigned)((K + 7) / 8), 1), 256, 0, st>>>(
-            feat, rois, out, w.hdr, ww.flags, mask7, 1, B, C, H, W, K, oh, ow, scale, sr, aligned, 4);
+            feat, rois, out, w.hdr, ww.flags, mask7, feat_hw, 1, B, C, H, W, K, oh, ow, scale, sr, aligned, 4);
         return cim_launch_status();
     }
     const bool glob = !p.tile && p.glob && ws_bytes >= ws_glob_off(K) + glob_copy_bytes(B, C, H, W);
     if (!p.tile && !glob) {
-        roi_align_generic_kernel<false><<<ggrid, 256, 0, st>>>(feat, rois, out, nullptr, nullptr, mask7, 0, B, C, H, W,
+        roi_align_generic_kernel<false><<<ggrid, 256, 0, st>>>(feat, rois, out, nullptr, nullptr, mask7, feat_hw, 0, B, C, H, W,
                                                                K, oh, ow, scale, sr, aligned);
         return cim_launch_status();
     }
-    if (!prepared && (rc = run_prep(rois, B, H, W, K, oh, ow, scale, sr, aligned, w, glob, st))) return rc;
+    if (!prepared && (rc = run_prep(rois, feat_hw, B, H, W, K, oh, ow, scale, sr, aligned, w, glob, st))) return rc;
     const long long units = (long long)(C / CH) * K;
     const int grid = (int)min((long long)cim_num_sms(), units);
     if (glob) {
@@ -1945,15 +1950,16 @@ static int roi_fwd_impl(const float *feat, const float *rois, const float *mask7
     if ((rc = cim_launch_status())) return rc;
     // leftover pass: one CTA per ROI, which exits at once unless the tile kernel skipped that ROI
     roi_align_generic_kernel<false><<<dim3((unsigned)((K + 7) / 8), 1), 256, 0, st>>>(
-        feat, rois, out, w.hdr, w.desc, mask7, 1, B, C, H, W, K, oh, ow, scale, sr, aligned,
+        feat, rois, out, w.hdr, w.desc, mask7, feat_hw, 1, B, C, H, W, K, oh, ow, scale, sr, aligned,
         glob ? DESC_WORDS_MAX : DESC_WORDS);
     return cim_launch_status();
 }
 
-static int roi_bwd_impl(const float *grad_out, const float *rois, const float *mask7, float *grad_feat, int B, int C,
-                        int H, int W, int K, int oh, int ow, float scale, int sr, int aligned, void *ws,
-                        size_t ws_bytes, cim_stream_t stream, bool prepared = false) {
+static int roi_bwd_impl(const float *grad_out, const float *rois, const int *feat_hw, const float *mask7,
+                        float *grad_feat, int B, int C, int H, int W, int K, int oh, int ow, float scale, int sr,
+                        int aligned, void *ws, size_t ws_bytes, cim_stream_t stream, bool prepared = false) {
     if (B > 4096) return CIM_ERR_SHAPE;
+    if (!cim_aligned(feat_hw, 4)) return CIM_ERR_ALIGN;
     if (K == 0 && grad_feat && B > 0 && C > 0 && H > 0 && W > 0) {                // no ROI: zero gradient
         cudaMemsetAsync(grad_feat, 0, sizeof(float) * (size_t)B * C * H * W, (cudaStream_t)stream);
         return cim_launch_status();
@@ -1967,7 +1973,7 @@ static int roi_bwd_impl(const float *grad_out, const float *rois, const float *m
     dim3 ggrid((unsigned)max(K, 1), (unsigned)min(64, (per_roi + 255) / 256));
     if (!p.tile && use_win(p, B, K, ws_bytes)) {
         const WinWs ww = carve_win(ws, p, B, K);
-        if (!prepared && (rc = run_prep_win(rois, B, H, W, K, scale, sr, aligned, w, ww, p, st))) return rc;
+        if (!prepared && (rc = run_prep_win(rois, feat_hw, B, H, W, K, scale, sr, aligned, w, ww, p, st))) return rc;
         cudaMemsetAsync(grad_feat, 0, sizeof(float) * (size_t)B * C * H * W, st);
         const int grid = cim_num_sms();
         if (mask7) {
@@ -1985,18 +1991,18 @@ static int roi_bwd_impl(const float *grad_out, const float *rois, const float *m
         }
         if ((rc = cim_launch_status())) return rc;
         roi_align_generic_kernel<true><<<dim3((unsigned)((K + 7) / 8), 1), 256, 0, st>>>(
-            grad_out, rois, grad_feat, w.hdr, ww.flags, mask7, 1, B, C, H, W, K, oh, ow, scale, sr, aligned, 4);
+            grad_out, rois, grad_feat, w.hdr, ww.flags, mask7, feat_hw, 1, B, C, H, W, K, oh, ow, scale, sr, aligned, 4);
         return cim_launch_status();
     }
     const bool glob = !p.tile && p.glob && K > 0 && ws_bytes >= ws_glob_off(K) + glob_copy_bytes(B, C, H, W);
     if ((!p.tile && !glob) || K == 0) {
         cudaMemsetAsync(grad_feat, 0, sizeof(float) * (size_t)B * C * H * W, st);
         if (K > 0)
-            roi_align_generic_kernel<true><<<ggrid, 256, 0, st>>>(grad_out, rois, grad_feat, nullptr, nullptr, mask7, 0,
+            roi_align_generic_kernel<true><<<ggrid, 256, 0, st>>>(grad_out, rois, grad_feat, nullptr, nullptr, mask7, feat_hw, 0,
                                                                   B, C, H, W, K, oh, ow, scale, sr, aligned);
         return cim_launch_status();
     }
-    if (!prepared && (rc = run_prep(rois, B, H, W, K, oh, ow, scale, sr, aligned, w, glob, st))) return rc;
+    if (!prepared && (rc = run_prep(rois, feat_hw, B, H, W, K, oh, ow, scale, sr, aligned, w, glob, st))) return rc;
     // two chunks per CTA (see the kernel): tensor-memory variant, an even number of chunks, no fused mask, and maps of
     // at most 8 row pairs, where it is what keeps all 16 warps busy (HRNet 16 x 16 x 2048: 2.36 -> 1.74 ms).  On 16
     // row pairs it only rebalances the centre-heavy load and loses more to its smaller batches (8 ROIs per barrier
@@ -2026,7 +2032,8 @@ static int roi_bwd_impl(const float *grad_out, const float *rois, const float *m
         pairs_to_nchw_kernel<<<cg, 256, 0, st>>>(reinterpret_cast<const float2 *>(gradP), grad_feat, C, H, W);
         if ((rc = cim_launch_status())) return rc;
         roi_align_generic_kernel<true><<<dim3((unsigned)((K + 7) / 8), 1), 256, 0, st>>>(
-            grad_out, rois, grad_feat, w.hdr, w.desc, mask7, 1, B, C, H, W, K, oh, ow, scale, sr, aligned, DESC_WORDS_MAX);
+            grad_out, rois, grad_feat, w.hdr, w.desc, mask7, feat_hw, 1, B, C, H, W, K, oh, ow, scale, sr, aligned,
+            DESC_WORDS_MAX);
         return cim_launch_status();
     }
     cudaMemsetAsync(grad_feat, 0, sizeof(float) * (size_t)B * C * H * W, st);
@@ -2052,62 +2059,87 @@ static int roi_bwd_impl(const float *grad_out, const float *rois, const float *m
     }
     if ((rc = cim_launch_status())) return rc;
     roi_align_generic_kernel<true><<<dim3((unsigned)((K + 7) / 8), 1), 256, 0, st>>>(grad_out, rois, grad_feat, w.hdr, w.desc,
-                                                                         mask7, 1, B, C, H, W, K, oh, ow, scale, sr,
+                                                                         mask7, feat_hw, 1, B, C, H, W, K, oh, ow, scale, sr,
                                                                          aligned);
     return cim_launch_status();
 }
 
 // Descriptors once for several calls on the same rois (forward + backward of one step share them): the same plan /
 // layout decision as the _impl functions, which then skip their own prep launch.
-CIM_API int cim_roi_align_prepare(const float *rois, int B, int C, int H, int W, int K, int oh, int ow, float scale,
-                                  int sr, int aligned, void *ws, size_t ws_bytes, cim_stream_t stream) {
+CIM_API int cim_roi_align_prepare_ex(const float *rois, const int32_t *feat_hw, int B, int C, int H, int W, int K, int oh,
+                                     int ow, float scale, int sr, int aligned, void *ws, size_t ws_bytes,
+                                     cim_stream_t stream) {
     if (B > 4096) return CIM_ERR_SHAPE;
     if (K == 0) return CIM_OK;
     if (!rois || B <= 0 || C <= 0 || H <= 0 || W <= 0 || K < 0 || oh <= 0 || ow <= 0) return CIM_ERR_ARG;
     if ((long long)H * W > (1 << 24) || (long long)C * oh * ow > (1LL << 30)) return CIM_ERR_SHAPE;
     if (!ws || ws_bytes < cim_roi_align_workspace_bytes(K)) return CIM_ERR_WORKSPACE;
-    if (!cim_aligned(ws, 16)) return CIM_ERR_ALIGN;
+    if (!cim_aligned(ws, 16) || !cim_aligned(feat_hw, 4)) return CIM_ERR_ALIGN;
     const Plan p = make_plan(C, H, W, oh, ow);
     if (!p.tile && use_win(p, B, K, ws_bytes))
-        return run_prep_win(rois, B, H, W, K, scale, sr, aligned, carve(ws, B, K), carve_win(ws, p, B, K), p,
+        return run_prep_win(rois, feat_hw, B, H, W, K, scale, sr, aligned, carve(ws, B, K), carve_win(ws, p, B, K), p,
                             (cudaStream_t)stream);
     const bool glob = !p.tile && p.glob && ws_bytes >= ws_glob_off(K) + glob_copy_bytes(B, C, H, W);
     if (!p.tile && !glob) return CIM_OK;                   // generic kernels: no descriptors
-    return run_prep(rois, B, H, W, K, oh, ow, scale, sr, aligned, carve(ws, B, K), glob, (cudaStream_t)stream);
+    return run_prep(rois, feat_hw, B, H, W, K, oh, ow, scale, sr, aligned, carve(ws, B, K), glob, (cudaStream_t)stream);
+}
+
+CIM_API int cim_roi_align_fwd_prepared_ex(const float *feat, const float *rois, const int32_t *feat_hw,
+                                          const float *masks7, float *out, int B, int C, int H, int W, int K, int oh,
+                                          int ow, float scale, int sr, int aligned, void *ws, size_t ws_bytes,
+                                          cim_stream_t stream) {
+    return roi_fwd_impl(feat, rois, feat_hw, masks7, out, B, C, H, W, K, oh, ow, scale, sr, aligned, ws, ws_bytes,
+                        stream, true);
+}
+
+CIM_API int cim_roi_align_bwd_prepared_ex(const float *grad_out, const float *rois, const int32_t *feat_hw,
+                                          const float *masks7, float *grad_feat, int B, int C, int H, int W, int K,
+                                          int oh, int ow, float scale, int sr, int aligned, void *ws, size_t ws_bytes,
+                                          cim_stream_t stream) {
+    return roi_bwd_impl(grad_out, rois, feat_hw, masks7, grad_feat, B, C, H, W, K, oh, ow, scale, sr, aligned, ws,
+                        ws_bytes, stream, true);
+}
+
+CIM_API int cim_roi_align_prepare(const float *rois, int B, int C, int H, int W, int K, int oh, int ow, float scale,
+                                  int sr, int aligned, void *ws, size_t ws_bytes, cim_stream_t stream) {
+    return cim_roi_align_prepare_ex(rois, nullptr, B, C, H, W, K, oh, ow, scale, sr, aligned, ws, ws_bytes, stream);
 }
 
 CIM_API int cim_roi_align_fwd_prepared(const float *feat, const float *rois, const float *masks7, float *out, int B,
                                        int C, int H, int W, int K, int oh, int ow, float scale, int sr, int aligned,
                                        void *ws, size_t ws_bytes, cim_stream_t stream) {
-    return roi_fwd_impl(feat, rois, masks7, out, B, C, H, W, K, oh, ow, scale, sr, aligned, ws, ws_bytes, stream, true);
+    return roi_fwd_impl(feat, rois, nullptr, masks7, out, B, C, H, W, K, oh, ow, scale, sr, aligned, ws, ws_bytes,
+                        stream, true);
 }
 
 CIM_API int cim_roi_align_bwd_prepared(const float *grad_out, const float *rois, const float *masks7,
                                        float *grad_feat, int B, int C, int H, int W, int K, int oh, int ow,
                                        float scale, int sr, int aligned, void *ws, size_t ws_bytes,
                                        cim_stream_t stream) {
-    return roi_bwd_impl(grad_out, rois, masks7, grad_feat, B, C, H, W, K, oh, ow, scale, sr, aligned, ws, ws_bytes,
-                        stream, true);
+    return roi_bwd_impl(grad_out, rois, nullptr, masks7, grad_feat, B, C, H, W, K, oh, ow, scale, sr, aligned, ws,
+                        ws_bytes, stream, true);
 }
 
 CIM_API int cim_roi_align_fwd(const float *feat, const float *rois, float *out, int B, int C, int H, int W,
                               int K, int oh, int ow, float scale, int sr, int aligned, void *ws,
                               size_t ws_bytes, cim_stream_t stream) {
-    return roi_fwd_impl(feat, rois, nullptr, out, B, C, H, W, K, oh, ow, scale, sr, aligned, ws, ws_bytes, stream);
+    return roi_fwd_impl(feat, rois, nullptr, nullptr, out, B, C, H, W, K, oh, ow, scale, sr, aligned, ws, ws_bytes,
+                        stream);
 }
 
 CIM_API int cim_roi_align_bwd(const float *grad_out, const float *rois, float *grad_feat, int B, int C, int H,
                               int W, int K, int oh, int ow, float scale, int sr, int aligned, void *ws,
                               size_t ws_bytes, cim_stream_t stream) {
-    return roi_bwd_impl(grad_out, rois, nullptr, grad_feat, B, C, H, W, K, oh, ow, scale, sr, aligned, ws, ws_bytes,
-                        stream);
+    return roi_bwd_impl(grad_out, rois, nullptr, nullptr, grad_feat, B, C, H, W, K, oh, ow, scale, sr, aligned, ws,
+                        ws_bytes, stream);
 }
 
 CIM_API int cim_roi_align_maskfuse_fwd(const float *feat, const float *rois, const float *masks7, float *out, int B,
                                        int C, int H, int W, int K, int oh, int ow, float scale, int sr, int aligned,
                                        void *ws, size_t ws_bytes, cim_stream_t stream) {
     if (!masks7 && K > 0) return CIM_ERR_ARG;
-    return roi_fwd_impl(feat, rois, masks7, out, B, C, H, W, K, oh, ow, scale, sr, aligned, ws, ws_bytes, stream);
+    return roi_fwd_impl(feat, rois, nullptr, masks7, out, B, C, H, W, K, oh, ow, scale, sr, aligned, ws, ws_bytes,
+                        stream);
 }
 
 CIM_API int cim_roi_align_maskfuse_bwd(const float *grad_out, const float *rois, const float *masks7,
@@ -2115,31 +2147,37 @@ CIM_API int cim_roi_align_maskfuse_bwd(const float *grad_out, const float *rois,
                                        float scale, int sr, int aligned, void *ws, size_t ws_bytes,
                                        cim_stream_t stream) {
     if (!masks7 && K > 0) return CIM_ERR_ARG;
-    return roi_bwd_impl(grad_out, rois, masks7, grad_feat, B, C, H, W, K, oh, ow, scale, sr, aligned, ws, ws_bytes,
-                        stream);
+    return roi_bwd_impl(grad_out, rois, nullptr, masks7, grad_feat, B, C, H, W, K, oh, ow, scale, sr, aligned, ws,
+                        ws_bytes, stream);
 }
 
 // Test hook (host only, no GPU): the window plan of roi_window.cuh evaluated on the CPU with the same
 // __host__ __device__ code the prep kernels run.  All pointers are HOST memory.  Sub-ROI descriptors come out in ROI
 // order (the device sorts them by window afterwards); key_out = window index wy * nwx + wx of each sub-ROI, flag_out[k]
-// = 1 for ROIs the window path leaves to the generic kernel, geom_out = {Hp, wh, ww, nwy, nwx, WIN_G}.
+// = 1 for ROIs the window path leaves to the generic kernel, geom_out = {Hp, wh, ww, nwy, nwx, WIN_G}.  feat_hw: host
+// [B][2] image extents, clamped like the device's (NULL: the canvas).
 // Returns the number of sub-ROIs, or a negative CIM_ERR_* code (CIM_ERR_WORKSPACE: more than `cap`).
-CIM_API int cim_debug_roi_window_plan(const float *rois, int K, int B, int H, int W, float scale, int sr, int aligned,
-                                      int *desc_out, int *key_out, int cap, int *flag_out, int *geom_out) {
+CIM_API int cim_debug_roi_window_plan_ex(const float *rois, const int32_t *feat_hw, int K, int B, int H, int W,
+                                         float scale, int sr, int aligned, int *desc_out, int *key_out, int cap,
+                                         int *flag_out, int *geom_out) {
     if (!rois || !desc_out || !key_out || !flag_out || !geom_out || K < 0 || B <= 0 || H <= 0 || W < MAXT)
         return CIM_ERR_ARG;
+    if (!cim_aligned(feat_hw, 4)) return CIM_ERR_ALIGN;
     const WinGeom g = win_geom(H, W);
     geom_out[0] = g.Hp; geom_out[1] = g.wh; geom_out[2] = g.ww; geom_out[3] = g.nwy; geom_out[4] = g.nwx;
     geom_out[5] = WIN_G;
     int n = 0;
     for (int k = 0; k < K; ++k) {
         const float *r = rois + 5 * (size_t)k;
-        const AxisGeom ay = win_axis_geom(r, 0, 7, scale, sr, aligned), ax = win_axis_geom(r, 1, 7, scale, sr, aligned);
-        AxisPlan py, px;
-        win_axis_plan(ay, H, g.Hp, g.wh, g.nwy, py);
-        win_axis_plan(ax, W, W, g.ww, g.nwx, px);
         const int b = (int)r[0];
-        flag_out[k] = (b < 0 || b >= B || py.nseg == 0 || px.nseg == 0) ? 1 : 0;
+        flag_out[k] = 1;
+        if (b < 0 || b >= B) continue;
+        const AxisGeom ay = win_axis_geom(r, 0, 7, scale, sr, aligned), ax = win_axis_geom(r, 1, 7, scale, sr, aligned);
+        const int Hb = img_extent(feat_hw, b, 0, H), Wb = img_extent(feat_hw, b, 1, W);
+        AxisPlan py, px;
+        win_axis_plan(ay, Hb, g.Hp, g.wh, g.nwy, py);
+        win_axis_plan(ax, Wb, W, g.ww, g.nwx, px);
+        flag_out[k] = (py.nseg == 0 || px.nseg == 0) ? 1 : 0;
         if (flag_out[k]) continue;
         const bool simple = py.nseg == 1 && px.nseg == 1 && py.nslots[0] == 7 && px.nslots[0] == 7;
         for (int sy = 0; sy < py.nseg; ++sy)
@@ -2147,11 +2185,17 @@ CIM_API int cim_debug_roi_window_plan(const float *rois, int K, int B, int H, in
                 if (n >= cap) return CIM_ERR_WORKSPACE;
                 int *d = desc_out + (size_t)n * DESC_WORDS;
                 for (int i = 0; i < DESC_WORDS; ++i) d[i] = 0;
-                win_axis_emit(ay, py, sy, 0, H, g.Hp, g.wh, k, simple, d);
-                win_axis_emit(ax, px, sx, 1, W, W, g.ww, k, simple, d);
+                win_axis_emit(ay, py, sy, 0, Hb, g.Hp, g.wh, k, simple, d);
+                win_axis_emit(ax, px, sx, 1, Wb, W, g.ww, k, simple, d);
                 key_out[n] = py.wcoord[sy] * g.nwx + px.wcoord[sx];
                 ++n;
             }
     }
     return n;
+}
+
+CIM_API int cim_debug_roi_window_plan(const float *rois, int K, int B, int H, int W, float scale, int sr, int aligned,
+                                      int *desc_out, int *key_out, int cap, int *flag_out, int *geom_out) {
+    return cim_debug_roi_window_plan_ex(rois, nullptr, K, B, H, W, scale, sr, aligned, desc_out, key_out, cap, flag_out,
+                                        geom_out);
 }

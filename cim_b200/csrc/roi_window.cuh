@@ -117,6 +117,19 @@ __host__ __device__ inline AxisGeom win_axis_geom(const float *r, int axis, int 
     return a;
 }
 
+// Border length of image b along an axis (0 = rows) of a canvas of length L: feat_hw [B][2] = (H_b, W_b), clamped to
+// [1, L]; NULL: every image fills the canvas.  Only the border rule (clamp to L_b - 1, drop beyond L_b) uses it; window
+// geometry, tile layout and addressing stay on the canvas.
+__host__ __device__ inline int img_extent(const int *feat_hw, int b, int axis, int L) {
+    if (!feat_hw) return L;
+#ifdef __CUDA_ARCH__
+    const int v = __ldg(feat_hw + 2 * b + axis);
+#else
+    const int v = feat_hw[2 * b + axis];
+#endif
+    return v < 1 ? 1 : v > L ? L : v;
+}
+
 // Plan of one (roi, axis): bins -> slots -> segments.
 struct AxisPlan {
     int nseg;              // 0: this ROI takes the generic kernel
@@ -127,7 +140,8 @@ struct AxisPlan {
 };
 __host__ __device__ inline int win_slots_of(int n) { return n <= 8 ? 1 : (n + 7) >> 3; }
 
-// L: map length along the axis, Lp: padded length (rows: even), wl: window length, nw: window positions
+// L: the image's length along the axis (border rule), Lp: padded canvas length (rows: even), wl: window length,
+// nw: window positions
 __host__ __device__ inline void win_axis_plan(const AxisGeom &a, int L, int Lp, int wl, int nw, AxisPlan &pl) {
     pl.nseg = 0;
     if (a.bad) return;
@@ -303,8 +317,8 @@ __device__ __forceinline__ int win_rec_coord(const int *r, int s) {
 }
 
 // pass 1: thread per (roi, axis): plan -> record
-__global__ void roi_win_plan_kernel(const float *__restrict__ rois, int K, int B, int H, int W, float scale, int sr,
-                                    int aligned, WinWs ws) {
+__global__ void roi_win_plan_kernel(const float *__restrict__ rois, const int *__restrict__ feat_hw, int K, int B, int H,
+                                    int W, float scale, int sr, int aligned, WinWs ws) {
     const int gid = blockIdx.x * blockDim.x + threadIdx.x;
     const int k = gid >> 1, axis = gid & 1;
     if (k >= K) return;
@@ -314,8 +328,8 @@ __global__ void roi_win_plan_kernel(const float *__restrict__ rois, int K, int B
     AxisPlan pl;
     const int b = (int)r[0];
     if (b < 0 || b >= B) pl.nseg = 0;
-    else if (axis == 0) win_axis_plan(a, H, g.Hp, g.wh, g.nwy, pl);
-    else win_axis_plan(a, W, W, g.ww, g.nwx, pl);
+    else if (axis == 0) win_axis_plan(a, img_extent(feat_hw, b, 0, H), g.Hp, g.wh, g.nwy, pl);
+    else win_axis_plan(a, img_extent(feat_hw, b, 1, W), W, g.ww, g.nwx, pl);
     win_pack_rec(pl, ws.rec + ((size_t)k * 2 + axis) * 4);
 }
 
@@ -457,8 +471,8 @@ roi_win_place_kernel(int K, WinWs ws) {
 }
 
 // pass 6: thread per (roi, axis): the axis' part of the descriptors of every sub-ROI of the ROI
-__global__ void roi_win_emit_kernel(const float *__restrict__ rois, int K, int H, int W, float scale, int sr,
-                                    int aligned, WinWs ws) {
+__global__ void roi_win_emit_kernel(const float *__restrict__ rois, const int *__restrict__ feat_hw, int K, int H, int W,
+                                    float scale, int sr, int aligned, WinWs ws) {
     const int gid = blockIdx.x * blockDim.x + threadIdx.x;
     const int k = gid >> 1, axis = gid & 1;
     if (k >= K) return;
@@ -466,9 +480,10 @@ __global__ void roi_win_emit_kernel(const float *__restrict__ rois, int K, int H
     const float *r = rois + 5 * (size_t)k;
     const WinGeom g = win_geom(H, W);
     const AxisGeom a = win_axis_geom(r, axis, 7, scale, sr, aligned);
+    const int Lb = img_extent(feat_hw, (int)r[0], axis, axis == 0 ? H : W);    // (flagged: b out of range, above)
     AxisPlan pl;
-    if (axis == 0) win_axis_plan(a, H, g.Hp, g.wh, g.nwy, pl);
-    else win_axis_plan(a, W, W, g.ww, g.nwx, pl);
+    if (axis == 0) win_axis_plan(a, Lb, g.Hp, g.wh, g.nwy, pl);
+    else win_axis_plan(a, Lb, W, g.ww, g.nwx, pl);
     const int *ry = ws.rec + ((size_t)k * 2) * 4, *rx = ry + 4;
     const int ny = ry[0] & 255, nx = rx[0] & 255;
     const bool simple = (ry[0] & 256) && (rx[0] & 256);
@@ -480,8 +495,8 @@ __global__ void roi_win_emit_kernel(const float *__restrict__ rois, int K, int H
             const int item = base + (axis == 0 ? s * nx + t : t * nx + s);
             int *d = ws.desc + (size_t)ws.slot[item] * DESC_WORDS;
             if (t == 0) {
-                if (axis == 0) win_axis_emit(a, pl, s, 0, H, g.Hp, g.wh, k, simple, d);
-                else win_axis_emit(a, pl, s, 1, W, W, g.ww, k, simple, d);
+                if (axis == 0) win_axis_emit(a, pl, s, 0, Lb, g.Hp, g.wh, k, simple, d);
+                else win_axis_emit(a, pl, s, 1, Lb, W, g.ww, k, simple, d);
                 d0 = d;
             } else if (axis == 0) {            // the row part: words 0, 1, 4, 5, 7, 8..23, 32..109
                 d[0] = d0[0]; d[1] = d0[1]; d[4] = d0[4]; d[5] = d0[5]; d[7] = d0[7];

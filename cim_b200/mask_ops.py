@@ -88,6 +88,44 @@ def crops_from_packed_host(packed, height, width):
                      height, width)
 
 
+def batch_crops_host(crops, R, height, width):
+    """CPU: the wire format of a batch of differently sized images.  crops: one MaskCrops per image (n_b <= R masks of
+    that image at its native size, e.g. from pack_crops_host), each image placed at the top left of a common
+    (height, width) canvas -> one MaskCrops of len(crops) * R rows, image b in rows [b * R, b * R + n_b) and EMPTY crops
+    (meta 0) in its padding rows, which the unpack turns into all-zero masks.  Zero padding changes neither
+    |a & b|, |a | b| nor |b|, so the overlap maps of an image on the canvas are those of the image alone.  A crop
+    that does not fit the canvas (rows, or 32-pixel words in x) raises."""
+    n_img = len(crops)
+    canvas_words = (width + 31) // 32
+    meta = np.zeros((n_img * R, 4), np.int32)
+    off = np.zeros(n_img * R, np.int64)
+    chunks, total = [], 0
+    for b, c in enumerate(crops):
+        m = np.asarray(c.meta, dtype=np.int64).reshape(-1, 4)
+        o = np.asarray(c.off, dtype=np.int64).reshape(-1)
+        w = np.asarray(c.words).view(np.int32).reshape(-1)
+        n = m.shape[0]
+        if n > R:
+            raise ValueError(f"image {b}: {n} masks exceed R = {R}")
+        if c.height > height or c.width > width:
+            raise ValueError(f"image {b}: native size {c.height} x {c.width} exceeds the canvas {height} x {width}")
+        full = (m[:, 2] > 0) & (m[:, 3] > 0)
+        if np.any(full & ((m[:, 0] < 0) | (m[:, 1] < 0) | (m[:, 0] + m[:, 2] > canvas_words) |
+                          (m[:, 1] + m[:, 3] > height))):
+            raise ValueError(f"image {b}: a crop does not fit the {height} x {width} canvas")
+        for i in range(R):
+            r = b * R + i
+            off[r] = total                                  # (empty and padding rows: no words)
+            if i < n and full[i]:
+                size = int(m[i, 2] * m[i, 3])
+                meta[r] = m[i]
+                chunks.append(w[o[i]:o[i] + size])
+                total += size
+    words = np.concatenate(chunks) if chunks else np.zeros(0, np.int32)
+    return MaskCrops(torch.from_numpy(words.astype(np.int32, copy=True)), torch.from_numpy(meta),
+                     torch.from_numpy(off), height, width)
+
+
 def tiled_ok(height, width):
     """The 8 x 16 patch pixel order (cim_mask_pack_tiled) needs whole patches."""
     return height % 8 == 0 and width % 16 == 0

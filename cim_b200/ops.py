@@ -8,6 +8,11 @@ a fresh module per call with positional arguments.  Same names, argument order a
 `cim_b200/shim` is on PYTHONPATH (INTEGRATION.md).
 
 rois: [K, 5] float32 rows (batch_idx, x1, y1, x2, y2) in input-image pixels.
+
+feat_hw (keyword, RoIAlign only): images of different sizes batched on one canvas.  input [N, C, H, W] is the canvas
+and image b occupies input[b, :, :H_b, :W_b]; feat_hw [N, 2] holds the (H_b, W_b) (see _lib.feat_hw_arg).  Each
+image's outputs and gradient then equal RoIAlign of its own map alone; the canvas outside the extents must be finite
+and gets a gradient of exactly 0.  None: every image fills the canvas.
 """
 import torch
 from torch import nn
@@ -38,7 +43,8 @@ def _check_inputs(feat, rois):
 
 class RoIAlignFunction(Function):
     @staticmethod
-    def forward(ctx, feat, rois, output_size, spatial_scale=1.0, sampling_ratio=0, pool_mode="avg", aligned=True):
+    def forward(ctx, feat, rois, output_size, spatial_scale=1.0, sampling_ratio=0, pool_mode="avg", aligned=True,
+                feat_hw=None):
         if pool_mode != "avg":
             raise NotImplementedError("only pool_mode='avg' is implemented (the reference never uses 'max')")
         _check_inputs(feat, rois)
@@ -46,17 +52,22 @@ class RoIAlignFunction(Function):
         feat, rois = feat.contiguous(), rois.contiguous()
         B, Cc, H, W = feat.shape
         K = rois.size(0)
+        hw = _lib.feat_hw_arg(feat_hw, B, H, W, feat.device)
         L = _lib.lib()
         with torch.cuda.device(feat.device):
             ws = torch.empty(L.cim_roi_align_workspace_bytes_ex(B, Cc, H, W, K, oh, ow), dtype=torch.uint8,
                              device=feat.device)
             out = torch.empty((K, Cc, oh, ow), dtype=torch.float32, device=feat.device)
-            rc = L.cim_roi_align_fwd(_lib.ptr(feat), _lib.ptr(rois), _lib.ptr(out), B, Cc, H, W, K, oh, ow,
-                                     float(spatial_scale), int(sampling_ratio), int(bool(aligned)),
-                                     _lib.ptr(ws), ws.numel(), _lib.stream_ptr(feat.device))
+            if hw is None:
+                rc = L.cim_roi_align_fwd(_lib.ptr(feat), _lib.ptr(rois), _lib.ptr(out), B, Cc, H, W, K, oh, ow,
+                                         float(spatial_scale), int(sampling_ratio), int(bool(aligned)),
+                                         _lib.ptr(ws), ws.numel(), _lib.stream_ptr(feat.device))
+            else:
+                rc = _fwd_ex(L, feat, rois, hw, None, out, oh, ow, spatial_scale, sampling_ratio, aligned, ws)
         _lib.check(rc, "cim_roi_align_fwd")
         ctx.save_for_backward(rois)
         ctx.ws = ws                 # the backward reuses the forward's ROI descriptors (cim_roi_align_bwd_prepared)
+        ctx.hw = hw
         ctx.cfg = (tuple(feat.shape), oh, ow, float(spatial_scale), int(sampling_ratio), int(bool(aligned)))
         return out
 
@@ -71,11 +82,25 @@ class RoIAlignFunction(Function):
         ws = ctx.ws
         with torch.cuda.device(grad_out.device):
             grad_feat = torch.empty((B, Cc, H, W), dtype=torch.float32, device=grad_out.device)
-            rc = L.cim_roi_align_bwd_prepared(_lib.ptr(grad_out), _lib.ptr(rois), None, _lib.ptr(grad_feat), B, Cc, H,
-                                              W, K, oh, ow, scale, sr, aligned, _lib.ptr(ws), ws.numel(),
-                                              _lib.stream_ptr(grad_out.device))
+            rc = L.cim_roi_align_bwd_prepared_ex(_lib.ptr(grad_out), _lib.ptr(rois), _lib.ptr(ctx.hw), None,
+                                                 _lib.ptr(grad_feat), B, Cc, H, W, K, oh, ow, scale, sr, aligned,
+                                                 _lib.ptr(ws), ws.numel(), _lib.stream_ptr(grad_out.device))
         _lib.check(rc, "cim_roi_align_bwd")
-        return grad_feat, None, None, None, None, None, None
+        return grad_feat, None, None, None, None, None, None, None
+
+
+def _fwd_ex(L, feat, rois, hw, masks, out, oh, ow, spatial_scale, sampling_ratio, aligned, ws):
+    """Descriptors with the image extents hw, then the forward that reuses them (the backward does too)."""
+    B, Cc, H, W = feat.shape
+    K = rois.size(0)
+    st = _lib.stream_ptr(feat.device)
+    args = (B, Cc, H, W, K, oh, ow, float(spatial_scale), int(sampling_ratio), int(bool(aligned)), _lib.ptr(ws),
+            ws.numel(), st)
+    rc = L.cim_roi_align_prepare_ex(_lib.ptr(rois), _lib.ptr(hw), *args)
+    if rc == 0:
+        rc = L.cim_roi_align_fwd_prepared_ex(_lib.ptr(feat), _lib.ptr(rois), _lib.ptr(hw), _lib.ptr(masks),
+                                             _lib.ptr(out), *args)
+    return rc
 
 
 #: RoIPool bin conventions (cim_roi_pool_fwd_ex): "mmcv" = mmcv 1.x's RoIPool, the op the reference imports
@@ -127,7 +152,7 @@ class RoIAlignMaskFuseFunction(Function):
     (the reference passes masks.detach(), model_builder.py:136)."""
 
     @staticmethod
-    def forward(ctx, feat, rois, masks, output_size, spatial_scale=1.0, sampling_ratio=0, aligned=True):
+    def forward(ctx, feat, rois, masks, output_size, spatial_scale=1.0, sampling_ratio=0, aligned=True, feat_hw=None):
         _check_inputs(feat, rois)
         _lib.require_cuda(masks, "masks", torch.float32)
         oh, ow = _pair(output_size)
@@ -135,18 +160,23 @@ class RoIAlignMaskFuseFunction(Function):
         B, Cc, H, W = feat.shape
         K = rois.size(0)
         masks = masks.reshape(K, oh, ow).contiguous()
+        hw = _lib.feat_hw_arg(feat_hw, B, H, W, feat.device)
         L = _lib.lib()
         with torch.cuda.device(feat.device):
             ws = torch.empty(L.cim_roi_align_workspace_bytes_ex(B, Cc, H, W, K, oh, ow), dtype=torch.uint8,
                              device=feat.device)
             out = torch.empty((K, 2 * Cc, oh, ow), dtype=torch.float32, device=feat.device)
-            rc = L.cim_roi_align_maskfuse_fwd(_lib.ptr(feat), _lib.ptr(rois), _lib.ptr(masks), _lib.ptr(out), B, Cc, H,
-                                              W, K, oh, ow, float(spatial_scale), int(sampling_ratio),
-                                              int(bool(aligned)), _lib.ptr(ws), ws.numel(),
-                                              _lib.stream_ptr(feat.device))
+            if hw is None:
+                rc = L.cim_roi_align_maskfuse_fwd(_lib.ptr(feat), _lib.ptr(rois), _lib.ptr(masks), _lib.ptr(out), B,
+                                                  Cc, H, W, K, oh, ow, float(spatial_scale), int(sampling_ratio),
+                                                  int(bool(aligned)), _lib.ptr(ws), ws.numel(),
+                                                  _lib.stream_ptr(feat.device))
+            else:
+                rc = _fwd_ex(L, feat, rois, hw, masks, out, oh, ow, spatial_scale, sampling_ratio, aligned, ws)
         _lib.check(rc, "cim_roi_align_maskfuse_fwd")
         ctx.save_for_backward(rois, masks)
         ctx.ws = ws
+        ctx.hw = hw
         ctx.cfg = (tuple(feat.shape), oh, ow, float(spatial_scale), int(sampling_ratio), int(bool(aligned)))
         return out
 
@@ -161,20 +191,24 @@ class RoIAlignMaskFuseFunction(Function):
         ws = ctx.ws
         with torch.cuda.device(grad_out.device):
             grad_feat = torch.empty((B, Cc, H, W), dtype=torch.float32, device=grad_out.device)
-            rc = L.cim_roi_align_bwd_prepared(_lib.ptr(grad_out), _lib.ptr(rois), _lib.ptr(masks), _lib.ptr(grad_feat),
-                                              B, Cc, H, W, K, oh, ow, scale, sr, aligned, _lib.ptr(ws), ws.numel(),
-                                              _lib.stream_ptr(grad_out.device))
+            rc = L.cim_roi_align_bwd_prepared_ex(_lib.ptr(grad_out), _lib.ptr(rois), _lib.ptr(ctx.hw), _lib.ptr(masks),
+                                                 _lib.ptr(grad_feat), B, Cc, H, W, K, oh, ow, scale, sr, aligned,
+                                                 _lib.ptr(ws), ws.numel(), _lib.stream_ptr(grad_out.device))
         _lib.check(rc, "cim_roi_align_maskfuse_bwd")
-        return grad_feat, None, None, None, None, None, None
+        return grad_feat, None, None, None, None, None, None, None
 
 
-def roi_align_maskfuse(input, rois, masks, output_size, spatial_scale=1.0, sampling_ratio=0, aligned=True):
+def roi_align_maskfuse(input, rois, masks, output_size, spatial_scale=1.0, sampling_ratio=0, aligned=True, *,
+                       feat_hw=None):
     """[K, 2C, oh, ow] = concat(RoIAlign(input, rois), RoIAlign(input, rois) * masks[:, None]) in one pass."""
-    return RoIAlignMaskFuseFunction.apply(input, rois, masks, output_size, spatial_scale, sampling_ratio, aligned)
+    return RoIAlignMaskFuseFunction.apply(input, rois, masks, output_size, spatial_scale, sampling_ratio, aligned,
+                                          feat_hw)
 
 
-def roi_align(input, rois, output_size, spatial_scale=1.0, sampling_ratio=0, pool_mode="avg", aligned=True):
-    return RoIAlignFunction.apply(input, rois, output_size, spatial_scale, sampling_ratio, pool_mode, aligned)
+def roi_align(input, rois, output_size, spatial_scale=1.0, sampling_ratio=0, pool_mode="avg", aligned=True, *,
+              feat_hw=None):
+    return RoIAlignFunction.apply(input, rois, output_size, spatial_scale, sampling_ratio, pool_mode, aligned,
+                                  feat_hw)
 
 
 def roi_pool(input, rois, output_size, spatial_scale=1.0, variant="mmcv"):
@@ -196,9 +230,9 @@ class RoIAlign(nn.Module):
         self.pool_mode = pool_mode
         self.aligned = aligned
 
-    def forward(self, input, rois):
+    def forward(self, input, rois, *, feat_hw=None):
         return roi_align(input, rois, self.output_size, self.spatial_scale, self.sampling_ratio, self.pool_mode,
-                         self.aligned)
+                         self.aligned, feat_hw=feat_hw)
 
     def __repr__(self):
         return (f"{self.__class__.__name__}(output_size={self.output_size}, spatial_scale={self.spatial_scale}, "

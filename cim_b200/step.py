@@ -72,6 +72,7 @@ class CIMHeadStep:
         self.anti = anti_noise_sampling
         self.p_seed = float(p_seed)
         self.n_props = None             # the device counts of the last run(): kept alive while its kernels may run
+        self.feat_hw = None             # the device image extents of the last run(), likewise
         self.order = order
         if rng not in ("hop", "stream"):
             raise ValueError("rng must be 'hop' or 'stream'")
@@ -167,7 +168,7 @@ class CIMHeadStep:
 
     # -------------------------------------------------------------------------------------
     def run(self, feat, rois, grad_out, packed_masks, seg_x, weight, bias, labels, labels_host=None, grad_scores=None,
-            mat=None, mid_hook=None, order=None, mask_meta=None, n_props=None):
+            mat=None, mid_hook=None, order=None, mask_meta=None, n_props=None, feat_hw=None):
         """feat [n_img,Cf,H,W] f32, rois [n_img*R,5] f32 grouped by image, grad_out [n_img*R,Cf,7,7]
         f32, packed_masks [n_img,R,words] i32, seg_x [n_img*R,D] f32, weight [2+2K,C+1,D],
         bias [2+2K,C+1], labels [n_img,C] f32 (labels_host is no longer needed: the sampling runs on the device).
@@ -185,6 +186,11 @@ class CIMHeadStep:
         pseudo labels, losses, PCL_loss, gradients; padding rows of all of them are 0).  Padding rows must hold finite
         seg_x, rois with the image's own index and finite coordinates, and grad_out rows of 0; the maps are computed
         for them but never read.  None: every image has R proposals.
+        feat_hw: image sizes of a batch of differently sized images (a host [n_img, 2] sequence / array / CPU tensor,
+        validated and copied, or a CUDA int32 [n_img, 2] tensor used as is; it may change from step to step).  feat is
+        then a canvas of the constructor's (feat_h, feat_w): image b occupies feat[b, :, :H_b, :W_b], and its roi_out
+        rows and grad_feat equal RoIAlign of that map alone (grad_feat is 0 outside it; the canvas there must be
+        finite).  Nothing else of the step depends on it.  None: every image fills the canvas.
 
         order (default: the constructor's):
           "graph"      the model's dependency order (model_builder.py:136-204): RoIAlign forward -> scoring heads ->
@@ -210,6 +216,7 @@ class CIMHeadStep:
         cur = torch.cuda.current_stream(dev)
         pcl_early = self.head_grads and grad_scores is None and mat is not None
         self.n_props = np_dev = _lib.n_props_arg(n_props, n_img, R, dev)
+        self.feat_hw = hw = _lib.feat_hw_arg(feat_hw, n_img, self.H, self.W, dev)
 
         def pcl(stream):
             # PCL_loss (model_builder.py:203) needs predict_cls and the cluster matrix only: 8 CTAs of pure latency;
@@ -234,9 +241,9 @@ class CIMHeadStep:
 
         def roi_fwd():
             with _nvtx("cim/roi_align_fwd"):
-                ck(L.cim_roi_align_fwd_prepared(P(feat), P(rois), None, P(self.roi_out), n_img, self.Cf, self.H,
-                                                self.W, n_img * R, 7, 7, self.scale, self.sr, self.aligned,
-                                                P(self.roi_ws), self.roi_ws.numel(), st), "cim_roi_align_fwd")
+                ck(L.cim_roi_align_fwd_prepared_ex(P(feat), P(rois), P(hw), None, P(self.roi_out), n_img, self.Cf,
+                                                   self.H, self.W, n_img * R, 7, 7, self.scale, self.sr, self.aligned,
+                                                   P(self.roi_ws), self.roi_ws.numel(), st), "cim_roi_align_fwd")
 
         def mine():
             self.ev_premine.record(cur)        # from here on the GPU is mostly idle until the hop is over
@@ -262,9 +269,9 @@ class CIMHeadStep:
             # the persistent RoIAlign forward is on the SMs before the overlap's tensor kernel asks for them -- which of
             # the two went first used to depend on launch timing (cfg3: 5.67 or 5.85 ms)
             with _nvtx("cim/roi_prepare"):
-                ck(L.cim_roi_align_prepare(P(rois), n_img, self.Cf, self.H, self.W, n_img * R, 7, 7, self.scale,
-                                           self.sr, self.aligned, P(self.roi_ws), self.roi_ws.numel(), st),
-                   "cim_roi_align_prepare")
+                ck(L.cim_roi_align_prepare_ex(P(rois), P(hw), n_img, self.Cf, self.H, self.W, n_img * R, 7, 7,
+                                              self.scale, self.sr, self.aligned, P(self.roi_ws), self.roi_ws.numel(),
+                                              st), "cim_roi_align_prepare")
             self.ev_prep.record(cur)
             roi_fwd()
             self.side.wait_event(self.ev_prep)
@@ -281,8 +288,8 @@ class CIMHeadStep:
             # the scoring GEMM (independent of the maps) runs on a side stream next to the overlap stage, whose small
             # serial helpers leave most of the GPU idle; RoI descriptors once per step, also off the critical path
             score_fwd(side_st, True)
-            ck(L.cim_roi_align_prepare(P(rois), n_img, self.Cf, self.H, self.W, n_img * R, 7, 7, self.scale, self.sr,
-                                       self.aligned, P(self.roi_ws), self.roi_ws.numel(), side_st),
+            ck(L.cim_roi_align_prepare_ex(P(rois), P(hw), n_img, self.Cf, self.H, self.W, n_img * R, 7, 7, self.scale,
+                                          self.sr, self.aligned, P(self.roi_ws), self.roi_ws.numel(), side_st),
                "cim_roi_align_prepare")
             overlap(st)
             cur.wait_stream(self.side)
@@ -350,9 +357,9 @@ class CIMHeadStep:
                                             st), "cim_score_heads_bwd")
                 reduce_work = cdist.allreduce_mean_async_(self.head_bucket)     # overlaps the RoIAlign backward
         with _nvtx("cim/roi_align_bwd"):
-            ck(L.cim_roi_align_bwd_prepared(P(grad_out), P(rois), None, P(self.grad_feat), n_img, self.Cf, self.H,
-                                            self.W, n_img * R, 7, 7, self.scale, self.sr, self.aligned,
-                                            P(self.roi_ws), self.roi_ws.numel(), st), "cim_roi_align_bwd")
+            ck(L.cim_roi_align_bwd_prepared_ex(P(grad_out), P(rois), P(hw), None, P(self.grad_feat), n_img, self.Cf,
+                                               self.H, self.W, n_img * R, 7, 7, self.scale, self.sr, self.aligned,
+                                               P(self.roi_ws), self.roi_ws.numel(), st), "cim_roi_align_bwd")
         if reduce_work is not None:
             reduce_work()                                       # current stream waits for the allreduce
         if tr is not None:
@@ -406,7 +413,7 @@ class CIMHeadStep:
         self.ustream.commit()
 
     # -------------------------------------------------------------------------------------
-    def alloc_host_io(self, mask_hw=None, crop_capacity_words=0, prefetch_depth=1):
+    def alloc_host_io(self, mask_hw=None, crop_capacity_words=0, prefetch_depth=1, ragged=False):
         """Pinned host buffers of the end-to-end call: inputs that originate on the host in the
         reference's pipeline (rois, labels: lib/roi_data/minibatch.py:45-61; proposal masks:
         the COB .mat files of tools/pre) and the step's results.  Device-side input buffers are
@@ -417,7 +424,11 @@ class CIMHeadStep:
         of the previous step, so the crop unpack can always run in that step's idle mining phase -- with eight ranks
         copying at once a rank's 60 MB take 2.5 ms instead of 1.3 (tools/h2d_bw.py) and the unpack used to slip behind
         the RoIAlign backward.  What run_host() finds in the pinned buffers at call t is then the input of step t + 2
-        (the first call also uses it for steps t and t + 1)."""
+        (the first call also uses it for steps t and t + 1).
+        ragged: a pinned hi_n_props int32 [n_img] (initialised to R) joins the inputs: the proposal counts of the step,
+        filled by the caller like hi_rois, validated when staged and carried with that step's rois, labels and masks
+        through the double buffer and the pre-stage (run(n_props=...) for what a padding row must hold; with crops,
+        mask_ops.batch_crops_host builds the wire format with empty crops for the padding rows)."""
         k, n_img, R, C1 = self.K, self.n_img, self.R, self.C + 1
         if prefetch_depth not in (1, 2) or (prefetch_depth == 2 and not crop_capacity_words):
             raise ValueError("prefetch_depth must be 1, or 2 with crop_capacity_words > 0")
@@ -425,6 +436,8 @@ class CIMHeadStep:
         pin = lambda shape, dt: torch.empty(shape, dtype=dt).pin_memory()
         self.hi_rois = pin((n_img * R, 5), torch.float32)
         self.hi_labels = pin((n_img, self.C), torch.float32)
+        self.ragged = bool(ragged)
+        self.hi_n_props = pin((n_img,), torch.int32).fill_(R) if self.ragged else None
         # masks arrive either as full bit masks (hi_masks) or, with crop_capacity_words > 0, as
         # bounding-box crops (mask_ops.MaskCrops: ~8x fewer bytes over PCIe) that the device unpacks
         self.crop_cap = int(crop_capacity_words)
@@ -458,6 +471,9 @@ class CIMHeadStep:
             self.di = [dict(rois=dv((n_img * R, 5), torch.float32), labels=dv((n_img, self.C), torch.float32),
                             masks=mk((n_img, R, self.words), dtype=torch.int32, device=self.dev),
                             ready=torch.cuda.Event(), free=torch.cuda.Event()) for _ in range(2)]
+            if self.ragged:
+                for buf in self.di:
+                    buf["n_props"] = dv((n_img,), torch.int32)
             if self.crop_cap:
                 for buf in self.di:
                     buf.update(crop_words=dv((self.crop_cap,), torch.int32), crop_meta=dv((n_img * R, 4), torch.int32),
@@ -475,8 +491,12 @@ class CIMHeadStep:
                                 crop_words=dv((self.crop_cap,), torch.int32), crop_meta=dv((n_img * R, 4), torch.int32),
                                 crop_off=dv((n_img * R,), torch.int64), n_words=0, valid=False,
                                 filled=torch.cuda.Event())
+                if self.ragged:
+                    self.pre["n_props"] = dv((n_img,), torch.int32)
                 self.copy_stream2 = torch.cuda.Stream(device=self.dev)
         self.h2d_bytes = sum(t.numel() * t.element_size() for t in (self.hi_rois, self.hi_labels))
+        if self.ragged:
+            self.h2d_bytes += self.hi_n_props.numel() * 4
         if not self.crop_cap:
             self.h2d_bytes += self.hi_masks.numel() * 4
         self.d2h_bytes = sum(t.numel() * t.element_size() for t in results + (self.ho_checksum,))
@@ -496,7 +516,7 @@ class CIMHeadStep:
 
     def wait_inputs_consumed(self):
         """Block until the last stage_host_inputs() has finished READING the pinned input buffers (hi_rois, hi_labels,
-        hi_masks / hi_crop_*).  The copies are asynchronous: refill those buffers for the following step only after
+        hi_masks / hi_crop_*, hi_n_props).  The copies are asynchronous: refill those buffers for the following step only after
         this returns (set_host_crops() calls it itself)."""
         if getattr(self, "_h2d_pending", False):
             self.h2d_ev.synchronize()
@@ -525,6 +545,10 @@ class CIMHeadStep:
         direct (prefetch_depth = 2 only): copy the pinned buffers straight into the device buffer, bypassing and
         invalidating the pre-stage (a step that was not prefetched)."""
         buf = self.di[self._slot ^ 1] if self._staged else self.di[self._slot]
+        if self.ragged:
+            n = self.hi_n_props.numpy()
+            if n.min() < 1 or n.max() > self.R:
+                raise ValueError(f"hi_n_props must lie in [1, {self.R}], got [{n.min()}, {n.max()}]")
 
         def kernels(after=None):
             with torch.cuda.stream(self.copy_stream):
@@ -561,6 +585,8 @@ class CIMHeadStep:
             """pinned input buffers -> dst (a device input buffer or the pre-stage); returns the crop word count"""
             dst["rois"].copy_(self.hi_rois, non_blocking=True)
             dst["labels"].copy_(self.hi_labels, non_blocking=True)
+            if self.ragged:
+                dst["n_props"].copy_(self.hi_n_props, non_blocking=True)
             n = 0
             if self.crop_cap:
                 n = self.n_crop_words
@@ -585,7 +611,7 @@ class CIMHeadStep:
                 # the input of this buffer's step arrived a step ago: device-to-device
                 self.copy_stream.wait_event(pre["filled"])
                 n = pre["n_words"]
-                for key in ("rois", "labels", "crop_meta", "crop_off"):
+                for key in ("rois", "labels", "crop_meta", "crop_off") + (("n_props",) if self.ragged else ()):
                     buf[key].copy_(pre[key], non_blocking=True)
                 buf["crop_words"][:n].copy_(pre["crop_words"][:n], non_blocking=True)
             else:
@@ -622,11 +648,12 @@ class CIMHeadStep:
         return self.results_host
 
     def run_host(self, feat, grad_out, seg_x, weight, bias, prefetch_next=True, grad_scores=None, mat=None,
-                 lag_results=False):
+                 lag_results=False, feat_hw=None):
         """End-to-end step: host rois / labels / bit-packed masks -> device, the step, results ->
-        host.  Every image has R proposals here (run() takes ragged batches; a ragged crop wire format, with empty
-        crops for the padding rows, is not implemented).  feat / seg_x / grad_out are produced on the device by the backbone, MaskFuse and
-        autograd in the real pipeline and therefore stay device tensors.
+        host.  With alloc_host_io(ragged=True) the proposal counts (hi_n_props) travel with the step's inputs and the
+        batch is ragged (run(n_props=...)).  feat / seg_x / grad_out are produced on the device by the backbone, MaskFuse
+        and autograd in the real pipeline and therefore stay device tensors; so does feat_hw, the image sizes of a
+        canvas-padded feat (run(feat_hw=...)), which goes straight through to run().
         With prefetch_next the copy of the NEXT step's inputs (whatever is in the pinned input
         buffers now) is enqueued on the copy stream first, so it overlaps this step's kernels;
         every call therefore moves one full set of inputs host->device."""
@@ -640,7 +667,8 @@ class CIMHeadStep:
             finish_stage = self.stage_host_inputs(defer_kernels=True)      # copies now, the other buffer
         cur_stream.wait_event(buf["ready"])
         self.run(feat, buf["rois"], grad_out, buf["masks"], seg_x, weight, bias, buf["labels"],
-                 None, grad_scores=grad_scores, mat=mat, mask_meta=buf.get("meta"),
+                 None, grad_scores=grad_scores, mat=mat, mask_meta=buf.get("meta"), n_props=buf.get("n_props"),
+                 feat_hw=feat_hw,
                  mid_hook=lambda: ((finish_stage(self.ev_premine) if finish_stage else None),
                                    (self._collect_results() if lag_results else None)))
         buf["free"].record(cur_stream)

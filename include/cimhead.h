@@ -30,9 +30,22 @@
  *   - every per-image quantity is computed for n_b, as running that image alone at R = n_b would: the detector
  *     softmax over its n_b proposals, keep_count = int(ceil(p_seed * n_b)) and big_thr = float32(0.9 * n_b)
  *     (cim_mine_image_constants), the containment counts over its n_b columns.
- * RoIAlign and the mask overlap maps have no _ex form: their padding rows are computed and nobody reads them.  Give
- * padding rois their own image index and finite coordinates, and grad_out rows of 0 at padding (what the scoring
- * backward's zero grad_x rows produce through a per-ROI head).  Zero padding masks let the overlap kernel skip them.
+ * RoIAlign and the mask overlap maps have no proposal-count form: their padding rows are computed and nobody reads
+ * them.  Give padding rois their own image index and finite coordinates, and grad_out rows of 0 at padding (what the
+ * scoring backward's zero grad_x rows produce through a per-ROI head).  Zero padding masks let the overlap kernel skip
+ * them.
+ *
+ * Images of different sizes (the RoIAlign _ex entry points).  feat [B,C,H,W] is a CANVAS: image b occupies the top
+ * left [0, H_b) x [0, W_b) of its plane.  feat_hw is a device int32 [B][2] array of the (H_b, W_b), 4-byte aligned;
+ * NULL means (H, W) for every image, and each RoIAlign entry point without _ex is its NULL case.  The kernels clamp
+ * the device values to [1, H] x [1, W].  Contract:
+ *   - the outputs of image b's rois (forward, backward, MaskFuse forward and backward) equal RoIAlign of
+ *     feat[b, :, :H_b, :W_b] alone: the border rule (a sample is clamped to row H_b - 1, dropped beyond H_b; the
+ *     same for columns) uses the image's extent, not the canvas';
+ *   - grad_feat is exactly 0 outside the extents;
+ *   - the canvas outside the extents must hold FINITE values: taps of weight 0 read it (0 * inf = NaN).  Its contents
+ *     change no output.  (Padding rows of a ragged batch follow the same rule: finite seg_x.)
+ * RoIPool has no _ex form: no shipped configuration selects it (DESIGN.md section 4.12).
  */
 #ifndef CIMHEAD_H
 #define CIMHEAD_H
@@ -46,7 +59,7 @@ extern "C" {
 
 typedef struct CUstream_st *cim_stream_t;   /* == cudaStream_t */
 
-#define CIM_ABI_VERSION 4
+#define CIM_ABI_VERSION 5
 
 enum {
     CIM_OK = 0,
@@ -80,6 +93,10 @@ unsigned cim_get_debug_flags(void);
  * sub-ROIs or a negative CIM_ERR_* code. */
 int cim_debug_roi_window_plan(const float *rois, int K, int B, int H, int W, float scale, int sampling_ratio,
                               int aligned, int *desc_out, int *key_out, int cap, int *flag_out, int *geom_out);
+/* The same with per-image extents: feat_hw HOST int32 [B][2] (NULL: the canvas), clamped as the device clamps them. */
+int cim_debug_roi_window_plan_ex(const float *rois, const int32_t *feat_hw, int K, int B, int H, int W, float scale,
+                                 int sampling_ratio, int aligned, int *desc_out, int *key_out, int cap, int *flag_out,
+                                 int *geom_out);
 
 /* ------------------------------------------------------------------ ROI operators
  * Replace mmcv.ops.RoIAlign / RoIPool as imported by lib/ops/__init__.py:6 and called at
@@ -142,6 +159,19 @@ int cim_roi_align_bwd_prepared(const float *grad_out, const float *rois, const f
                                int B, int C, int H, int W, int K, int oh, int ow,
                                float spatial_scale, int sampling_ratio, int aligned,
                                void *workspace, size_t workspace_bytes, cim_stream_t stream);
+/* Per-image extents (see the top of this file): feat_hw device int32 [B][2] or NULL.  The _prepared_ex calls take the
+ * feat_hw of their prepare_ex call (same pointer, same contents).  Same workspace as the calls above. */
+int cim_roi_align_prepare_ex(const float *rois, const int32_t *feat_hw, int B, int C, int H, int W, int K, int oh,
+                             int ow, float spatial_scale, int sampling_ratio, int aligned,
+                             void *workspace, size_t workspace_bytes, cim_stream_t stream);
+int cim_roi_align_fwd_prepared_ex(const float *feat, const float *rois, const int32_t *feat_hw, const float *masks7,
+                                  float *out, int B, int C, int H, int W, int K, int oh, int ow,
+                                  float spatial_scale, int sampling_ratio, int aligned,
+                                  void *workspace, size_t workspace_bytes, cim_stream_t stream);
+int cim_roi_align_bwd_prepared_ex(const float *grad_out, const float *rois, const int32_t *feat_hw,
+                                  const float *masks7, float *grad_feat, int B, int C, int H, int W, int K, int oh,
+                                  int ow, float spatial_scale, int sampling_ratio, int aligned,
+                                  void *workspace, size_t workspace_bytes, cim_stream_t stream);
 
 /* RoIPool: lib/model/roi_pooling/src/roi_pooling_kernel.cu:24-93 (fwd), :128-203 (bwd).
  * argmax [K,C,oh,ow] int32 = index inside the H*W plane, -1 for an empty bin. */
