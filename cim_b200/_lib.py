@@ -13,7 +13,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libcimhead.so")
-ABI_VERSION = 5
+ABI_VERSION = 6
 MAX_LAYERS = 4
 OVERLAP_ALGOS = {"auto": 0, "popc": 1, "tensor": 2}
 #: cim_set_debug_flags bits (include/cimhead.h): diagnostic kernel selection for A/B timing and bit-identity tests
@@ -71,6 +71,7 @@ _SIGNATURES = {
     "cim_mask_meta": (_I, [_P, _I, _I, _I64, _I, _P, _SZ, _P]),
     "cim_mask_overlap_meta": (_I, [_P, _P, _I, _I, _I64, _I, _P, _P, _P, _P, _P, _SZ, _I, _P]),
     "cim_mask_pair_ratio": (_I, [_P, _P, _I, _I, _I64, _I, _P, _P, _P, _P, _P]),
+    "cim_mask_rle": (_I, [_P, _I, _I, _I64, _I, _I, _I, _P, _P, _P, _I, _P, _I64, _P, _P, _P, _P, _P, _P]),
     "cim_score_heads_workspace_bytes": (_SZ, [_I, _I, _I, _I, _I]),
     "cim_score_heads": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _SZ, _P]),
     "cim_score_heads_bwd_workspace_bytes": (_SZ, [_I, _I, _I, _I, _I]),

@@ -268,6 +268,72 @@ def mask_overlap_maps(masks):
     return mask_overlap(mask_pack(masks))
 
 
+# ------------------------------------------------------------------ COCO RLE of selected masks
+def rle_chars_cap(n_slots, height, width):
+    """Default string capacity of mask_rle: 4 * (height + width) characters per slot, enough for masks with a couple
+    of runs per column (need[0] tells the exact total)."""
+    return int(n_slots) * 4 * (int(height) + int(width))
+
+
+def _mask_rle_into(packed, sel_count, sel_idx, height, width, mask_hw, kb_per_row, chars, off, len_, area, bbox,
+                   need):
+    n_img, R, words = packed.shape
+    cap = sel_idx.shape[1]
+    with torch.cuda.device(packed.device):
+        rc = _lib.lib().cim_mask_rle(_lib.ptr(packed), n_img, R, words, int(height), int(width), int(kb_per_row),
+                                     _lib.ptr(mask_hw), _lib.ptr(sel_count), _lib.ptr(sel_idx), cap, _lib.ptr(chars),
+                                     chars.numel(), _lib.ptr(off), _lib.ptr(len_), _lib.ptr(area), _lib.ptr(bbox),
+                                     _lib.ptr(need), _lib.stream_ptr(packed.device))
+    _lib.check(rc, "cim_mask_rle")
+
+
+def _rle_args(packed, sel_count, sel_idx, height, width, mask_hw, kb_per_row):
+    _lib.require_cuda(packed, "packed", torch.int32)
+    _lib.require_cuda(sel_count, "sel_count", torch.int32)
+    _lib.require_cuda(sel_idx, "sel_idx", torch.int32)
+    if kb_per_row is None:
+        kb_per_row = int(getattr(packed, "cim_kb_per_row", 0))
+    if packed.dim() == 2:
+        packed = packed.unsqueeze(0)
+    if packed.dim() != 3:
+        raise ValueError("packed must be [N, words] or [n_img, N, words]")
+    n_img = packed.shape[0]
+    if sel_count.shape != (n_img,) or sel_idx.dim() != 2 or sel_idx.shape[0] != n_img:
+        raise ValueError(f"sel_count must be [{n_img}] and sel_idx [{n_img}, cap]")
+    mask_hw = _lib.feat_hw_arg(mask_hw, n_img, height, width, packed.device)
+    return packed.contiguous(), sel_count.contiguous(), sel_idx.contiguous(), mask_hw, int(kb_per_row)
+
+
+def mask_rle(packed, sel_count, sel_idx, height, width, mask_hw=None, kb_per_row=None, chars_cap=None):
+    """Selected bit masks as COCO compressed RLE on the device (cim_mask_rle): what pycocotools.mask.encode returns
+    as 'counts', with mask.area and mask.toBbox, for every slot of a selection.
+      packed [n_img, R, words] int32 on a height x width canvas (mask_pack / unpack_crops, flat or tiled order;
+        kb_per_row = W // 16 for tiled, 0 for flat, None = what mask_pack / unpack_crops recorded);
+      sel_count [n_img], sel_idx [n_img, cap] int32 CUDA tensors (count / idx of postproc.detections_batched): slot
+        (b, j), j < min(sel_count[b], cap), selects mask sel_idx[b, j] of image b;
+      mask_hw: per-image native (h, w) [n_img, 2] (None: the canvas); set bits outside it are ignored.
+    Returns device tensors (chars uint8 [chars_cap], off int64 [n_img, cap], len int32 [n_img, cap], area int32
+    [n_img, cap], bbox int32 [n_img, cap, 4] (x, y, w, h), need int64 [2]): slot (b, j)'s string is
+    chars[off : off + len] when off + len <= chars_cap; need[0] = total characters, need[1] = selected indices
+    outside [0, R) (their slots get len 0).  No host synchronisation.  chars_cap None: rle_chars_cap(...)."""
+    packed, sel_count, sel_idx, mask_hw, kb_per_row = _rle_args(packed, sel_count, sel_idx, height, width, mask_hw,
+                                                                kb_per_row)
+    n_img, cap = sel_idx.shape
+    if chars_cap is None:
+        chars_cap = rle_chars_cap(n_img * cap, height, width)
+    if int(chars_cap) < 0:
+        raise ValueError("chars_cap must be >= 0")
+    dev = packed.device
+    chars = torch.empty(int(chars_cap), dtype=torch.uint8, device=dev)
+    off = torch.empty((n_img, cap), dtype=torch.int64, device=dev)
+    len_ = torch.empty((n_img, cap), dtype=torch.int32, device=dev)
+    area = torch.empty((n_img, cap), dtype=torch.int32, device=dev)
+    bbox = torch.empty((n_img, cap, 4), dtype=torch.int32, device=dev)
+    need = torch.empty(2, dtype=torch.int64, device=dev)
+    _mask_rle_into(packed, sel_count, sel_idx, height, width, mask_hw, kb_per_row, chars, off, len_, area, bbox, need)
+    return chars, off, len_, area, bbox, need
+
+
 # ------------------------------------------------------------------ offline callers of lib/utils/mask_utils.py
 _RATIO_MODES = {"iou": 0, "asymmetric": 1, "inside": 2, "outside": 3}
 

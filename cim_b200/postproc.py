@@ -8,14 +8,16 @@
   TestScoreMean(n_passes)                      lib/core/test.py:149-226 (TEST.BBOX_AUG, SCORE_HEUR 'AVG')
   detections_batched(...)                      :57-110 for a batch of images, results left on the device
   results_with_nms_and_limit_batched(...)      the same, as the reference's per-image host lists
+  segms_batched(packed, detections, ...)       the detections' proposal masks as pycocotools.mask.encode dicts,
+                                               with mask.area / mask.toBbox, per class like cls_boxes
 
-All arithmetic runs in libcimhead.so (cim_test_scores[_tta] / cim_box_nms[_batched] / cim_box_detections); there is
-no CPU path.
+All arithmetic runs in libcimhead.so (cim_test_scores[_tta] / cim_box_nms[_batched] / cim_box_detections,
+cim_mask_rle); there is no CPU path.
 """
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, mask_ops
 
 
 def test_scores(scores, k):
@@ -204,3 +206,73 @@ def results_with_nms_and_limit(scores, boxes, score_thresh=1e-5, nms_thresh=0.3,
         raise ValueError("scores must be [n, C] and boxes [n, 4]")
     return results_with_nms_and_limit_batched(scores[None], boxes[None], score_thresh, nms_thresh,
                                               detections_per_im)[0]
+
+
+def segms_batched(packed, detections, height, width, n_classes, mask_hw=None, kb_per_row=None):
+    """The proposal masks of a batch's detections as COCO compressed RLE, on the device (cim_mask_rle), in the layout
+    of results_with_nms_and_limit_batched.  packed [B, R, words]: the proposal bit masks on a height x width canvas
+    (mask_ops.mask_pack / unpack_crops; kb_per_row as mask_ops.mask_rle takes it); detections: what
+    detections_batched / box_detections returned for the same B images and R proposals; mask_hw: per-image native
+    (h, w) [B, 2] (None: the canvas).  Returns a list of B tuples (cls_segms, cls_areas, cls_bboxes), each a list of
+    n_classes + 1 entries, entry 0 empty, aligned with cls_boxes / cls_inds: cls_segms[j] = [{'size': [h, w],
+    'counts': bytes}, ...] (pycocotools.mask.encode), cls_areas[j] uint32 [k] (mask.area), cls_bboxes[j] float64
+    [k, 4] (mask.toBbox).  One pinned copy and one synchronisation; a second round with the exact string capacity
+    only when the first was too small.  Raises when a detection names a proposal outside [0, R), or when an image
+    has more detections than the detection lists hold."""
+    count, cls, idx = detections[0], detections[1], detections[2]
+    packed, count, idx, mask_hw_d, kb_per_row = mask_ops._rle_args(packed, count, idx, height, width, mask_hw,
+                                                                   kb_per_row)
+    _lib.require_cuda(cls, "cls", torch.int32)
+    b, cap = idx.shape
+    e = b * cap
+    dev = packed.device
+    stream = torch.cuda.current_stream(dev)
+    def fetch(chars_cap):
+        # need [2] i64 | bbox [e, 4] i32 | off [e] i64 | len, area, cls [e] i32 | count [b] i32 | hw [b, 2] i32 | chars
+        o = np.cumsum([0, 16, 16 * e, 8 * e, 4 * e, 4 * e, 4 * e, 4 * b, 8 * b, chars_cap])
+        buf = torch.empty(int(o[-1]), dtype=torch.uint8, device=dev)
+        part = lambda i, dt: buf[o[i]:o[i + 1]].view(dt)
+        need, bbox, off, len_, area = (part(0, torch.int64), part(1, torch.int32), part(2, torch.int64),
+                                       part(3, torch.int32), part(4, torch.int32))
+        part(5, torch.int32).copy_(cls.reshape(-1))
+        part(6, torch.int32).copy_(count)
+        hw = part(7, torch.int32).view(b, 2)
+        for c, lim in enumerate((height, width)):             # as the kernel clamps them
+            if mask_hw_d is None:
+                hw[:, c].fill_(lim)
+            else:
+                hw[:, c].copy_(mask_hw_d[:, c].clamp(1, lim))
+        mask_ops._mask_rle_into(packed, count, idx, height, width, mask_hw_d, kb_per_row, part(8, torch.uint8),
+                                off, len_, area, bbox, need)
+        host = torch.empty(buf.shape, dtype=torch.uint8, pin_memory=True)
+        host.copy_(buf, non_blocking=True)
+        stream.synchronize()
+        h = host.numpy()
+        hp = lambda i, dt: h[o[i]:o[i + 1]].view(dt)
+        return (hp(0, np.int64), hp(1, np.int32).reshape(b, cap, 4), hp(2, np.int64).reshape(b, cap),
+                hp(3, np.int32).reshape(b, cap), hp(4, np.int32).reshape(b, cap), hp(5, np.int32).reshape(b, cap),
+                hp(6, np.int32), hp(7, np.int32).reshape(b, 2), hp(8, np.uint8))
+
+    chars_cap = mask_ops.rle_chars_cap(e, height, width)
+    need, bbox, off, len_, area, cls_h, count_h, sizes, chars = fetch(chars_cap)
+    if need[1]:
+        raise ValueError(f"{int(need[1])} detections name a proposal outside [0, {packed.shape[1]})")
+    if b and int(count_h.max()) > cap:
+        raise ValueError(f"an image has {int(count_h.max())} detections but the detection lists hold {cap}: "
+                         "call box_detections with cap >= count")
+    if need[0] > chars_cap:
+        need, bbox, off, len_, area, cls_h, count_h, sizes, chars = fetch(int(need[0]))
+    results = []
+    for i in range(b):
+        k = int(count_h[i])
+        size = [int(sizes[i, 0]), int(sizes[i, 1])]
+        bounds = np.searchsorted(cls_h[i, :k], np.arange(n_classes + 1))
+        segms, areas, boxes = [[]], [[]], [[]]
+        for j in range(n_classes):
+            lo, hi = bounds[j], bounds[j + 1]
+            segms.append([{"size": list(size), "counts": chars[off[i, s]:off[i, s] + len_[i, s]].tobytes()}
+                          for s in range(lo, hi)])
+            areas.append(area[i, lo:hi].astype(np.uint32))
+            boxes.append(bbox[i, lo:hi].astype(np.float64))
+        results.append((segms, areas, boxes))
+    return results

@@ -59,7 +59,7 @@ extern "C" {
 
 typedef struct CUstream_st *cim_stream_t;   /* == cudaStream_t */
 
-#define CIM_ABI_VERSION 5
+#define CIM_ABI_VERSION 6
 
 enum {
     CIM_OK = 0,
@@ -288,6 +288,28 @@ int cim_mask_overlap_meta(const uint32_t *packed, const void *meta, int n_img, i
  *   area_a [na], area_b [nb] int32 (outputs: the row popcounts).  words * 32 <= 2^24. */
 int cim_mask_pair_ratio(const uint32_t *packed_a, const uint32_t *packed_b, int na, int nb, int64_t words, int mode,
                         float *ratio, int32_t *inter, int32_t *area_a, int32_t *area_b, cim_stream_t stream);
+
+/* Selected masks as COCO compressed RLE: what pycocotools.mask.encode / area / toBbox return (common/maskApi.c
+ * rleEncode + rleToString, rleArea, rleToBbox) for the detections of cim_box_detections, which name proposal masks.
+ *   packed [n_img, R, words]: bit masks on an H x W canvas in the flat order (kb_per_row = 0; words >= ceil(H*W/32))
+ *     or the tiled 8 x 16 order (kb_per_row = W/16, H % 8 == 0, W % 16 == 0), as cim_mask_pack[_tiled] write them;
+ *   mask_hw [n_img][2] int32 (may be NULL = the canvas): image b's native (h, w), clamped to [1, H] x [1, W]; its
+ *     mask is the top-left h x w of the canvas and set bits outside it are ignored;
+ *   sel_count [n_img], sel_idx [n_img, cap] int32 (the count / det_idx of cim_box_detections): slot (b, j) with
+ *     j < min(sel_count[b], cap) selects mask sel_idx[b, j] of image b.
+ * Per slot: the string (column-major counts over h x w, rleToString's characters, no terminator) at chars[off, off +
+ *   len), off [n_img, cap] int64 = exclusive scan of len in slot order, len [n_img, cap] int32; area [n_img, cap]
+ *   int32 (rleArea, may be NULL); bbox [n_img, cap, 4] int32 (x, y, w, h: rleToBbox, the tight box of the ones, all 0
+ *   for an empty mask; 16-byte aligned; may be NULL).  Unused slots and selected indices outside [0, R) get len = 0,
+ *   area 0 and box 0.  need [2] int64: need[0] = total characters, need[1] = selected indices outside [0, R).
+ *   Offsets, lengths, areas, boxes and need are always written; a string is written only when off + len <=
+ *   chars_cap (chars may be NULL when chars_cap == 0), so a caller that reads need[0] can size a second call exactly.
+ * Three launches (length pass, scan of the lengths, emit pass), no host synchronisation, no workspace, deterministic
+ * output.  H * W <= 2^31 - 1. */
+int cim_mask_rle(const uint32_t *packed, int n_img, int R, int64_t words, int H, int W, int kb_per_row,
+                 const int32_t *mask_hw, const int32_t *sel_count, const int32_t *sel_idx, int cap, uint8_t *chars,
+                 int64_t chars_cap, int64_t *off, int32_t *len, int32_t *area, int32_t *bbox, int64_t *need,
+                 cim_stream_t stream);
 
 /* ------------------------------------------------------------------ scoring heads
  * Replace heads.cls_iou_model.forward (lib/modeling/heads.py:194-219): n_heads = 2 + 2*K
