@@ -13,7 +13,7 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libcimhead.so")
-ABI_VERSION = 6
+ABI_VERSION = 7
 MAX_LAYERS = 4
 OVERLAP_ALGOS = {"auto": 0, "popc": 1, "tensor": 2}
 #: cim_set_debug_flags bits (include/cimhead.h): diagnostic kernel selection for A/B timing and bit-identity tests
@@ -78,6 +78,11 @@ _SIGNATURES = {
     "cim_score_heads_bwd": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _SZ, _P]),
     "cim_score_heads_ex": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _SZ, _P]),
     "cim_score_heads_bwd_ex": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _SZ, _P]),
+    "cim_score_heads_compact_workspace_bytes": (_SZ, [_I, _I, _I, _I, _I, _I]),
+    "cim_score_heads_compact": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P, _SZ, _P]),
+    "cim_score_heads_bwd_compact_workspace_bytes": (_SZ, [_I, _I, _I, _I, _I, _I]),
+    "cim_score_heads_bwd_compact": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P, _SZ, _P]),
+    "cim_debug_compact_row_map": (_I, [_P, _I, _I, _I, _P]),
     "cim_head_losses": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _F, _F, _F, _P]),
     "cim_pcl_loss": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _F, _I, _P]),
     "cim_pcl_loss_ex": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _I, _P]),
@@ -170,6 +175,12 @@ def n_props_arg(n_props, n_img, R, device):
         if n_props.numel() != n_img or n_props.dim() != 1:
             raise ValueError(f"n_props must have shape [{n_img}], got {tuple(n_props.shape)}")
         return n_props.contiguous()
+    return torch.from_numpy(host_counts(n_props, n_img, R)).to(device, non_blocking=True)
+
+
+def host_counts(n_props, n_img, R):
+    """Validated host copy of proposal counts (a sequence, numpy array or CPU tensor: integers in [1, R], shape
+    [n_img]) -> int32 numpy array."""
     a = n_props.numpy() if isinstance(n_props, torch.Tensor) else np.asarray(n_props)
     if a.dtype.kind not in "iu":
         raise TypeError(f"n_props must hold integers, got {a.dtype}")
@@ -177,7 +188,30 @@ def n_props_arg(n_props, n_img, R, device):
         raise ValueError(f"n_props must have shape [{n_img}], got {a.shape}")
     if a.size and (a.min() < 1 or a.max() > R):
         raise ValueError(f"n_props must lie in [1, {R}], got [{a.min()}, {a.max()}]")
-    return torch.from_numpy(a.astype(np.int32)).to(device, non_blocking=True)
+    return a.astype(np.int32)
+
+
+def compact_rows_arg(n_props, n_img, R, device):
+    """The counts of a compact ragged batch -> (CUDA int32 [n_img] counts on `device`, N = their sum).  Image b's
+    proposals are then rows [off_b, off_b + n_b) of the per-proposal tensors, off_b = n_0 + ... + n_{b-1}.  N sizes
+    host-side tensors, so the counts must come from the host (a sequence, numpy array or CPU tensor, validated as by
+    n_props_arg); a CUDA tensor is refused, because reading it would cost a synchronisation."""
+    if n_props is None:
+        raise ValueError("a compact batch needs its proposal counts")
+    if isinstance(n_props, torch.Tensor) and n_props.device.type != "cpu":
+        raise ValueError("the counts of a compact batch must be on the host (N = their sum sizes the tensors); "
+                         f"got a tensor on {n_props.device}")
+    a = host_counts(n_props, n_img, R)
+    return torch.from_numpy(a).to(device, non_blocking=True), int(a.sum(dtype=np.int64))
+
+
+def compact_row_map(n_props, n_img, R, N):
+    """cim_debug_compact_row_map (host, no GPU): padded row of each compact row, -1 past the counts' sum."""
+    a = None if n_props is None else np.ascontiguousarray(n_props, dtype=np.int32)
+    out = np.empty(N, np.int32)
+    check(lib().cim_debug_compact_row_map(a.ctypes.data_as(C.c_void_p) if a is not None else None, n_img, R, N,
+                                          out.ctypes.data_as(C.c_void_p)), "cim_debug_compact_row_map")
+    return out
 
 
 def feat_hw_arg(feat_hw, B, H, W, device):

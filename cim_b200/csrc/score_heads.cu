@@ -9,22 +9,27 @@
 //   heads 2+K..2+2K-1 (refine_iou): sigmoid                                      (heads.py:216)
 // fp32 FFMA accumulation (TF32 would miss the 1e-5 parity bar).
 #include "common.cuh"
+#include "ragged.cuh"
 
 // score_heads_tc.cu: 3xTF32 tcgen05 + TMA path
 bool cim_score_tc_eligible(long long M, int D, int C1, int n_ref);
 size_t cim_score_tc_workspace_bytes(int D, int C1, int n_ref);
 int cim_score_tc_launch(const float *x, const float *weight, const float *bias, float *scores, long long M, int D,
-                        int C1, int n_ref, void *workspace, cudaStream_t st);
+                        int C1, int n_ref, void *workspace, cudaStream_t st, const int32_t *row_map,
+                        long long M_out);
 
 namespace {
 
 constexpr int BM = 128, BN = 64, BK = 16;
 constexpr int APITCH = BM + 4, BPITCH = BN + 4;
 
-// logits[h][m][c] = sum_k x[m][k] * w[h*C1 + c][k] + bias[h*C1 + c]
+// logits[h][m][c] = sum_k x[m][k] * w[h*C1 + c][k] + bias[h*C1 + c].  REMAP (compact ragged rows, ragged.cuh): row m
+// goes to row row_map[m] of heads of M_out rows, nowhere for row_map[m] < 0.
+template <bool REMAP>
 __global__ void __launch_bounds__(256)
 score_gemm_kernel(const float *__restrict__ x, const float *__restrict__ w, const float *__restrict__ bias,
-                  float *__restrict__ out, int M, int N, int D, int C1) {
+                  float *__restrict__ out, int M, int N, int D, int C1, const int32_t *__restrict__ row_map,
+                  int M_out) {
     __shared__ __align__(16) float As[BK][APITCH];
     __shared__ __align__(16) float Bs[BK][BPITCH];
     const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
@@ -88,25 +93,38 @@ score_gemm_kernel(const float *__restrict__ x, const float *__restrict__ w, cons
     for (int i = 0; i < 8; ++i) {
         const int m = m0 + ty * 8 + i;
         if (m >= M) continue;
+        int out_row = m, out_rows = M;
+        if constexpr (REMAP) {
+            out_row = row_map[m];
+            out_rows = M_out;
+            if (out_row < 0) continue;
+        }
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const int n = n0 + tx * 4 + j;
             if (n >= N) continue;
             const int h = n / C1, c = n - h * C1;
-            out[((size_t)h * M + m) * C1 + c] = acc[i][j] + __ldg(bias + n);
+            out[((size_t)h * out_rows + out_row) * C1 + c] = acc[i][j] + __ldg(bias + n);
         }
     }
 }
 
 // softmax over classes / sigmoid, in place, one thread per (head, row); the detector head (1)
-// is left as logits for the column pass below.
-__global__ void score_row_act_kernel(float *__restrict__ s, int M, int C1, int K) {
+// is left as logits for the column pass below.  REMAP: M compact rows, whose rows in heads of M_out rows row_map gives.
+template <bool REMAP>
+__global__ void score_row_act_kernel(float *__restrict__ s, int M, int C1, int K, const int32_t *__restrict__ row_map,
+                                     int M_out) {
     const int nheads = 2 + 2 * K;
     const long long idx = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (idx >= (long long)nheads * M) return;
     const int h = (int)(idx / M);
     if (h == 1) return;
     float *row = s + (size_t)idx * C1;
+    if constexpr (REMAP) {
+        const int r = row_map[idx - (long long)h * M];
+        if (r < 0) return;
+        row = s + ((size_t)h * M_out + r) * C1;
+    }
     if (h == 0 || h < 2 + K) {
         float mx = -INFINITY;
         for (int c = 0; c < C1; ++c) mx = fmaxf(mx, row[c]);
@@ -171,6 +189,39 @@ CIM_API size_t cim_score_heads_workspace_bytes(int n_img, int R, int D, int C1, 
     return cim_score_tc_workspace_bytes(D, C1, K);          // W_hi / W_lo of the tensor-core path
 }
 
+// the FFMA / tensor-core GEMM + activations into padded scores [nheads, n_img*R, C1]: x has n_img*R rows, or with a
+// row map (compact ragged rows) M = N rows
+static int score_heads_run(const float *x, const float *weight, const float *bias, float *scores,
+                           const int32_t *n_props, int n_img, int R, long long M, const int32_t *row_map, int D, int C1,
+                           int K, void *workspace, size_t ws_bytes, size_t tc_ws_bytes, cudaStream_t st) {
+    const int nheads = 2 + 2 * K, N = nheads * C1;
+    const long long M_out = (long long)n_img * R;
+    const dim3 col_grid((unsigned)C1, (unsigned)n_img);
+    // tensor cores (3xTF32, fp32-accurate) when the shape allows and the caller gave the workspace;
+    // CIM_DBG_SCORE_FFMA forces the FFMA kernel (tuning / A-B aid)
+    if (!(cim_get_debug_flags() & CIM_DBG_SCORE_FFMA) && cim_score_tc_eligible(M, D, C1, K) && workspace &&
+        ws_bytes >= tc_ws_bytes) {
+        int rc2 = cim_score_tc_launch(x, weight, bias, scores, M, D, C1, K, workspace, st, row_map, M_out);
+        if (rc2) return rc2;
+        score_col_softmax_kernel<<<col_grid, 256, 0, st>>>(scores, n_props, M_out, nheads, R, C1);
+        return cim_launch_status();
+    }
+    dim3 grid((unsigned)((M + BM - 1) / BM), (unsigned)((N + BN - 1) / BN));
+    if (row_map) score_gemm_kernel<true><<<grid, 256, 0, st>>>(x, weight, bias, scores, (int)M, N, D, C1, row_map, (int)M_out);
+    else score_gemm_kernel<false><<<grid, 256, 0, st>>>(x, weight, bias, scores, (int)M, N, D, C1, nullptr, 0);
+    int rc = cim_launch_status();
+    if (rc) return rc;
+    const long long rows = (long long)nheads * M;
+    if (row_map)
+        score_row_act_kernel<true><<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(scores, (int)M, C1, K, row_map,
+                                                                                   (int)M_out);
+    else
+        score_row_act_kernel<false><<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(scores, (int)M, C1, K, nullptr, 0);
+    if ((rc = cim_launch_status())) return rc;
+    score_col_softmax_kernel<<<col_grid, 256, 0, st>>>(scores, n_props, M_out, nheads, R, C1);
+    return cim_launch_status();
+}
+
 CIM_API int cim_score_heads_ex(const float *x, const float *weight, const float *bias, float *scores,
                                const int32_t *n_props, int n_img, int R, int D, int C1, int K, void *workspace,
                                size_t ws_bytes, cim_stream_t stream) {
@@ -182,26 +233,38 @@ CIM_API int cim_score_heads_ex(const float *x, const float *weight, const float 
     cudaStream_t st = (cudaStream_t)stream;
     const long long M = (long long)n_img * R;
     if (M > (1LL << 30)) return CIM_ERR_SHAPE;
-    const int nheads = 2 + 2 * K, N = nheads * C1;
-    const dim3 col_grid((unsigned)C1, (unsigned)n_img);
-    // tensor cores (3xTF32, fp32-accurate) when the shape allows and the caller gave the workspace;
-    // CIM_DBG_SCORE_FFMA forces the FFMA kernel (tuning / A-B aid)
-    if (!(cim_get_debug_flags() & CIM_DBG_SCORE_FFMA) && cim_score_tc_eligible(M, D, C1, K) && workspace &&
-        ws_bytes >= cim_score_tc_workspace_bytes(D, C1, K)) {
-        int rc2 = cim_score_tc_launch(x, weight, bias, scores, M, D, C1, K, workspace, st);
-        if (rc2) return rc2;
-        score_col_softmax_kernel<<<col_grid, 256, 0, st>>>(scores, n_props, M, nheads, R, C1);
-        return cim_launch_status();
-    }
-    dim3 grid((unsigned)((M + BM - 1) / BM), (unsigned)((N + BN - 1) / BN));
-    score_gemm_kernel<<<grid, 256, 0, st>>>(x, weight, bias, scores, (int)M, N, D, C1);
-    int rc = cim_launch_status();
+    return score_heads_run(x, weight, bias, scores, n_props, n_img, R, M, nullptr, D, C1, K, workspace, ws_bytes,
+                           cim_score_tc_workspace_bytes(D, C1, K), st);
+}
+
+// compact ragged rows: the tensor-core workspace, then the row map (ragged.cuh), each 256-byte aligned
+static size_t tc_part_bytes(int D, int C1, int K) {
+    return (cim_score_tc_workspace_bytes(D, C1, K) + 255) & ~(size_t)255;
+}
+
+CIM_API size_t cim_score_heads_compact_workspace_bytes(int n_img, int R, int N, int D, int C1, int K) {
+    (void)R;
+    if (n_img <= 0 || N <= 0 || D <= 0 || C1 <= 0 || K < 0) return 256;
+    return 256 + tc_part_bytes(D, C1, K) + compact_map_bytes(n_img, N);
+}
+
+CIM_API int cim_score_heads_compact(const float *x, const float *weight, const float *bias, float *scores,
+                                    const int32_t *n_props, int n_img, int R, int N, int D, int C1, int K,
+                                    void *workspace, size_t ws_bytes, cim_stream_t stream) {
+    if (!x || !weight || !bias || !scores || !workspace) return CIM_ERR_ARG;
+    if (n_img <= 0 || R <= 0 || N <= 0 || D <= 0 || C1 <= 0 || K < 0 || K > 8) return CIM_ERR_ARG;
+    if (!cim_aligned(x, 16) || !cim_aligned(weight, 16) || !cim_aligned(n_props, 4)) return CIM_ERR_ALIGN;
+    if (n_img > 65535 || C1 > 65535) return CIM_ERR_SHAPE;
+    if ((long long)n_img * R > (1LL << 30) || N > n_img * R) return CIM_ERR_SHAPE;
+    if (ws_bytes < cim_score_heads_compact_workspace_bytes(n_img, R, N, D, C1, K)) return CIM_ERR_WORKSPACE;
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned char *base = reinterpret_cast<unsigned char *>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+    unsigned char *map_ws = base + tc_part_bytes(D, C1, K);
+    int rc = compact_row_map_launch(n_props, n_img, R, N, map_ws, st);
     if (rc) return rc;
-    const long long rows = (long long)nheads * M;
-    score_row_act_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, st>>>(scores, (int)M, C1, K);
-    if ((rc = cim_launch_status())) return rc;
-    score_col_softmax_kernel<<<col_grid, 256, 0, st>>>(scores, n_props, M, nheads, R, C1);
-    return cim_launch_status();
+    // the tensor-core operands at `base` (cim_score_tc_launch aligns `workspace` the same way)
+    return score_heads_run(x, weight, bias, scores, n_props, n_img, R, N, reinterpret_cast<const int32_t *>(map_ws),
+                           D, C1, K, base, tc_part_bytes(D, C1, K), cim_score_tc_workspace_bytes(D, C1, K), st);
 }
 
 CIM_API int cim_score_heads(const float *x, const float *weight, const float *bias, float *scores, int n_img,

@@ -26,6 +26,7 @@
 // Shapes the tensor path does not take (M < 128, D % 4 != 0, no TMA driver entry) run two plain fp32
 // kernels (correctness path for tiny problems).
 #include "common.cuh"
+#include "ragged.cuh"
 #include "score_tc.cuh"
 
 namespace {
@@ -78,11 +79,14 @@ score_det_dot_kernel(const float *__restrict__ g, const float *__restrict__ y, c
 // runs: dz rows in C1-float runs, dz^T rows as 128 B (32 proposals) per class -- one thread per (head, row) writing
 // its row with a 768-byte stride took 57 us at cfg2 for 43 MB.  Padding rows (r >= n of their image) get dz = 0
 // whatever grad_scores holds there, so their grad_x rows and their share of grad_W / grad_b are 0.
+// COMPACT (compact ragged rows, ragged.cuh): dz row m is read from y / g row row_map[m] of heads of M_in rows; a row
+// with row_map[m] < 0 gets dz = 0 and reads nothing.
+template <bool COMPACT>
 __global__ void __launch_bounds__(256)
 score_act_bwd_kernel(const float *__restrict__ y_all, const float *__restrict__ g_all,
                      const float *__restrict__ det_dot, const int32_t *__restrict__ n_props, float *__restrict__ dz_hi, float *__restrict__ dz_lo,
                      float *__restrict__ dzT_hi, float *__restrict__ dzT_lo, int M, int R, int C1, int K, int NP,
-                     long long MP) {
+                     long long MP, const int32_t *__restrict__ row_map, int M_in) {
     extern __shared__ float act_smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
     const int pitch = C1 | 1;                                  // odd: lane = row reads / writes conflict-free
@@ -91,7 +95,28 @@ score_act_bwd_kernel(const float *__restrict__ y_all, const float *__restrict__ 
     const int m0 = blockIdx.x * 32;
     for (int h = warp; h < nheads; h += nw) {
         const int m = m0 + lane;
-        if (m < M) {
+        if constexpr (COMPACT) {
+            const int pm = m < M ? row_map[m] : -1;
+            if (pm >= 0) {
+                const size_t row = (size_t)h * M_in + pm;
+                const float *y = y_all + row * C1, *g = g_all + row * C1;
+                float dot = 0.f;
+                const bool row_softmax = (h == 0) || (h >= 2 && h < 2 + K);
+                if (row_softmax)
+                    for (int c = 0; c < C1; ++c) dot = fmaf(g[c], y[c], dot);
+                const float *ddot = det_dot + (size_t)(pm / R) * C1;
+                for (int c = 0; c < C1; ++c) {
+                    const float yy = y[c], gg = g[c];
+                    float v;
+                    if (row_softmax) v = yy * (gg - dot);
+                    else if (h == 1) v = yy * (gg - ddot[c]);
+                    else v = gg * yy * (1.f - yy);
+                    tile[lane * pitch + c] = v;
+                }
+            } else if (m < M) {
+                for (int c = 0; c < C1; ++c) tile[lane * pitch + c] = 0.f;
+            }
+        } else if (m < M) {
             const size_t row = (size_t)h * M + m;
             const float *y = y_all + row * C1, *g = g_all + row * C1;
             float dot = 0.f;
@@ -498,9 +523,10 @@ struct BwdLayout {
     size_t off_dot, off_dzh, off_dzl, off_dth, off_dtl, off_wth, off_wtl, off_part, total;
 };
 inline size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
-BwdLayout bwd_layout(int n_img, int R, int D, int C1, int K) {
+// M rows of x and dz: n_img * R, or N with compact ragged rows (their row map then follows at `total`)
+BwdLayout bwd_layout(int n_img, long long M, int D, int C1, int K) {
     BwdLayout L;
-    L.M = (long long)n_img * R;
+    L.M = M;
     L.N = (2 + 2 * K) * C1;
     L.NP = (L.N + 31) & ~31;
     L.MP = (L.M + 31) & ~31LL;
@@ -528,39 +554,24 @@ BwdLayout bwd_layout(int n_img, int R, int D, int C1, int K) {
 
 CIM_API size_t cim_score_heads_bwd_workspace_bytes(int n_img, int R, int D, int C1, int K) {
     if (n_img <= 0 || R <= 0 || D <= 0 || C1 <= 0 || K < 0) return 256;
-    return bwd_layout(n_img, R, D, C1, K).total;
+    return bwd_layout(n_img, (long long)n_img * R, D, C1, K).total;
 }
 
-CIM_API int cim_score_heads_bwd_ex(const float *x, const float *weight, const float *scores, const float *grad_scores,
-                                   const int32_t *n_props, float *grad_x, float *grad_weight, float *grad_bias,
-                                   int n_img, int R, int D, int C1, int K, void *workspace, size_t ws_bytes,
-                                   cim_stream_t stream) {
-    if (!x || !weight || !scores || !grad_scores || !workspace) return CIM_ERR_ARG;
-    if (n_img < 0 || R < 0 || D <= 0 || C1 <= 0 || K < 0 || K > 8) return CIM_ERR_ARG;
-    if (!grad_x && !grad_weight && !grad_bias) return CIM_OK;
-    if (n_img > 65535 || C1 > 65535) return CIM_ERR_SHAPE;
-    cudaStream_t st = (cudaStream_t)stream;
+// everything after the argument checks: scores / grad_scores padded (heads of n_img * R rows), x / grad_x / dz of L.M
+// rows; row_map (compact ragged rows) maps dz row m to its padded row, NULL when L.M = n_img * R rows are padded rows
+static int score_heads_bwd_run(const float *x, const float *weight, const float *scores, const float *grad_scores,
+                               const int32_t *n_props, const int32_t *row_map, float *grad_x, float *grad_weight,
+                               float *grad_bias, int n_img, int R, int D, int C1, int K, const BwdLayout &L,
+                               unsigned char *ws, cudaStream_t st) {
     const int nheads = 2 + 2 * K;
-    if (n_img == 0 || R == 0) {                        // no proposals: the parameter gradients are zero
-        if (grad_weight) cudaMemsetAsync(grad_weight, 0, sizeof(float) * (size_t)nheads * C1 * D, st);
-        if (grad_bias) cudaMemsetAsync(grad_bias, 0, sizeof(float) * (size_t)nheads * C1, st);
-        return cim_launch_status();
-    }
-    const BwdLayout L = bwd_layout(n_img, R, D, C1, K);
-    if (L.M > (1LL << 30)) return CIM_ERR_SHAPE;
-    if (ws_bytes < L.total) return CIM_ERR_WORKSPACE;
-    if (!cim_aligned(x, 16) || !cim_aligned(weight, 16) || (grad_x && !cim_aligned(grad_x, 16)) ||
-        !cim_aligned(n_props, 4))
-        return CIM_ERR_ALIGN;
-    unsigned char *ws = reinterpret_cast<unsigned char *>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
     auto F = [&](size_t off) { return reinterpret_cast<float *>(ws + off - 256); };
     float *dot = F(L.off_dot), *dzh = F(L.off_dzh), *dzl = F(L.off_dzl), *dth = F(L.off_dth), *dtl = F(L.off_dtl);
     float *wth = F(L.off_wth), *wtl = F(L.off_wtl), *part = F(L.off_part);
-    const int M = (int)L.M, N = L.N;
+    const int M = (int)L.M, N = L.N, M_in = n_img * R;
     const bool want_t = grad_weight || grad_bias;
 
-    score_det_dot_kernel<<<dim3((unsigned)C1, (unsigned)n_img), 256, 0, st>>>(grad_scores + (size_t)M * C1,
-                                                                             scores + (size_t)M * C1, n_props, dot, R, C1);
+    score_det_dot_kernel<<<dim3((unsigned)C1, (unsigned)n_img), 256, 0, st>>>(grad_scores + (size_t)M_in * C1,
+                                                                             scores + (size_t)M_in * C1, n_props, dot, R, C1);
     int rc = cim_launch_status();
     if (rc) return rc;
     const long long rows = (long long)nheads * M;
@@ -568,11 +579,19 @@ CIM_API int cim_score_heads_bwd_ex(const float *x, const float *weight, const fl
     while (act_warps > 1 && (size_t)act_warps * 32 * (C1 | 1) * sizeof(float) > 96 * 1024) act_warps >>= 1;
     const size_t act_smem = (size_t)act_warps * 32 * (C1 | 1) * sizeof(float);
     if (act_smem > (size_t)cim_max_smem_optin()) return CIM_ERR_SHAPE;         // C1 > ~1700
-    if (act_smem > 48 * 1024)
-        cudaFuncSetAttribute(score_act_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)act_smem);
-    score_act_bwd_kernel<<<(unsigned)((M + 31) / 32), act_warps * 32, act_smem, st>>>(scores, grad_scores, dot, n_props, grad_x ? dzh : nullptr,
-                                                                        dzl, want_t ? dth : nullptr, dtl, M, R, C1, K,
-                                                                        L.NP, L.MP);
+    if (row_map) {
+        if (act_smem > 48 * 1024)
+            cudaFuncSetAttribute(score_act_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)act_smem);
+        score_act_bwd_kernel<true><<<(unsigned)((M + 31) / 32), act_warps * 32, act_smem, st>>>(
+            scores, grad_scores, dot, n_props, grad_x ? dzh : nullptr, dzl, want_t ? dth : nullptr, dtl, M, R, C1, K,
+            L.NP, L.MP, row_map, M_in);
+    } else {
+        if (act_smem > 48 * 1024)
+            cudaFuncSetAttribute(score_act_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)act_smem);
+        score_act_bwd_kernel<false><<<(unsigned)((M + 31) / 32), act_warps * 32, act_smem, st>>>(
+            scores, grad_scores, dot, n_props, grad_x ? dzh : nullptr, dzl, want_t ? dth : nullptr, dtl, M, R, C1, K,
+            L.NP, L.MP, nullptr, 0);
+    }
     if ((rc = cim_launch_status())) return rc;
     if (grad_bias) {
         score_bias_grad_kernel<<<(unsigned)N, 256, 0, st>>>(dth, dtl, grad_bias, M, L.MP);
@@ -621,6 +640,70 @@ CIM_API int cim_score_heads_bwd_ex(const float *x, const float *weight, const fl
         if ((rc = cim_launch_status())) return rc;
     }
     return CIM_OK;
+}
+
+// the checks both entry points make; rows = n_img * R (padded) or N (compact)
+static int score_heads_bwd_args(const float *x, const float *weight, const float *scores, const float *grad_scores,
+                                const int32_t *n_props, const float *grad_x, int n_img, int R, int D, int C1, int K,
+                                const void *workspace) {
+    if (!x || !weight || !scores || !grad_scores || !workspace) return CIM_ERR_ARG;
+    if (n_img < 0 || R < 0 || D <= 0 || C1 <= 0 || K < 0 || K > 8) return CIM_ERR_ARG;
+    if (n_img > 65535 || C1 > 65535) return CIM_ERR_SHAPE;
+    if ((long long)n_img * R > (1LL << 30)) return CIM_ERR_SHAPE;
+    if (!cim_aligned(x, 16) || !cim_aligned(weight, 16) || (grad_x && !cim_aligned(grad_x, 16)) ||
+        !cim_aligned(n_props, 4))
+        return CIM_ERR_ALIGN;
+    return CIM_OK;
+}
+
+CIM_API int cim_score_heads_bwd_ex(const float *x, const float *weight, const float *scores, const float *grad_scores,
+                                   const int32_t *n_props, float *grad_x, float *grad_weight, float *grad_bias,
+                                   int n_img, int R, int D, int C1, int K, void *workspace, size_t ws_bytes,
+                                   cim_stream_t stream) {
+    if (!x || !weight || !scores || !grad_scores || !workspace) return CIM_ERR_ARG;
+    if (n_img < 0 || R < 0 || D <= 0 || C1 <= 0 || K < 0 || K > 8) return CIM_ERR_ARG;
+    if (!grad_x && !grad_weight && !grad_bias) return CIM_OK;
+    if (n_img > 65535 || C1 > 65535) return CIM_ERR_SHAPE;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int nheads = 2 + 2 * K;
+    if (n_img == 0 || R == 0) {                        // no proposals: the parameter gradients are zero
+        if (grad_weight) cudaMemsetAsync(grad_weight, 0, sizeof(float) * (size_t)nheads * C1 * D, st);
+        if (grad_bias) cudaMemsetAsync(grad_bias, 0, sizeof(float) * (size_t)nheads * C1, st);
+        return cim_launch_status();
+    }
+    const BwdLayout L = bwd_layout(n_img, (long long)n_img * R, D, C1, K);
+    if (L.M > (1LL << 30)) return CIM_ERR_SHAPE;
+    if (ws_bytes < L.total) return CIM_ERR_WORKSPACE;
+    int rc = score_heads_bwd_args(x, weight, scores, grad_scores, n_props, grad_x, n_img, R, D, C1, K, workspace);
+    if (rc) return rc;
+    unsigned char *ws = reinterpret_cast<unsigned char *>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+    return score_heads_bwd_run(x, weight, scores, grad_scores, n_props, nullptr, grad_x, grad_weight, grad_bias, n_img,
+                               R, D, C1, K, L, ws, st);
+}
+
+CIM_API size_t cim_score_heads_bwd_compact_workspace_bytes(int n_img, int R, int N, int D, int C1, int K) {
+    (void)R;
+    if (n_img <= 0 || N <= 0 || D <= 0 || C1 <= 0 || K < 0) return 256;
+    return bwd_layout(n_img, N, D, C1, K).total + compact_map_bytes(n_img, N);
+}
+
+CIM_API int cim_score_heads_bwd_compact(const float *x, const float *weight, const float *scores,
+                                        const float *grad_scores, const int32_t *n_props, float *grad_x,
+                                        float *grad_weight, float *grad_bias, int n_img, int R, int N, int D, int C1,
+                                        int K, void *workspace, size_t ws_bytes, cim_stream_t stream) {
+    int rc = score_heads_bwd_args(x, weight, scores, grad_scores, n_props, grad_x, n_img, R, D, C1, K, workspace);
+    if (rc) return rc;
+    if (n_img <= 0 || R <= 0 || N <= 0) return CIM_ERR_ARG;
+    if (N > n_img * R) return CIM_ERR_SHAPE;
+    if (!grad_x && !grad_weight && !grad_bias) return CIM_OK;
+    if (ws_bytes < cim_score_heads_bwd_compact_workspace_bytes(n_img, R, N, D, C1, K)) return CIM_ERR_WORKSPACE;
+    cudaStream_t st = (cudaStream_t)stream;
+    const BwdLayout L = bwd_layout(n_img, N, D, C1, K);
+    unsigned char *ws = reinterpret_cast<unsigned char *>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+    unsigned char *map_ws = ws + L.total - 256;                  // offsets in the layout count the 256 B of slack
+    if ((rc = compact_row_map_launch(n_props, n_img, R, N, map_ws, st))) return rc;
+    return score_heads_bwd_run(x, weight, scores, grad_scores, n_props, reinterpret_cast<const int32_t *>(map_ws),
+                               grad_x, grad_weight, grad_bias, n_img, R, D, C1, K, L, ws, st);
 }
 
 CIM_API int cim_score_heads_bwd(const float *x, const float *weight, const float *scores, const float *grad_scores,

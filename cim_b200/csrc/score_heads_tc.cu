@@ -55,10 +55,14 @@ __global__ void score_split_w_kernel(const float *__restrict__ w, float *__restr
     }
 }
 
+// REMAP (compact ragged rows, ragged.cuh): x row m is written to scores row row_map[m] of heads of M_out rows, and
+// not at all for row_map[m] < 0; without it, to row m of heads of M rows (row_map / M_out unused).
+template <bool REMAP>
 __global__ void __launch_bounds__(THREADS_TC, 1)
 score_gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_whi,
                      const __grid_constant__ CUtensorMap tm_wlo, const float *__restrict__ bias,
-                     float *__restrict__ scores, int M, int D, int C1, int n_ref, int heads_per_tile) {
+                     float *__restrict__ scores, int M, int D, int C1, int n_ref, int heads_per_tile,
+                     const int32_t *__restrict__ row_map, int M_out) {
     extern __shared__ unsigned char smem_raw[];
     unsigned char *smem = reinterpret_cast<unsigned char *>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
     unsigned char *raw = smem + (size_t)NSTAGE * STAGE;                 // [NRAW][A_TILE]
@@ -220,12 +224,19 @@ score_gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_cons
 #pragma unroll
         for (int j = 0; j < NT; ++j) zrow[j] = acc[j];
         const int m = m0 + 32 * q4 + lane;
-        if (m < M) {
+        int out_row = m, out_rows = M;
+        bool live = m < M;
+        if constexpr (REMAP) {
+            out_row = live ? row_map[m] : -1;
+            out_rows = M_out;
+            live = out_row >= 0;
+        }
+        if (live) {
             for (int hh = 0; hh < nh; ++hh) {
                 const int h = h0 + hh;
                 float *z = zrow + hh * C1;
                 const float *bh = s_bias + hh * C1;
-                float *dst = scores + ((size_t)h * M + m) * C1;
+                float *dst = scores + ((size_t)h * out_rows + out_row) * C1;
                 const bool softmax = (h == 0) || (h >= 2 && h < 2 + n_ref);
                 if (softmax) {
                     float mx = -INFINITY;
@@ -267,9 +278,11 @@ size_t cim_score_tc_workspace_bytes(int D, int C1, int n_ref) {
     return 2 * sizeof(float) * (size_t)(2 + 2 * n_ref) * C1 * D + 512;
 }
 
-// logits + row activations for every head into `scores`; the detector head (1) is left as logits
+// logits + row activations for every head into `scores`; the detector head (1) is left as logits.  row_map != NULL:
+// x holds M compact rows, scores heads of M_out padded rows (ragged.cuh)
 int cim_score_tc_launch(const float *x, const float *weight, const float *bias, float *scores, long long M, int D,
-                        int C1, int n_ref, void *workspace, cudaStream_t st) {
+                        int C1, int n_ref, void *workspace, cudaStream_t st, const int32_t *row_map,
+                        long long M_out) {
     const int nheads = 2 + 2 * n_ref, N = nheads * C1;
     float *w_hi = reinterpret_cast<float *>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
     float *w_lo = w_hi + (size_t)N * D;
@@ -284,8 +297,14 @@ int cim_score_tc_launch(const float *x, const float *weight, const float *bias, 
     const size_t smem = score_tc_smem_bytes(heads_per_tile * C1);
     if ((M + BM - 1) / BM > 65535) return CIM_ERR_SHAPE;
     dim3 grid((unsigned)ntiles, (unsigned)((M + BM - 1) / BM));
-    cudaFuncSetAttribute(score_gemm_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    score_gemm_tc_kernel<<<grid, THREADS_TC, smem, st>>>(tx, twh, twl, bias, scores, (int)M, D, C1, n_ref,
-                                                         heads_per_tile);
+    if (row_map) {
+        cudaFuncSetAttribute(score_gemm_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        score_gemm_tc_kernel<true><<<grid, THREADS_TC, smem, st>>>(tx, twh, twl, bias, scores, (int)M, D, C1, n_ref,
+                                                                   heads_per_tile, row_map, (int)M_out);
+    } else {
+        cudaFuncSetAttribute(score_gemm_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        score_gemm_tc_kernel<false><<<grid, THREADS_TC, smem, st>>>(tx, twh, twl, bias, scores, (int)M, D, C1, n_ref,
+                                                                    heads_per_tile, nullptr, 0);
+    }
     return cim_launch_status();
 }

@@ -34,19 +34,38 @@ from . import _lib
 class ScoreHeadsFunction(Function):
     """scores[h] = act_h(x @ W_h^T + b_h) for the 2+2K heads; see cim_score_heads in cimhead.h.
     n_props (optional): proposals per image of a ragged batch (_lib.n_props_arg); image b owns rows [0, n_b) of its R
-    rows, the detector softmax runs over those and every head is 0 on the others (cim_score_heads_ex)."""
+    rows, the detector softmax runs over those and every head is 0 on the others (cim_score_heads_ex).
+    capacity (compact ragged batch, cim_score_heads_compact): x holds only the N = sum(n_props) real rows, image b's at
+    [off_b, off_b + n_b); n_props must then be host counts (_lib.compact_rows_arg).  The scores come back padded to
+    [2+2K, n_img * capacity, C1] as with n_props alone, and the backward returns grad_x [N, D]."""
 
     @staticmethod
-    def forward(ctx, x, weight, bias, n_img, k, n_props=None):
+    def forward(ctx, x, weight, bias, n_img, k, n_props=None, capacity=None):
         _lib.require_cuda(x, "seg_feature", torch.float32)
         _lib.require_cuda(weight, "weight", torch.float32)
         _lib.require_cuda(bias, "bias", torch.float32)
         x, weight, bias = x.contiguous(), weight.contiguous(), bias.contiguous()
         m, d = x.shape
         nh, c1, _ = weight.shape
+        L = _lib.lib()
+        if capacity is not None:
+            R = int(capacity)
+            with torch.cuda.device(x.device):
+                n_props, n = _lib.compact_rows_arg(n_props, n_img, R, x.device)
+                if m != n:
+                    raise ValueError(f"a compact seg_feature must have sum(n_props) = {n} rows, got {m}")
+                scores = torch.empty((nh, n_img * R, c1), dtype=torch.float32, device=x.device)
+                ws = torch.empty(L.cim_score_heads_compact_workspace_bytes(n_img, R, n, d, c1, k), dtype=torch.uint8,
+                                 device=x.device)
+                rc = L.cim_score_heads_compact(_lib.ptr(x), _lib.ptr(weight), _lib.ptr(bias), _lib.ptr(scores),
+                                               _lib.ptr(n_props), n_img, R, n, d, c1, k, _lib.ptr(ws), ws.numel(),
+                                               _lib.stream_ptr(x.device))
+            _lib.check(rc, "cim_score_heads_compact")
+            ctx.save_for_backward(x, weight, scores)
+            ctx.cfg = (n_img, k, n_props, R)
+            return scores
         if m % n_img:
             raise ValueError("rows of seg_feature must be n_img * R")
-        L = _lib.lib()
         with torch.cuda.device(x.device):
             n_props = _lib.n_props_arg(n_props, n_img, m // n_img, x.device)
             scores = torch.empty((nh, m, c1), dtype=torch.float32, device=x.device)
@@ -57,7 +76,7 @@ class ScoreHeadsFunction(Function):
                                       _lib.stream_ptr(x.device))
         _lib.check(rc, "cim_score_heads")
         ctx.save_for_backward(x, weight, scores)
-        ctx.cfg = (n_img, k, n_props)
+        ctx.cfg = (n_img, k, n_props, None)
         return scores
 
     @staticmethod
@@ -66,9 +85,9 @@ class ScoreHeadsFunction(Function):
         """cim_score_heads_bwd: activation backward + grad_x / grad_weight / grad_bias in one call
         (autograd of heads.py:194-219)."""
         x, weight, s = ctx.saved_tensors
-        n_img, k, n_props = ctx.cfg
+        n_img, k, n_props, capacity = ctx.cfg
         nh, m, c1 = s.shape
-        d = x.shape[1]
+        n, d = x.shape
         grad = _lib.require_cuda(grad, "grad_scores", torch.float32).contiguous()
         L = _lib.lib()
         need_x, need_w, need_b = ctx.needs_input_grad[:3]
@@ -76,13 +95,21 @@ class ScoreHeadsFunction(Function):
             gx = torch.empty_like(x) if need_x else None
             gw = torch.empty_like(weight) if need_w else None
             gb = torch.empty((nh, c1), dtype=torch.float32, device=x.device) if need_b else None
-            ws = torch.empty(L.cim_score_heads_bwd_workspace_bytes(n_img, m // n_img, d, c1, k), dtype=torch.uint8,
-                             device=x.device)
-            rc = L.cim_score_heads_bwd_ex(_lib.ptr(x), _lib.ptr(weight), _lib.ptr(s), _lib.ptr(grad),
-                                          _lib.ptr(n_props), _lib.ptr(gx), _lib.ptr(gw), _lib.ptr(gb), n_img, m // n_img,
-                                          d, c1, k, _lib.ptr(ws), ws.numel(), _lib.stream_ptr(x.device))
+            if capacity is not None:
+                ws = torch.empty(L.cim_score_heads_bwd_compact_workspace_bytes(n_img, capacity, n, d, c1, k),
+                                 dtype=torch.uint8, device=x.device)
+                rc = L.cim_score_heads_bwd_compact(_lib.ptr(x), _lib.ptr(weight), _lib.ptr(s), _lib.ptr(grad),
+                                                   _lib.ptr(n_props), _lib.ptr(gx), _lib.ptr(gw), _lib.ptr(gb), n_img,
+                                                   capacity, n, d, c1, k, _lib.ptr(ws), ws.numel(),
+                                                   _lib.stream_ptr(x.device))
+            else:
+                ws = torch.empty(L.cim_score_heads_bwd_workspace_bytes(n_img, m // n_img, d, c1, k), dtype=torch.uint8,
+                                 device=x.device)
+                rc = L.cim_score_heads_bwd_ex(_lib.ptr(x), _lib.ptr(weight), _lib.ptr(s), _lib.ptr(grad),
+                                              _lib.ptr(n_props), _lib.ptr(gx), _lib.ptr(gw), _lib.ptr(gb), n_img,
+                                              m // n_img, d, c1, k, _lib.ptr(ws), ws.numel(), _lib.stream_ptr(x.device))
         _lib.check(rc, "cim_score_heads_bwd")
-        return gx, gw, gb, None, None, None
+        return gx, gw, gb, None, None, None, None
 
 
 class cls_iou_model(nn.Module):
@@ -102,13 +129,15 @@ class cls_iou_model(nn.Module):
         layers = [self.classifier, self.detector, *self.refine_cls, *self.refine_iou]
         return torch.stack([l.weight for l in layers]), torch.stack([l.bias for l in layers])
 
-    def forward_batched(self, seg_feature, n_img=1, n_props=None):
+    def forward_batched(self, seg_feature, n_img=1, n_props=None, capacity=None):
         """seg_feature [n_img*R, D] -> scores [2+2K, n_img*R, C1] (detector softmax per image).  n_props: proposals
-        per image of a ragged batch (R is then a capacity; see ScoreHeadsFunction)."""
+        per image of a ragged batch (R is then a capacity; see ScoreHeadsFunction).  capacity=R: a compact ragged batch,
+        seg_feature [sum(n_props), D] holds the real proposals only (image b's at rows [off_b, off_b + n_b)), n_props
+        are host counts, and the scores come back padded [2+2K, n_img*R, C1]."""
         if seg_feature.dim() == 4:
             seg_feature = seg_feature.squeeze(3).squeeze(2)
         weight, bias = self._stacked()
-        return ScoreHeadsFunction.apply(seg_feature, weight, bias, n_img, len(self.refine_cls), n_props)
+        return ScoreHeadsFunction.apply(seg_feature, weight, bias, n_img, len(self.refine_cls), n_props, capacity)
 
     def forward(self, seg_feature):
         k = len(self.refine_cls)

@@ -91,7 +91,10 @@ class CIMHeadStep:
             self.area = e((n_img, R), torch.int32)
             self.overlap_ws = e((self.L.cim_mask_overlap_workspace_bytes(n_img, R, mask_words, 0),), torch.uint8)
             self.scores = e((nh, n_img * R, C1), torch.float32)
-            self.score_ws = e((max(256, self.L.cim_score_heads_workspace_bytes(n_img, R, feat_dim, C1, k)),), torch.uint8)
+            # large enough for the padded and the compact form (the latter at N = n_img * R covers every N)
+            self.score_ws = e((max(256, self.L.cim_score_heads_workspace_bytes(n_img, R, feat_dim, C1, k),
+                                   self.L.cim_score_heads_compact_workspace_bytes(n_img, R, n_img * R, feat_dim, C1,
+                                                                                  k)),), torch.uint8)
             self.head_grads = bool(head_grads)
             if self.head_grads:
                 # grad_weight and grad_bias share one buffer: the bucket of the data-parallel allreduce
@@ -99,7 +102,9 @@ class CIMHeadStep:
                 self.grad_weight = self.head_bucket[:nh * C1 * feat_dim].view(nh, C1, feat_dim)
                 self.grad_bias = self.head_bucket[nh * C1 * feat_dim:].view(nh, C1)
                 self.grad_seg_x = e((n_img * R, feat_dim), torch.float32)
-                self.score_bwd_ws = e((self.L.cim_score_heads_bwd_workspace_bytes(n_img, R, feat_dim, C1, k),),
+                self.score_bwd_ws = e((max(self.L.cim_score_heads_bwd_workspace_bytes(n_img, R, feat_dim, C1, k),
+                                           self.L.cim_score_heads_bwd_compact_workspace_bytes(n_img, R, n_img * R,
+                                                                                              feat_dim, C1, k)),),
                                       torch.uint8)
                 self.losses = e((n_img, k + 1, 3), torch.float32)
                 self.pcl_loss = torch.zeros((n_img,), dtype=torch.float32, device=dev)
@@ -168,7 +173,7 @@ class CIMHeadStep:
 
     # -------------------------------------------------------------------------------------
     def run(self, feat, rois, grad_out, packed_masks, seg_x, weight, bias, labels, labels_host=None, grad_scores=None,
-            mat=None, mid_hook=None, order=None, mask_meta=None, n_props=None, feat_hw=None):
+            mat=None, mid_hook=None, order=None, mask_meta=None, n_props=None, feat_hw=None, compact=False):
         """feat [n_img,Cf,H,W] f32, rois [n_img*R,5] f32 grouped by image, grad_out [n_img*R,Cf,7,7]
         f32, packed_masks [n_img,R,words] i32, seg_x [n_img*R,D] f32, weight [2+2K,C+1,D],
         bias [2+2K,C+1], labels [n_img,C] f32 (labels_host is no longer needed: the sampling runs on the device).
@@ -191,6 +196,12 @@ class CIMHeadStep:
         then a canvas of the constructor's (feat_h, feat_w): image b occupies feat[b, :, :H_b, :W_b], and its roi_out
         rows and grad_feat equal RoIAlign of that map alone (grad_feat is 0 outside it; the canvas there must be
         finite).  Nothing else of the step depends on it.  None: every image fills the canvas.
+        compact: a compact ragged batch.  n_props must then be host counts (a sequence, numpy array or CPU tensor); with
+        N = sum(n_props), image b's proposals are rows [off_b, off_b + n_b) (off_b = n_0 + ... + n_{b-1}) of rois,
+        grad_out and seg_x, which have exactly N rows, and the results of those rows land in roi_out[:N] and
+        grad_seg_x[:N].  RoIAlign, the scoring GEMMs and the caller's per-proposal head then process N rows instead of
+        n_img * R; everything from the scores on (maps, mining, losses, PCL) keeps the padded capacity layout, with the
+        same values as a padded call.  The buffers stay allocated at capacity, so N may change from step to step.
 
         order (default: the constructor's):
           "graph"      the model's dependency order (model_builder.py:136-204): RoIAlign forward -> scoring heads ->
@@ -215,7 +226,16 @@ class CIMHeadStep:
         ck = _lib.check
         cur = torch.cuda.current_stream(dev)
         pcl_early = self.head_grads and grad_scores is None and mat is not None
-        self.n_props = np_dev = _lib.n_props_arg(n_props, n_img, R, dev)
+        if compact:
+            np_dev, n_rows = _lib.compact_rows_arg(n_props, n_img, R, dev)
+            self.n_props = np_dev
+            for name, t in (("rois", rois), ("grad_out", grad_out), ("seg_x", seg_x)):
+                if t.shape[0] != n_rows:
+                    raise ValueError(f"{name} of a compact batch must have sum(n_props) = {n_rows} rows, "
+                                     f"got {t.shape[0]}")
+        else:
+            self.n_props = np_dev = _lib.n_props_arg(n_props, n_img, R, dev)
+            n_rows = n_img * R
         self.feat_hw = hw = _lib.feat_hw_arg(feat_hw, n_img, self.H, self.W, dev)
 
         def pcl(stream):
@@ -227,9 +247,14 @@ class CIMHeadStep:
 
         def score_fwd(stream, with_pcl):
             with _nvtx("cim/score_heads"):
-                ck(L.cim_score_heads_ex(P(seg_x), P(weight), P(bias), P(self.scores), P(np_dev), n_img, R, self.D,
-                                        self.C + 1, k, P(self.score_ws), self.score_ws.numel(), stream),
-                   "cim_score_heads")
+                if compact:
+                    ck(L.cim_score_heads_compact(P(seg_x), P(weight), P(bias), P(self.scores), P(np_dev), n_img, R,
+                                                 n_rows, self.D, self.C + 1, k, P(self.score_ws),
+                                                 self.score_ws.numel(), stream), "cim_score_heads_compact")
+                else:
+                    ck(L.cim_score_heads_ex(P(seg_x), P(weight), P(bias), P(self.scores), P(np_dev), n_img, R, self.D,
+                                            self.C + 1, k, P(self.score_ws), self.score_ws.numel(), stream),
+                       "cim_score_heads")
             if with_pcl and pcl_early:
                 pcl(stream)
 
@@ -242,7 +267,7 @@ class CIMHeadStep:
         def roi_fwd():
             with _nvtx("cim/roi_align_fwd"):
                 ck(L.cim_roi_align_fwd_prepared_ex(P(feat), P(rois), P(hw), None, P(self.roi_out), n_img, self.Cf,
-                                                   self.H, self.W, n_img * R, 7, 7, self.scale, self.sr, self.aligned,
+                                                   self.H, self.W, n_rows, 7, 7, self.scale, self.sr, self.aligned,
                                                    P(self.roi_ws), self.roi_ws.numel(), st), "cim_roi_align_fwd")
 
         def mine():
@@ -269,7 +294,7 @@ class CIMHeadStep:
             # the persistent RoIAlign forward is on the SMs before the overlap's tensor kernel asks for them -- which of
             # the two went first used to depend on launch timing (cfg3: 5.67 or 5.85 ms)
             with _nvtx("cim/roi_prepare"):
-                ck(L.cim_roi_align_prepare_ex(P(rois), P(hw), n_img, self.Cf, self.H, self.W, n_img * R, 7, 7,
+                ck(L.cim_roi_align_prepare_ex(P(rois), P(hw), n_img, self.Cf, self.H, self.W, n_rows, 7, 7,
                                               self.scale, self.sr, self.aligned, P(self.roi_ws), self.roi_ws.numel(),
                                               st), "cim_roi_align_prepare")
             self.ev_prep.record(cur)
@@ -288,7 +313,7 @@ class CIMHeadStep:
             # the scoring GEMM (independent of the maps) runs on a side stream next to the overlap stage, whose small
             # serial helpers leave most of the GPU idle; RoI descriptors once per step, also off the critical path
             score_fwd(side_st, True)
-            ck(L.cim_roi_align_prepare_ex(P(rois), P(hw), n_img, self.Cf, self.H, self.W, n_img * R, 7, 7, self.scale,
+            ck(L.cim_roi_align_prepare_ex(P(rois), P(hw), n_img, self.Cf, self.H, self.W, n_rows, 7, 7, self.scale,
                                           self.sr, self.aligned, P(self.roi_ws), self.roi_ws.numel(), side_st),
                "cim_roi_align_prepare")
             overlap(st)
@@ -351,14 +376,20 @@ class CIMHeadStep:
                         self.grad_scores[0].add_(self.pcl_grad)
                 grad_scores = self.grad_scores
             with _nvtx("cim/score_heads_bwd"):
-                ck(L.cim_score_heads_bwd_ex(P(seg_x), P(weight), P(self.scores), P(grad_scores), P(np_dev),
-                                            P(self.grad_seg_x), P(self.grad_weight), P(self.grad_bias), n_img, R,
-                                            self.D, self.C + 1, k, P(self.score_bwd_ws), self.score_bwd_ws.numel(),
-                                            st), "cim_score_heads_bwd")
+                if compact:
+                    ck(L.cim_score_heads_bwd_compact(P(seg_x), P(weight), P(self.scores), P(grad_scores), P(np_dev),
+                                                     P(self.grad_seg_x), P(self.grad_weight), P(self.grad_bias), n_img,
+                                                     R, n_rows, self.D, self.C + 1, k, P(self.score_bwd_ws),
+                                                     self.score_bwd_ws.numel(), st), "cim_score_heads_bwd_compact")
+                else:
+                    ck(L.cim_score_heads_bwd_ex(P(seg_x), P(weight), P(self.scores), P(grad_scores), P(np_dev),
+                                                P(self.grad_seg_x), P(self.grad_weight), P(self.grad_bias), n_img, R,
+                                                self.D, self.C + 1, k, P(self.score_bwd_ws), self.score_bwd_ws.numel(),
+                                                st), "cim_score_heads_bwd")
                 reduce_work = cdist.allreduce_mean_async_(self.head_bucket)     # overlaps the RoIAlign backward
         with _nvtx("cim/roi_align_bwd"):
             ck(L.cim_roi_align_bwd_prepared_ex(P(grad_out), P(rois), P(hw), None, P(self.grad_feat), n_img, self.Cf,
-                                               self.H, self.W, n_img * R, 7, 7, self.scale, self.sr, self.aligned,
+                                               self.H, self.W, n_rows, 7, 7, self.scale, self.sr, self.aligned,
                                                P(self.roi_ws), self.roi_ws.numel(), st), "cim_roi_align_bwd")
         if reduce_work is not None:
             reduce_work()                                       # current stream waits for the allreduce
@@ -413,7 +444,7 @@ class CIMHeadStep:
         self.ustream.commit()
 
     # -------------------------------------------------------------------------------------
-    def alloc_host_io(self, mask_hw=None, crop_capacity_words=0, prefetch_depth=1, ragged=False):
+    def alloc_host_io(self, mask_hw=None, crop_capacity_words=0, prefetch_depth=1, ragged=False, compact=False):
         """Pinned host buffers of the end-to-end call: inputs that originate on the host in the
         reference's pipeline (rois, labels: lib/roi_data/minibatch.py:45-61; proposal masks:
         the COB .mat files of tools/pre) and the step's results.  Device-side input buffers are
@@ -428,7 +459,10 @@ class CIMHeadStep:
         ragged: a pinned hi_n_props int32 [n_img] (initialised to R) joins the inputs: the proposal counts of the step,
         filled by the caller like hi_rois, validated when staged and carried with that step's rois, labels and masks
         through the double buffer and the pre-stage (run(n_props=...) for what a padding row must hold; with crops,
-        mask_ops.batch_crops_host builds the wire format with empty crops for the padding rows)."""
+        mask_ops.batch_crops_host builds the wire format with empty crops for the padding rows).
+        compact (with ragged): the batch is compact (run(compact=True)).  hi_rois holds the N = sum(hi_n_props) real rois
+        in its first N rows and only those are copied; each staged step keeps its own host counts and N, and run_host()
+        runs it with them (next_step_rows() tells how many rows its seg_x / grad_out need).  The masks stay padded."""
         k, n_img, R, C1 = self.K, self.n_img, self.R, self.C + 1
         if prefetch_depth not in (1, 2) or (prefetch_depth == 2 and not crop_capacity_words):
             raise ValueError("prefetch_depth must be 1, or 2 with crop_capacity_words > 0")
@@ -437,6 +471,9 @@ class CIMHeadStep:
         self.hi_rois = pin((n_img * R, 5), torch.float32)
         self.hi_labels = pin((n_img, self.C), torch.float32)
         self.ragged = bool(ragged)
+        if compact and not self.ragged:
+            raise ValueError("compact host I/O needs ragged=True")
+        self.compact = bool(compact)
         self.hi_n_props = pin((n_img,), torch.int32).fill_(R) if self.ragged else None
         # masks arrive either as full bit masks (hi_masks) or, with crop_capacity_words > 0, as
         # bounding-box crops (mask_ops.MaskCrops: ~8x fewer bytes over PCIe) that the device unpacks
@@ -583,7 +620,12 @@ class CIMHeadStep:
 
         def h2d(dst, stream):
             """pinned input buffers -> dst (a device input buffer or the pre-stage); returns the crop word count"""
-            dst["rois"].copy_(self.hi_rois, non_blocking=True)
+            if self.compact:
+                dst["counts"] = self.hi_n_props.numpy().copy()        # this step's host counts travel with it
+                dst["N"] = int(dst["counts"].sum())
+                dst["rois"][:dst["N"]].copy_(self.hi_rois[:dst["N"]], non_blocking=True)
+            else:
+                dst["rois"].copy_(self.hi_rois, non_blocking=True)
             dst["labels"].copy_(self.hi_labels, non_blocking=True)
             if self.ragged:
                 dst["n_props"].copy_(self.hi_n_props, non_blocking=True)
@@ -613,6 +655,8 @@ class CIMHeadStep:
                 n = pre["n_words"]
                 for key in ("rois", "labels", "crop_meta", "crop_off") + (("n_props",) if self.ragged else ()):
                     buf[key].copy_(pre[key], non_blocking=True)
+                if self.compact:
+                    buf["counts"], buf["N"] = pre["counts"], pre["N"]
                 buf["crop_words"][:n].copy_(pre["crop_words"][:n], non_blocking=True)
             else:
                 h2d(buf, self.copy_stream)
@@ -647,13 +691,22 @@ class CIMHeadStep:
         self._collect_results()
         return self.results_host
 
+    def next_step_rows(self):
+        """alloc_host_io(compact=True): N, the rows of seg_x / grad_out that the next run_host() call needs -- the
+        proposal count of the step it runs (staged earlier, or the pinned buffers' if nothing is staged)."""
+        if self._staged:
+            return self.di[self._slot]["N"]
+        return int(self.hi_n_props.numpy().sum())
+
     def run_host(self, feat, grad_out, seg_x, weight, bias, prefetch_next=True, grad_scores=None, mat=None,
                  lag_results=False, feat_hw=None):
         """End-to-end step: host rois / labels / bit-packed masks -> device, the step, results ->
         host.  With alloc_host_io(ragged=True) the proposal counts (hi_n_props) travel with the step's inputs and the
         batch is ragged (run(n_props=...)).  feat / seg_x / grad_out are produced on the device by the backbone, MaskFuse
         and autograd in the real pipeline and therefore stay device tensors; so does feat_hw, the image sizes of a
-        canvas-padded feat (run(feat_hw=...)), which goes straight through to run().
+        canvas-padded feat (run(feat_hw=...)), which goes straight through to run().  With alloc_host_io(compact=True)
+        the step runs compact with the counts staged with its inputs: seg_x and grad_out must have that step's N rows
+        (next_step_rows()), else ValueError before the step is enqueued.
         With prefetch_next the copy of the NEXT step's inputs (whatever is in the pinned input
         buffers now) is enqueued on the copy stream first, so it overlaps this step's kernels;
         every call therefore moves one full set of inputs host->device."""
@@ -662,13 +715,18 @@ class CIMHeadStep:
             self.stage_host_inputs(direct=True)
             self._staged = True
         buf = self.di[self._slot]
+        if self.compact:
+            for name, t in (("seg_x", seg_x), ("grad_out", grad_out)):
+                if t.shape[0] != buf["N"]:
+                    raise ValueError(f"{name} must have the {buf['N']} rows of the step being run, got {t.shape[0]}")
         finish_stage = None
         if prefetch_next:
             finish_stage = self.stage_host_inputs(defer_kernels=True)      # copies now, the other buffer
         cur_stream.wait_event(buf["ready"])
-        self.run(feat, buf["rois"], grad_out, buf["masks"], seg_x, weight, bias, buf["labels"],
-                 None, grad_scores=grad_scores, mat=mat, mask_meta=buf.get("meta"), n_props=buf.get("n_props"),
-                 feat_hw=feat_hw,
+        compact = self.compact
+        self.run(feat, buf["rois"][:buf["N"]] if compact else buf["rois"], grad_out, buf["masks"], seg_x, weight, bias,
+                 buf["labels"], None, grad_scores=grad_scores, mat=mat, mask_meta=buf.get("meta"),
+                 n_props=buf["counts"] if compact else buf.get("n_props"), feat_hw=feat_hw, compact=compact,
                  mid_hook=lambda: ((finish_stage(self.ev_premine) if finish_stage else None),
                                    (self._collect_results() if lag_results else None)))
         buf["free"].record(cur_stream)
@@ -677,7 +735,7 @@ class CIMHeadStep:
         # the step's stream; everything else of the read-back -- the other checksum and the device -> host copies --
         # runs on a results stream behind `ev_done`, so the next step's first kernels do not queue behind the copies.
         # The next step waits for `res_ev` right before the first kernel that overwrites a result (cim_assign).
-        ro, gf = self.roi_out.view(-1), self.grad_feat.view(-1)
+        ro, gf = (self.roi_out[:buf["N"]] if compact else self.roi_out).reshape(-1), self.grad_feat.view(-1)
         torch.sum(ro[::max(1, ro.numel() // 509)], dim=0, out=self.d_checksum[0])
         self.ev_done.record(cur_stream)
         with torch.cuda.stream(self.res_stream):

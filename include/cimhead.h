@@ -35,6 +35,16 @@
  * scoring backward's zero grad_x rows produce through a per-ROI head).  Zero padding masks let the overlap kernel skip
  * them.
  *
+ * Compact ragged batches (cim_score_heads_compact, cim_score_heads_bwd_compact).  The per-proposal features need not
+ * be padded: with N = sum_b n_b, proposal r < n_b of image b sits at row off_b + r, off_b = sum_{i<b} n_i, of x /
+ * grad_x [N, D], and the caller runs RoIAlign (K = N rois, grouped by image in ascending order; no kernel has a
+ * proposal-count form, each roi carries its image index) and its per-proposal head on N rows only.  The scores and
+ * everything after them (mining, assignment, losses, PCL) stay padded with capacity R, exactly as above.  The library
+ * maps compact row m to padded row b * R + r on the device from n_props (clamped to [1, R]) and N, with no host
+ * synchronisation; the counts behind N must be the ones in n_props.  If they are not: compact rows m >= sum_b n_b are
+ * ignored (their grad_x rows are 0); if sum_b n_b > N, the proposals past row N have no compact row and the score
+ * rows they would fill are left unwritten.  No memory is touched out of bounds in either case.
+ *
  * Images of different sizes (the RoIAlign _ex entry points).  feat [B,C,H,W] is a CANVAS: image b occupies the top
  * left [0, H_b) x [0, W_b) of its plane.  feat_hw is a device int32 [B][2] array of the (H_b, W_b), 4-byte aligned;
  * NULL means (H, W) for every image, and each RoIAlign entry point without _ex is its NULL case.  The kernels clamp
@@ -59,7 +69,7 @@ extern "C" {
 
 typedef struct CUstream_st *cim_stream_t;   /* == cudaStream_t */
 
-#define CIM_ABI_VERSION 6
+#define CIM_ABI_VERSION 7
 
 enum {
     CIM_OK = 0,
@@ -97,6 +107,10 @@ int cim_debug_roi_window_plan(const float *rois, int K, int B, int H, int W, flo
 int cim_debug_roi_window_plan_ex(const float *rois, const int32_t *feat_hw, int K, int B, int H, int W, float scale,
                                  int sampling_ratio, int aligned, int *desc_out, int *key_out, int cap, int *flag_out,
                                  int *geom_out);
+/* Test hook, HOST memory only: the row map of compact ragged batches (see "Compact ragged batches" above) from host
+ * counts n_props [n_img] (NULL: R each), computed by the code the device builder runs.  map_out [N]: the padded row
+ * b * R + r of each compact row, -1 for rows past sum_b n_b.  N <= n_img * R. */
+int cim_debug_compact_row_map(const int32_t *n_props, int n_img, int R, int N, int32_t *map_out);
 
 /* ------------------------------------------------------------------ ROI operators
  * Replace mmcv.ops.RoIAlign / RoIPool as imported by lib/ops/__init__.py:6 and called at
@@ -330,6 +344,17 @@ int cim_score_heads_ex(const float *x, const float *weight, const float *bias, f
                        int n_img, int R, int D, int C1, int K,
                        void *workspace, size_t workspace_bytes, cim_stream_t stream);
 
+/* Compact ragged form: x [N, D] holds the proposals of the images back to back (see the top of this file), scores
+ * [n_heads, n_img*R, C1] is padded as for cim_score_heads_ex, with the same values on every proposal row and 0 on the
+ * padding rows.  Each row's result does not depend on the other rows: a proposal's scores equal those of the padded
+ * call bit for bit.  N <= n_img*R; n_props may be NULL (n_b = R, then N = n_img*R is the padded call's x).  workspace:
+ * cim_score_heads_compact_workspace_bytes() bytes, required (it also holds the row map); the value for N = n_img*R
+ * covers every smaller N.  The GEMM runs on the tensor cores when N >= 128, as fp32 FFMA otherwise. */
+size_t cim_score_heads_compact_workspace_bytes(int n_img, int R, int N, int D, int C1, int K);
+int cim_score_heads_compact(const float *x, const float *weight, const float *bias, float *scores,
+                            const int32_t *n_props, int n_img, int R, int N, int D, int C1, int K,
+                            void *workspace, size_t workspace_bytes, cim_stream_t stream);
+
 /* Backward of cim_score_heads = autograd of heads.cls_iou_model.forward (lib/modeling/heads.py:194-219; the
  * reference gets it from eight nn.Linear backward calls + softmax / sigmoid backward, run by loss.backward(),
  * tools/train.py:436).  grad_weight / grad_bias are the head gradients a data-parallel run all-reduces
@@ -355,6 +380,16 @@ int cim_score_heads_bwd_ex(const float *x, const float *weight, const float *sco
                            const int32_t *n_props, float *grad_x, float *grad_weight, float *grad_bias,
                            int n_img, int R, int D, int C1, int K,
                            void *workspace, size_t workspace_bytes, cim_stream_t stream);
+/* Compact ragged form: x and grad_x [N, D] compact, scores and grad_scores padded [n_heads, n_img*R, C1] (the
+ * output of cim_score_heads_compact and its gradient).  The real rows of grad_x equal the padded call's rows bit for
+ * bit; grad_weight / grad_bias sum over N rows instead of n_img*R, so they agree with the padded call to fp32
+ * summation order.  workspace: cim_score_heads_bwd_compact_workspace_bytes() bytes, required; the value for
+ * N = n_img*R covers every smaller N.  Tensor cores when N >= 128 and D % 4 == 0. */
+size_t cim_score_heads_bwd_compact_workspace_bytes(int n_img, int R, int N, int D, int C1, int K);
+int cim_score_heads_bwd_compact(const float *x, const float *weight, const float *scores, const float *grad_scores,
+                                const int32_t *n_props, float *grad_x, float *grad_weight, float *grad_bias,
+                                int n_img, int R, int N, int D, int C1, int K,
+                                void *workspace, size_t workspace_bytes, cim_stream_t stream);
 
 /* ------------------------------------------------------------------ CIM mining + assignment
  * Replace heads.CIM_layer (lib/modeling/heads.py:222-503) for n_img images x n_layers

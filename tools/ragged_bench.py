@@ -1,12 +1,16 @@
-"""Cost of ragged batches in CIMHeadStep.run at bench.py's cfg2 shape (ResNet-50, VOC, 8 images x 2000 proposals,
-head gradients and PCL_loss on).  Three forms run alternately in one process, on the same inputs and buffers:
-  none    n_props = None (every image has R proposals; the entry points' NULL case)
-  full    n_props = R for every image, through the ragged kernels
-  ragged  a seeded draw of n_b uniform in [200, 2000]: what padding to the capacity costs against a batch
-          that would hold only sum(n_b) proposals
-Prints the card, its power limit and the median / spread of the per-step times of each form.
+"""Cost of ragged batches in CIMHeadStep.run at one of bench.py's 8 x 2000 shapes (default cfg2: ResNet-50, VOC; cfg3:
+VGG-16, whose 64 x 64 maps take the RoIAlign window path), head gradients and PCL_loss on.  Four forms run alternately
+in one process, on the same inputs and buffers:
+  none     n_props = None (every image has R proposals; the entry points' NULL case)
+  full     n_props = R for every image, through the ragged kernels
+  ragged   a seeded draw of n_b uniform in [200, 2000] in the padded layout: every stage but mining still does the
+           work of n_img x R rows
+  compact  the same draw in the compact layout (run(compact=True)): rois, RoIAlign outputs and seg_x hold the
+           sum(n_b) real rows only
+Prints the card, its power limit, the median / spread of the per-step times of each form, and the rows that RoIAlign,
+the scoring GEMMs and a caller's MaskFuse process in each form (a count: MaskFuse is not part of the step).
 
-    python tools/ragged_bench.py [--steps 20] [--rounds 5] [--sampling stream|hop]
+    python tools/ragged_bench.py [--workload cfg3_vgg16_voc_8x2000] [--steps 20] [--rounds 5] [--sampling stream|hop]
 """
 import argparse
 import os
@@ -37,11 +41,12 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--sampling", default="stream", choices=["stream", "hop"])
     ap.add_argument("--seed", type=int, default=2024, help="seed of the ragged draw")
+    ap.add_argument("--workload", default="cfg2_r50_voc_8x2000", choices=["cfg2_r50_voc_8x2000", "cfg3_vgg16_voc_8x2000"])
     a = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit("ragged_bench.py measures on the GPU; no CUDA device found")
     dev = torch.device("cuda:0")
-    cfg = bench.WORKLOADS["cfg2_r50_voc_8x2000"]
+    cfg = bench.WORKLOADS[a.workload]
     inp = bench.build_inputs(cfg, dev, 1234)
     Cf, H, W, scale = inp["shape"]
     n_img, R = cfg["n_img"], cfg["R"]
@@ -50,11 +55,18 @@ def main():
     ragged = np.random.RandomState(a.seed).randint(200, R + 1, size=n_img).astype(np.int32)
     forms = {"none": None,
              "full": torch.full((n_img,), R, dtype=torch.int32, device=dev),
-             "ragged": torch.from_numpy(ragged).to(dev)}
+             "ragged": torch.from_numpy(ragged).to(dev),
+             "compact": ragged}
+    # the compact form's inputs: the real rows of the padded ones (rois keep their image index)
+    idx = torch.from_numpy(np.concatenate([b * R + np.arange(n) for b, n in enumerate(ragged)])).to(dev)
+    comp = {k: inp[k].index_select(0, idx).contiguous() for k in ("rois", "grad_out", "seg_x")}
+    n_rows = int(ragged.sum())
 
     def run(n_props):
-        step.run(inp["feat"], inp["rois"], inp["grad_out"], inp["packed"], inp["seg_x"], inp["weight"], inp["bias"],
-                 inp["labels"], mat=inp["mat"], mask_meta=inp["mask_meta"], n_props=n_props)
+        src = comp if isinstance(n_props, np.ndarray) else inp
+        step.run(inp["feat"], src["rois"], src["grad_out"], inp["packed"], src["seg_x"], inp["weight"], inp["bias"],
+                 inp["labels"], mat=inp["mat"], mask_meta=inp["mask_meta"], n_props=n_props,
+                 compact=src is comp)
 
     np.random.seed(3)
     for n_props in forms.values():
@@ -73,15 +85,17 @@ def main():
             ev1.synchronize()
             step.sync_rng()
             times[name].append(ev0.elapsed_time(ev1) / a.steps)
-    print(f"{torch.cuda.get_device_name(dev)}, power limit {power_limit()}: CIMHeadStep.run at cfg2 "
+    print(f"{torch.cuda.get_device_name(dev)}, power limit {power_limit()}: CIMHeadStep.run at {a.workload} "
           f"({n_img} x {R}, head gradients, PCL_loss, sampling {a.sampling}), {a.rounds} rounds x {a.steps} steps")
     print(f"ragged n_b = {ragged.tolist()}: {int(ragged.sum())} of {n_img * R} rows "
           f"({100.0 * (1 - ragged.sum() / (n_img * R)):.1f} % padding)")
     med = {k: float(np.median(v)) for k, v in times.items()}
     for name, v in times.items():
-        print(f"  {name:6s} median {med[name]:.3f} ms/step  (min {min(v):.3f}, max {max(v):.3f}); "
-              f"{n_img / med[name] * 1e3:.0f} images/s")
-    print(f"  full / none = {med['full'] / med['none']:.4f}; ragged / none = {med['ragged'] / med['none']:.4f}")
+        rows = n_rows if name == "compact" else n_img * R
+        print(f"  {name:7s} median {med[name]:.3f} ms/step  (min {min(v):.3f}, max {max(v):.3f}); "
+              f"{n_img / med[name] * 1e3:.0f} images/s; rows through RoIAlign, scoring GEMMs and MaskFuse: {rows}")
+    print(f"  full / none = {med['full'] / med['none']:.4f}; ragged / none = {med['ragged'] / med['none']:.4f}; "
+          f"compact / ragged = {med['compact'] / med['ragged']:.4f}")
 
 
 if __name__ == "__main__":
