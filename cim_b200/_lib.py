@@ -68,6 +68,8 @@ _SIGNATURES = {
     "cim_mask_meta_bytes": (_SZ, [_I, _I, _I64]),
     "cim_mask_unpack_crops_tiled_meta": (_I, [_P, _P, _P, _P, _P, _SZ, _I, _I, _I, _I, _I64, _P]),
     "cim_mask_unpack_crops_tiled_meta_sparse": (_I, [_P, _P, _P, _P, _P, _P, _SZ, _I, _I, _I, _I, _I64, _P]),
+    "cim_mask_unpack_rle_tiled_meta_sparse": (_I, [_P, _I64, _P, _P, _P, _P, _P, _P, _SZ, _I, _I, _I, _I, _I64, _P,
+                                                    _P]),
     "cim_mask_meta": (_I, [_P, _I, _I, _I64, _I, _P, _SZ, _P]),
     "cim_mask_overlap_meta": (_I, [_P, _P, _I, _I, _I64, _I, _P, _P, _P, _P, _P, _SZ, _I, _P]),
     "cim_mask_pair_ratio": (_I, [_P, _P, _I, _I, _I64, _I, _P, _P, _P, _P, _P]),

@@ -22,6 +22,7 @@
 //                         upper triangle of tiles is computed, the mirror tile is written from
 //                         the same counts (inter is symmetric, asy is not)
 #include "common.cuh"
+#include "mask_patch.cuh"
 
 // mask_overlap_tc.cu: the tcgen05 (tensor core) path for large problems
 bool cim_mask_overlap_tc_eligible(int n, long long words);
@@ -29,6 +30,11 @@ int cim_mask_overlap_tc_launch(const uint32_t *packed, const int32_t *area, cons
                                const uint32_t *umap_a, const uint32_t *umap_b, int bw, unsigned long long *visited,
                                const int32_t *tile_order, int n_img, int n, long long words, int32_t *inter,
                                __half *iou, __half *asy, cudaStream_t st);
+// mask_rle.cu: COCO RLE strings -> tiled bit masks + metadata (cim_mask_unpack_rle_tiled_meta_sparse)
+int cim_mask_unpack_rle_launch(const uint8_t *chars, long long n_chars, const int64_t *off, const int32_t *len,
+                               const int32_t *mask_hw, uint32_t *packed, int32_t *prev_rects, int32_t *area,
+                               uint32_t *kbmap, int4 *kinfo, long long n_masks, int n, int H, int W, long long words,
+                               int bw, int32_t *bad, cudaStream_t st);
 
 namespace {
 
@@ -204,13 +210,11 @@ __global__ void mask_unpack_crops_tiled_meta_sparse_kernel(const uint32_t *__res
     const uint32_t *src = crop_words + off[m];
     uint4 *row4 = reinterpret_cast<uint4 *>(packed + m * words);
     const int bpr = W >> 4, nby = H >> 3;
-    // patch rectangles (16-pixel columns x 8-pixel rows) of the new and the old crop, clipped to the image
-    int bx_lo = bpr, bx_hi = 0, by_lo = nby, by_hi = 0;          // [lo, hi)
-    if (ww > 0 && h > 0) { bx_lo = min(bx_lo, 2 * wx0); bx_hi = max(bx_hi, 2 * (wx0 + ww)); by_lo = min(by_lo, y0 >> 3); by_hi = max(by_hi, ((y0 + h - 1) >> 3) + 1); }
-    if (pv.z > 0 && pv.w > 0) { bx_lo = min(bx_lo, 2 * pv.x); bx_hi = max(bx_hi, 2 * (pv.x + pv.z)); by_lo = min(by_lo, pv.y >> 3); by_hi = max(by_hi, ((pv.y + pv.w - 1) >> 3) + 1); }
-    bx_lo = max(bx_lo, 0); by_lo = max(by_lo, 0); bx_hi = min(bx_hi, bpr); by_hi = min(by_hi, nby);
+    // patch rectangle (16-pixel columns x 8-pixel rows) of the new and the old crop, clipped to the image
+    int bx_lo, bx_hi, by_lo, by_hi;                              // [lo, hi)
+    patch_union(make_int4(wx0, y0, ww, h), pv, bpr, nby, &bx_lo, &bx_hi, &by_lo, &by_hi);
     const int nx = max(bx_hi - bx_lo, 0), cells = nx * max(by_hi - by_lo, 0);
-    int s = 0, alo = 0x7fffffff, ahi = -1, blo = 0x7fffffff, bhi = -1;
+    PatchMeta acc;
     __syncwarp();
     for (int e = lane; e < cells; e += 32) {
         const int by = by_lo + e / nx, bx = bx_lo + e % nx, kb = by * bpr + bx;
@@ -228,26 +232,13 @@ __global__ void mask_unpack_crops_tiled_meta_sparse_kernel(const uint32_t *__res
             }
             v = make_uint4(o[0], o[1], o[2], o[3]);
         }
-        row4[kb] = v;
-        s += __popc(v.x) + __popc(v.y) + __popc(v.z) + __popc(v.w);
-        if ((v.x | v.y | v.z | v.w) != 0u) {
-            atomicOr(bm + (kb >> 5), 1u << (kb & 31));
-            alo = min(alo, bx); ahi = max(ahi, bx); blo = min(blo, by); bhi = max(bhi, by);
-        }
+        acc.store(row4, bm, kb, bx, by, v);
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        s += __shfl_xor_sync(0xffffffffu, s, o);
-        alo = min(alo, __shfl_xor_sync(0xffffffffu, alo, o));
-        ahi = max(ahi, __shfl_xor_sync(0xffffffffu, ahi, o));
-        blo = min(blo, __shfl_xor_sync(0xffffffffu, blo, o));
-        bhi = max(bhi, __shfl_xor_sync(0xffffffffu, bhi, o));
-    }
+    acc.warp_reduce();
     __syncwarp();
     for (int j = lane; j < bw; j += 32) kbmap[m * bw + j] = bm[j];
     if (lane == 0) {
-        area[m] = s;
-        kinfo[m] = ahi >= 0 ? make_int4(1, alo + ahi, blo + bhi, 0) : make_int4(0, 0, 0, 0);
+        acc.write(area, kinfo, m);
         prev[m] = make_int4(wx0, y0, ww, h);
     }
 }
@@ -739,6 +730,29 @@ CIM_API int cim_mask_unpack_crops_tiled_meta_sparse(const uint32_t *crop_words, 
         crop_words, crop_meta, reinterpret_cast<const long long *>(crop_off), packed, reinterpret_cast<int4 *>(prev_rects),
         mm.area, mm.kbmap, mm.kinfo, n_masks, H, W, words, bw);
     return cim_launch_status();
+}
+
+CIM_API int cim_mask_unpack_rle_tiled_meta_sparse(const uint8_t *chars, int64_t n_chars, const int64_t *off,
+                                                  const int32_t *len, const int32_t *mask_hw, uint32_t *packed,
+                                                  int32_t *prev_rects, void *meta, size_t meta_bytes, int n_img, int n,
+                                                  int H, int W, int64_t words, int32_t *bad, cim_stream_t stream) {
+    if (!off || !len || !packed || !prev_rects || !meta || (n_chars > 0 && !chars) || n_chars < 0 || n_img < 0 ||
+        n < 0 || H <= 0 || W <= 0)
+        return CIM_ERR_ARG;
+    if ((H & 7) || (W & 15) || (int64_t)H * W > 0x7fffffffLL || ((W + 31) & ~31) > CIM_RLE_UNPACK_BITMAP_WORDS)
+        return CIM_ERR_SHAPE;
+    if (words * 32 != (int64_t)H * W || (words & 3) || !cim_aligned(packed, 16) || !cim_aligned(prev_rects, 16) ||
+        !cim_aligned(off, 8) || !cim_aligned(len, 4) || (mask_hw && !cim_aligned(mask_hw, 4)) ||
+        (bad && !cim_aligned(bad, 4)))
+        return CIM_ERR_ALIGN;
+    if (meta_bytes < cim_mask_meta_bytes(n_img, n, words) || !cim_aligned(meta, 256)) return CIM_ERR_WORKSPACE;
+    const long long n_masks = (long long)n_img * n;
+    if (n_masks > 0x7fffffffLL) return CIM_ERR_SHAPE;
+    const int bw = (int)(((words + 3) / 4 + 31) / 32);
+    if (bw > 2048) return CIM_ERR_SHAPE;                                // the row's K-block bitmap in shared memory
+    const MaskMeta mm = carve_meta(meta, n_img, n, words);
+    return cim_mask_unpack_rle_launch(chars, n_chars, off, len, mask_hw, packed, prev_rects, mm.area, mm.kbmap,
+                                      mm.kinfo, n_masks, n, H, W, words, bw, bad, (cudaStream_t)stream);
 }
 
 CIM_API size_t cim_mask_overlap_workspace_bytes(int n_img, int n, int64_t words, int want_inter) {

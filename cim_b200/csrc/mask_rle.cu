@@ -11,7 +11,20 @@
 //                 transition positions i .. i-3, so the CTA keeps the last three positions across chunks and stores
 //                 no counts.  The same template runs twice: a length pass (string length, area, box), a scan of
 //                 the lengths over all slots (offsets, need[]), then an emit pass that writes the characters.
+//
+//  cim_mask_unpack_rle_kernel : the way back, COCO compressed RLE strings (rleFrString + rleDecode) -> tiled bit masks
+//                 and their metadata, as the sparse update of mask_patch.cuh.  One CTA per row.  The string is parsed
+//                 256 characters at a time: a ballot over the continuation bit finds where counts end, a block scan
+//                 numbers them, and the count's value is read from its first (at most 7) characters -- only the low
+//                 32 bits of rleFrString's long survive its (uint) cast.  The delta coding (x += cnts[m-2], m > 2) is
+//                 two interleaved prefix sums (even and odd counts), a third scan gives the run boundaries; the last
+//                 count index, the two chain sums and the running position are carried across chunks.  The ones-runs
+//                 are painted as column intervals into a column-major bitmap of a band of rows in shared memory (32
+//                 rows per word), 32 x 32 blocks are transposed back with ballots into 8 x 16 patches, and the union
+//                 of the old and the new rectangle is written.  An image too large for one band re-walks the string
+//                 per band.  A malformed string gives an empty row and is counted.
 #include "common.cuh"
+#include "mask_patch.cuh"
 
 #include <limits.h>
 
@@ -307,7 +320,243 @@ cim_mask_rle_scan_kernel(const int32_t *__restrict__ sel_count, const int32_t *_
     }
 }
 
+// ------------------------------------------------------------------------------- RLE strings -> tiled bit masks
+constexpr int RU_THREADS = 256;
+constexpr int RU_WARPS = RU_THREADS / 32;
+// 4 CTAs per SM: 64 registers (no spills) and 32 KB of band bitmap + the K-block bitmap + 3.6 KB static each
+
+__global__ void __launch_bounds__(RU_THREADS, 4)
+cim_mask_unpack_rle_kernel(const uint8_t *__restrict__ chars, long long n_chars, const long long *__restrict__ off,
+                           const int32_t *__restrict__ len, const int32_t *__restrict__ mask_hw,
+                           uint32_t *__restrict__ packed, int4 *__restrict__ prev, int32_t *__restrict__ area,
+                           uint32_t *__restrict__ kbmap, int4 *__restrict__ kinfo, int n, int H, int W,
+                           long long words, int bw, int32_t *__restrict__ bad) {
+    extern __shared__ uint32_t s_dyn[];
+    uint32_t *const s_bmp = s_dyn;                       // [RLE_UNPACK_BITMAP_WORDS] word (rb, x) = rows 32 rb.. of x
+    uint32_t *const s_kb = s_dyn + CIM_RLE_UNPACK_BITMAP_WORDS;     // [bw] the row's K-block bitmap
+    __shared__ int s_wi[32];
+    __shared__ unsigned s_wu[32];
+    __shared__ long long s_wl[32];
+    __shared__ int s_wlast[RU_WARPS];                   // last count-ending character of each warp of the chunk
+    __shared__ int s_seg[RU_THREADS], s_ra[RU_THREADS], s_rb[RU_THREADS];   // column segments (inclusive scan), runs
+    __shared__ int s_box[4];                            // xmin, xmax, ymin, ymax of the ones
+    __shared__ int s_acc[5];                            // PatchMeta of the CTA
+    const long long m = blockIdx.x;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int b = (int)(m / n);
+    int h = H, w = W;
+    if (mask_hw) {
+        h = min(max(mask_hw[2 * b], 1), H);
+        w = min(max(mask_hw[2 * b + 1], 1), W);
+    }
+    const long long hw = (long long)h * w;
+    const long long o = off[m];
+    const int L = len[m];
+    bool row_bad = L < 0 || o < 0 || o > n_chars - L;
+    const uint8_t *s = chars + (row_bad ? 0 : o);
+    const int bpr = W >> 4, nby = H >> 3;
+    const int bc = (w + 31) & ~31;                                   // bitmap columns
+    const int nrb = min(CIM_RLE_UNPACK_BITMAP_WORDS / bc, (h + 31) >> 5);   // 32-row blocks per band
+    const int BR = 32 * nrb;
+
+    for (int i = tid; i < nrb * bc; i += RU_THREADS) s_bmp[i] = 0u;
+    for (int i = tid; i < bw; i += RU_THREADS) s_kb[i] = 0u;
+    if (tid == 0) {
+        s_box[0] = INT_MAX; s_box[1] = -1; s_box[2] = INT_MAX; s_box[3] = -1;
+        s_acc[0] = 0; s_acc[1] = INT_MAX; s_acc[2] = -1; s_acc[3] = INT_MAX; s_acc[4] = -1;
+    }
+    __syncthreads();
+
+    int xmin = INT_MAX, xmax = -1, ymin = INT_MAX, ymax = -1;
+    // rleFrString + rleDecode over the whole string: paints the ones of rows [yb0, yb1) into s_bmp; with `first` also
+    // validates and records the box.  Returns true (block-uniform) for a malformed string.
+    auto walk = [&](int yb0, int yb1, bool first) {
+        unsigned cE = 0u, cO = 0u;                      // sums of the even (m >= 2) / odd deltas before the chunk
+        long long pos = 0, mbase = 0;                   // pixels / counts before the chunk
+        int last_end = -1;                              // last count-ending character before the chunk
+        for (int c0 = 0; c0 < L; c0 += RU_THREADS) {
+            const int i = c0 + tid;
+            const bool have = i < L;
+            const int v = have ? (int)__ldg(s + i) - 48 : 0;
+            bool my_bad = have && (v < 0 || v > 63);
+            const bool cont = have && (v & 0x20);
+            const bool end = have && !cont;
+            if (i == L - 1 && cont) my_bad = true;      // the string stops inside a count
+            const unsigned eb = __ballot_sync(0xffffffffu, end);
+            if (lane == 0) s_wlast[warp] = eb ? c0 + 32 * warp + 31 - __clz(eb) : -1;
+            int n_end;
+            const int r0 = block_scan<int>(end ? 1 : 0, s_wi, &n_end);   // (its barriers publish s_wlast)
+            unsigned x = 0u;
+            if (end) {                                  // the count spans characters st .. i
+                const unsigned below = eb & ((1u << lane) - 1u);
+                int pe = last_end;
+                if (below) {
+                    pe = c0 + 32 * warp + 31 - __clz(below);
+                } else {
+                    for (int q = 0; q < warp; ++q) pe = max(pe, s_wlast[q]);
+                }
+                const int st = pe + 1, K = i - st + 1;
+                for (int k = 0; k < min(K, 7); ++k) x |= (unsigned)((__ldg(s + st + k) - 48) & 0x1f) << (5 * k);
+                if ((v & 0x10) && K <= 6) x |= 0xffffffffu << (5 * K);     // sign extension (mod 2^32)
+            }
+            const long long mi = mbase + r0;            // count index
+            const unsigned ev = (end && mi >= 2 && !(mi & 1)) ? x : 0u, ov = (end && (mi & 1)) ? x : 0u;
+            unsigned tE, tO;
+            const unsigned E = cE + block_scan<unsigned>(ev, s_wu, &tE) + ev;
+            const unsigned O = cO + block_scan<unsigned>(ov, s_wu, &tO) + ov;
+            const unsigned cnt = mi == 0 ? x : ((mi & 1) ? O : E);
+            long long tP;
+            const long long c64 = end ? (long long)cnt : 0;
+            const long long P = pos + block_scan<long long>(c64, s_wl, &tP) + c64;   // end of run mi
+            if (end && (c64 > hw || P > hw)) my_bad = true;
+            const bool run = end && (mi & 1) && cnt > 0u && c64 <= hw && P <= hw;
+            const int ra = run ? (int)(P - c64) : 0, rb = run ? (int)P : 0;
+            const int xa = run ? ra / h : 0, xb = run ? (rb - 1) / h : -1;
+            if (first && run) {
+                xmin = min(xmin, xa);
+                xmax = max(xmax, xb);
+                if (xa == xb) {
+                    ymin = min(ymin, ra - xa * h);
+                    ymax = max(ymax, rb - 1 - xb * h);
+                } else {                                // a run across a column boundary covers rows 0 and h-1
+                    ymin = 0;
+                    ymax = h - 1;
+                }
+            }
+            int n_seg;
+            const int sg = block_scan<int>(xb - xa + 1, s_wi, &n_seg);
+            s_seg[tid] = sg + xb - xa + 1;
+            s_ra[tid] = ra;
+            s_rb[tid] = rb;
+            if (n_end) {                                // (s_wlast is rewritten only after the barrier below)
+                int le = -1;
+                for (int q = 0; q < RU_WARPS; ++q) le = max(le, s_wlast[q]);
+                last_end = le;
+            }
+            __syncthreads();
+            for (int j = tid; j < n_seg; j += RU_THREADS) {     // one column segment of one run per iteration
+                int lo = 0, hi = RU_THREADS - 1;
+                while (lo < hi) {
+                    const int mid = (lo + hi) >> 1;
+                    if (s_seg[mid] > j) hi = mid; else lo = mid + 1;
+                }
+                const int a = s_ra[lo], e = s_rb[lo], ca = a / h, ce = (e - 1) / h;
+                const int xc = ce + 1 + j - s_seg[lo];
+                const int y0 = max(xc == ca ? a - ca * h : 0, yb0), y1 = min(xc == ce ? e - 1 - ce * h : h - 1, yb1 - 1);
+                for (int y = y0; y <= y1;) {
+                    const int r = (y - yb0) >> 5, ye = min(y1, yb0 + 32 * r + 31);
+                    const unsigned bits = (0xffffffffu >> (31 - ((ye - yb0) & 31))) & (0xffffffffu << ((y - yb0) & 31));
+                    uint32_t *wp = s_bmp + r * bc + xc;
+                    if (bits == 0xffffffffu) *wp = bits;        // no other run touches a word this one fills
+                    else atomicOr(wp, bits);
+                    y = ye + 1;
+                }
+            }
+            if (__syncthreads_or(my_bad)) return true;
+            cE += tE;
+            cO += tO;
+            pos += tP;
+            mbase += n_end;
+        }
+        return pos != hw;
+    };
+
+    uint4 *row4 = reinterpret_cast<uint4 *>(packed + m * words);
+    const int4 pv = prev[m];
+    int4 nr = make_int4(0, 0, 0, 0);
+    int ytop = 0, bx_lo = 0, bx_hi = 0, by_lo = 0, by_hi = 0;
+    PatchMeta acc;
+    for (int yb0 = 0;; yb0 += BR) {
+        // band 0: the walk that validates and finds the box; later bands re-walk only where the new mask has rows
+        if (yb0 == 0 ? !row_bad && L > 0 : nr.w > 0 && yb0 < nr.y + nr.w && yb0 + BR > nr.y) {
+            const bool wb = walk(yb0, yb0 + BR, yb0 == 0);
+            if (yb0 == 0) row_bad = wb;
+        }
+        if (yb0 == 0) {
+            if (row_bad) {
+                for (int i = tid; i < nrb * bc; i += RU_THREADS) s_bmp[i] = 0u;
+            } else if (xmax >= 0) {
+                atomicMin(&s_box[0], xmin);
+                atomicMax(&s_box[1], xmax);
+                atomicMin(&s_box[2], ymin);
+                atomicMax(&s_box[3], ymax);
+            }
+            __syncthreads();
+            if (s_box[1] >= 0 && !row_bad)
+                nr = make_int4(s_box[0] >> 5, s_box[2], (s_box[1] >> 5) - (s_box[0] >> 5) + 1, s_box[3] - s_box[2] + 1);
+            if (nr.z > 0 && nr.w > 0) ytop = nr.y + nr.w;
+            if (pv.z > 0 && pv.w > 0) ytop = max(ytop, pv.y + pv.w);
+            patch_union(nr, pv, bpr, nby, &bx_lo, &bx_hi, &by_lo, &by_hi);
+        }
+        // the union's patches in this band: 32 x 32 blocks of the bitmap (cleared as they are read) -> 8 patches each
+        const int pl = max(by_lo, yb0 >> 3), ph = min(by_hi, (yb0 + BR) >> 3);
+        if (bx_hi > bx_lo && ph > pl) {
+            const int wx_lo = bx_lo >> 1, nwx = ((bx_hi + 1) >> 1) - wx_lo;
+            const int rb_lo = (8 * pl - yb0) >> 5, nblk = nwx * (((8 * ph - 1 - yb0) >> 5) + 1 - rb_lo);
+            for (int t = warp; t < nblk; t += RU_WARPS) {
+                const int r = rb_lo + t / nwx, wx = wx_lo + t % nwx;
+                const int col = 32 * wx + lane;
+                uint32_t cw = 0u;
+                if (col < bc) {
+                    cw = s_bmp[r * bc + col];
+                    s_bmp[r * bc + col] = 0u;
+                }
+                uint32_t rw = 0u;                       // row yb0 + 32 r + lane, columns 32 wx ..
+                if (__ballot_sync(0xffffffffu, cw != 0u)) {
+#pragma unroll
+                    for (int c = 0; c < 32; ++c) {
+                        const uint32_t bal = __ballot_sync(0xffffffffu, (cw >> c) & 1u);
+                        if (lane == c) rw = bal;
+                    }
+                }
+                const int pr = (lane >> 1) & 3, sh = 16 * (lane & 1);      // lanes 0..7: patch row pr, left / right
+                uint32_t q[8];
+#pragma unroll
+                for (int j = 0; j < 8; ++j) q[j] = (__shfl_sync(0xffffffffu, rw, 8 * pr + j) >> sh) & 0xffffu;
+                const int by = (yb0 >> 3) + 4 * r + pr, bx = 2 * wx + (lane & 1);
+                if (lane < 8 && by >= pl && by < ph && bx >= bx_lo && bx < bx_hi)
+                    acc.store(row4, s_kb, by * bpr + bx, bx, by,
+                              make_uint4(q[0] | (q[1] << 16), q[2] | (q[3] << 16), q[4] | (q[5] << 16), q[6] | (q[7] << 16)));
+            }
+        }
+        __syncthreads();                                // the bitmap is clear again
+        if (yb0 + BR >= ytop) break;
+    }
+    acc.warp_reduce();
+    if (lane == 0 && acc.ahi >= 0) {
+        atomicAdd(&s_acc[0], acc.s);
+        atomicMin(&s_acc[1], acc.alo);
+        atomicMax(&s_acc[2], acc.ahi);
+        atomicMin(&s_acc[3], acc.blo);
+        atomicMax(&s_acc[4], acc.bhi);
+    }
+    __syncthreads();
+    for (int j = tid; j < bw; j += RU_THREADS) kbmap[m * bw + j] = s_kb[j];
+    if (tid == 0) {
+        PatchMeta tot;
+        tot.s = s_acc[0]; tot.alo = s_acc[1]; tot.ahi = s_acc[2]; tot.blo = s_acc[3]; tot.bhi = s_acc[4];
+        tot.write(area, kinfo, m);
+        prev[m] = nr;
+        if (row_bad && bad) atomicAdd(bad, 1);
+    }
+}
+
 }  // namespace
+
+// The launch behind cim_mask_unpack_rle_tiled_meta_sparse (mask_overlap.cu, which owns the metadata layout); the
+// arguments are checked there.
+int cim_mask_unpack_rle_launch(const uint8_t *chars, long long n_chars, const int64_t *off, const int32_t *len,
+                               const int32_t *mask_hw, uint32_t *packed, int32_t *prev_rects, int32_t *area,
+                               uint32_t *kbmap, int4 *kinfo, long long n_masks, int n, int H, int W, long long words,
+                               int bw, int32_t *bad, cudaStream_t st) {
+    if (bad) cudaMemsetAsync(bad, 0, sizeof(int32_t), st);
+    if (n_masks > 0)
+        cim_mask_unpack_rle_kernel<<<(unsigned)n_masks, RU_THREADS,
+                                     ((size_t)CIM_RLE_UNPACK_BITMAP_WORDS + bw) * sizeof(uint32_t), st>>>(
+            chars, n_chars, reinterpret_cast<const long long *>(off), len, mask_hw, packed,
+            reinterpret_cast<int4 *>(prev_rects), area, kbmap, kinfo, n, H, W, words, bw, bad);
+    return cim_launch_status();
+}
 
 CIM_API int cim_mask_rle(const uint32_t *packed, int n_img, int R, int64_t words, int H, int W, int kb_per_row,
                          const int32_t *mask_hw, const int32_t *sel_count, const int32_t *sel_idx, int cap,

@@ -126,6 +126,114 @@ def batch_crops_host(crops, R, height, width):
                      torch.from_numpy(off), height, width)
 
 
+@dataclass
+class MaskRLE:
+    """Proposal masks as COCO compressed RLE strings (what pycocotools.mask.encode returns as 'counts'), the other wire
+    format: row m's string is chars[off[m] : off[m] + len[m]], len 0 = a row of zeros.  chars uint8 [total], off int64
+    [rows], len int32 [rows], hw int32 [n_img, 2] = each image's native (h, w) on the (height, width) canvas, where its
+    masks sit at the top left.  Host (pinned torch) or device tensors.  mask_rle's device outputs (chars, off, len) plug
+    in directly."""
+    chars: torch.Tensor
+    off: torch.Tensor
+    len: torch.Tensor
+    hw: torch.Tensor
+    height: int
+    width: int
+
+    @property
+    def nbytes(self):
+        return sum(t.numel() * t.element_size() for t in (self.chars, self.off, self.len, self.hw))
+
+
+def batch_rle_host(per_image, R, height, width):
+    """CPU: the RLE wire format of a batch.  per_image: one list per image of COCO dicts {'size': [h, w], 'counts':
+    bytes | str} (compressed strings, e.g. from pycocotools.mask.encode), n_b <= R of them, all of one size -> a
+    MaskRLE of len(per_image) * R rows, image b in rows [b * R, b * R + n_b) and len 0 in its padding rows.  An image
+    whose masks differ in size or exceed the (height, width) canvas raises, and so do uncompressed (list) counts.  An
+    image without masks takes the canvas size."""
+    n_img = len(per_image)
+    off = np.zeros(n_img * R, np.int64)
+    lens = np.zeros(n_img * R, np.int32)
+    hw = np.zeros((n_img, 2), np.int32)
+    chunks, total = [], 0
+    for b, dicts in enumerate(per_image):
+        if len(dicts) > R:
+            raise ValueError(f"image {b}: {len(dicts)} masks exceed R = {R}")
+        sizes = {tuple(int(v) for v in d["size"]) for d in dicts}
+        if len(sizes) > 1:
+            raise ValueError(f"image {b}: masks of different sizes {sorted(sizes)}")
+        h, w = sizes.pop() if sizes else (height, width)
+        if not (1 <= h <= height and 1 <= w <= width):
+            raise ValueError(f"image {b}: native size {h} x {w} exceeds the canvas {height} x {width}")
+        hw[b] = (h, w)
+        for i, d in enumerate(dicts):
+            c = d["counts"]
+            if isinstance(c, str):
+                c = c.encode("ascii")
+            if not isinstance(c, (bytes, bytearray)):
+                raise ValueError(f"image {b}, mask {i}: uncompressed (list) counts; only compressed RLE strings "
+                                 "(bytes or str) are taken")
+            r = b * R + i
+            off[r], lens[r] = total, len(c)
+            chunks.append(np.frombuffer(bytes(c), np.uint8))
+            total += len(c)
+        off[b * R + len(dicts):(b + 1) * R] = total
+    chars = np.concatenate(chunks) if chunks else np.zeros(0, np.uint8)
+    return MaskRLE(torch.from_numpy(chars.copy()), torch.from_numpy(off), torch.from_numpy(lens), torch.from_numpy(hw),
+                   int(height), int(width))
+
+
+def _unpack_rle_into(rle, packed, prev_rects, meta, bad, n_img, n, stream):
+    """cim_mask_unpack_rle_tiled_meta_sparse of a device MaskRLE into packed [n_img * n, words] (sparse update against
+    prev_rects), metadata into meta, the malformed-string count into bad (int32 [1])."""
+    words = rle.height * rle.width // 32
+    rc = _lib.lib().cim_mask_unpack_rle_tiled_meta_sparse(
+        _lib.ptr(rle.chars), rle.chars.numel(), _lib.ptr(rle.off), _lib.ptr(rle.len), _lib.ptr(rle.hw),
+        _lib.ptr(packed), _lib.ptr(prev_rects), _lib.ptr(meta), meta.numel(), n_img, n, rle.height, rle.width, words,
+        _lib.ptr(bad), stream)
+    _lib.check(rc, "cim_mask_unpack_rle_tiled_meta_sparse")
+
+
+def unpack_rle(rle, out=None, meta=None):
+    """MaskRLE on the device -> tiled bit masks [n_img, R, H*W/32] int32 (tagged kb_per_row = W // 16), or (masks,
+    metadata) when meta is True or a uint8 tensor to fill (mask_meta's format, tied to those masks).  out: a buffer to
+    overwrite.  Needs H % 8 == 0 and W % 16 == 0.  A malformed string raises ValueError with their number (a host
+    synchronisation); its row would be all zero."""
+    _lib.require_cuda(rle.chars, "rle.chars", torch.uint8)
+    _lib.require_cuda(rle.off, "rle.off", torch.int64)
+    _lib.require_cuda(rle.len, "rle.len", torch.int32)
+    _lib.require_cuda(rle.hw, "rle.hw", torch.int32)
+    if not tiled_ok(rle.height, rle.width):
+        raise ValueError("unpack_rle writes the tiled layout: it needs height % 8 == 0 and width % 16 == 0")
+    n_img = rle.hw.shape[0]
+    rows = rle.off.numel()
+    if rle.hw.shape != (n_img, 2) or rle.len.numel() != rows or (n_img and rows % n_img):
+        raise ValueError(f"rle.hw must be [n_img, 2] and rle.off / rle.len [n_img * R], got {tuple(rle.hw.shape)}, "
+                         f"{rows} and {rle.len.numel()}")
+    n = rows // n_img if n_img else 0
+    words = rle.height * rle.width // 32
+    dev = rle.chars.device
+    if out is None:
+        out = torch.empty((n_img, n, words), dtype=torch.int32, device=dev)
+    if out.shape != (n_img, n, words) or out.dtype != torch.int32 or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous int32 [{n_img}, {n}, {words}] tensor")
+    want_meta = meta is not None and meta is not False
+    L = _lib.lib()
+    with torch.cuda.device(dev):
+        out.zero_()
+        prev = torch.zeros((max(rows, 1), 4), dtype=torch.int32, device=dev)
+        nbytes = L.cim_mask_meta_bytes(n_img, n, words)
+        if meta is True or not want_meta:
+            meta = torch.empty(max(nbytes, 256), dtype=torch.uint8, device=dev)
+        bad = torch.zeros(1, dtype=torch.int32, device=dev)
+        _unpack_rle_into(rle, out, prev, meta, bad, n_img, n, _lib.stream_ptr(dev))
+    n_bad = int(bad.item())
+    if n_bad:
+        raise ValueError(f"{n_bad} malformed RLE string(s): those rows are empty")
+    _tag(out, rle.width // 16)
+    return (out, meta) if want_meta else out
+
+
 def tiled_ok(height, width):
     """The 8 x 16 patch pixel order (cim_mask_pack_tiled) needs whole patches."""
     return height % 8 == 0 and width % 16 == 0

@@ -444,14 +444,21 @@ class CIMHeadStep:
         self.ustream.commit()
 
     # -------------------------------------------------------------------------------------
-    def alloc_host_io(self, mask_hw=None, crop_capacity_words=0, prefetch_depth=1, ragged=False, compact=False):
+    def alloc_host_io(self, mask_hw=None, crop_capacity_words=0, prefetch_depth=1, ragged=False, compact=False,
+                      rle_capacity_bytes=0):
         """Pinned host buffers of the end-to-end call: inputs that originate on the host in the
         reference's pipeline (rois, labels: lib/roi_data/minibatch.py:45-61; proposal masks:
         the COB .mat files of tools/pre) and the step's results.  Device-side input buffers are
         DOUBLE buffered and filled on a separate copy stream, so the host->device copy of step
         i+1 overlaps the kernels of step i (what a prefetching data loader does).
-        prefetch_depth = 2 (crops only): the host->device copy runs TWO steps ahead, into a third set of (small) crop
-        buffers on its own stream; the copy into the step's input buffer is then a device-to-device copy at the start
+        rle_capacity_bytes > 0: the masks arrive as COCO compressed RLE strings instead (mask_ops.MaskRLE, set_host_rle:
+        ~11x fewer bytes than the crops for COB-like proposals at 512 x 512), decoded on the device by
+        cim_mask_unpack_rle_tiled_meta_sparse into the same buffer; it excludes crop_capacity_words and needs the tiled
+        layout.  A malformed string gives an empty mask, and the step's results raise ValueError when they are
+        collected: at the end of the run_host() call that ran the step, or with lag_results one call later (or in
+        flush_results()), after that call's step has been enqueued.
+        prefetch_depth = 2 (crops or RLE only): the host->device copy runs TWO steps ahead, into a third set of (small)
+        wire buffers on its own stream; the copy into the step's input buffer is then a device-to-device copy at the start
         of the previous step, so the crop unpack can always run in that step's idle mining phase -- with eight ranks
         copying at once a rank's 60 MB take 2.5 ms instead of 1.3 (tools/h2d_bw.py) and the unpack used to slip behind
         the RoIAlign backward.  What run_host() finds in the pinned buffers at call t is then the input of step t + 2
@@ -464,8 +471,12 @@ class CIMHeadStep:
         in its first N rows and only those are copied; each staged step keeps its own host counts and N, and run_host()
         runs it with them (next_step_rows() tells how many rows its seg_x / grad_out need).  The masks stay padded."""
         k, n_img, R, C1 = self.K, self.n_img, self.R, self.C + 1
-        if prefetch_depth not in (1, 2) or (prefetch_depth == 2 and not crop_capacity_words):
-            raise ValueError("prefetch_depth must be 1, or 2 with crop_capacity_words > 0")
+        if crop_capacity_words and rle_capacity_bytes:
+            raise ValueError("the masks arrive as crops or as RLE strings, not both")
+        if rle_capacity_bytes and not self.kb_per_row:
+            raise ValueError("the RLE wire needs the tiled mask layout (mask_kb_per_row = W // 16)")
+        if prefetch_depth not in (1, 2) or (prefetch_depth == 2 and not (crop_capacity_words or rle_capacity_bytes)):
+            raise ValueError("prefetch_depth must be 1, or 2 with crop_capacity_words > 0 or rle_capacity_bytes > 0")
         self.prefetch_depth = prefetch_depth
         pin = lambda shape, dt: torch.empty(shape, dtype=dt).pin_memory()
         self.hi_rois = pin((n_img * R, 5), torch.float32)
@@ -478,6 +489,7 @@ class CIMHeadStep:
         # masks arrive either as full bit masks (hi_masks) or, with crop_capacity_words > 0, as
         # bounding-box crops (mask_ops.MaskCrops: ~8x fewer bytes over PCIe) that the device unpacks
         self.crop_cap = int(crop_capacity_words)
+        self.rle_cap = int(rle_capacity_bytes)
         self.mask_hw = mask_hw
         if self.crop_cap:
             self.hi_masks = None
@@ -485,6 +497,13 @@ class CIMHeadStep:
             self.hi_crop_meta = pin((n_img * R, 4), torch.int32)
             self.hi_crop_off = pin((n_img * R,), torch.int64)
             self.n_crop_words = 0
+        elif self.rle_cap:
+            self.hi_masks = None
+            self.hi_rle_chars = pin((self.rle_cap,), torch.uint8)
+            self.hi_rle_off = pin((n_img * R,), torch.int64)
+            self.hi_rle_len = pin((n_img * R,), torch.int32).zero_()
+            self.hi_rle_hw = pin((n_img, 2), torch.int32)
+            self.n_rle_chars = 0
         else:
             self.hi_masks = pin((n_img, R, self.words), torch.int32)
         # what the host reads back every step: with the loss block in the step (head_grads) the step's result
@@ -500,11 +519,14 @@ class CIMHeadStep:
             self.ho_weights = pin((k, n_img, R), torch.float32)
             results = (self.ho_labels, self.ho_iou, self.ho_weights, self.ho_valid)
         self.ho_checksum = pin((2,), torch.float32)
+        if self.rle_cap:
+            self.ho_bad = pin((1,), torch.int32)              # malformed strings among the step's masks
+            results = results + (self.ho_bad,)
         with torch.cuda.device(self.dev):
             dv = lambda shape, dt: torch.empty(shape, dtype=dt, device=self.dev)
-            # masks: ZERO-filled when they are produced from crops -- the fused unpack is a sparse update that only
-            # touches the rectangles of the crop a row held before (prev_rects) and of the new one
-            mk = torch.zeros if self.crop_cap else torch.empty
+            # masks: ZERO-filled when they are produced from crops or RLE -- the fused unpack is a sparse update that
+            # only touches the rectangles of the mask a row held before (prev_rects) and of the new one
+            mk = torch.zeros if self.crop_cap or self.rle_cap else torch.empty
             self.di = [dict(rois=dv((n_img * R, 5), torch.float32), labels=dv((n_img, self.C), torch.float32),
                             masks=mk((n_img, R, self.words), dtype=torch.int32, device=self.dev),
                             ready=torch.cuda.Event(), free=torch.cuda.Event()) for _ in range(2)]
@@ -516,6 +538,13 @@ class CIMHeadStep:
                     buf.update(crop_words=dv((self.crop_cap,), torch.int32), crop_meta=dv((n_img * R, 4), torch.int32),
                                crop_off=dv((n_img * R,), torch.int64),
                                prev_rects=torch.zeros((n_img * R, 4), dtype=torch.int32, device=self.dev))
+            if self.rle_cap:
+                for buf in self.di:
+                    buf.update(rle_chars=dv((self.rle_cap,), torch.uint8), rle_off=dv((n_img * R,), torch.int64),
+                               rle_len=dv((n_img * R,), torch.int32), rle_hw=dv((n_img, 2), torch.int32),
+                               prev_rects=torch.zeros((n_img * R, 4), dtype=torch.int32, device=self.dev),
+                               bad=dv((1,), torch.int32))
+                self.d_bad = torch.zeros((1,), dtype=torch.int32, device=self.dev)
             # mask metadata (areas, K-block bitmaps) produced on the copy stream right after the masks land
             self.use_meta = self.words % 4 == 0
             if self.use_meta:
@@ -525,16 +554,20 @@ class CIMHeadStep:
             self.copy_stream = torch.cuda.Stream(device=self.dev)
             if prefetch_depth == 2:
                 self.pre = dict(rois=dv((n_img * R, 5), torch.float32), labels=dv((n_img, self.C), torch.float32),
-                                crop_words=dv((self.crop_cap,), torch.int32), crop_meta=dv((n_img * R, 4), torch.int32),
-                                crop_off=dv((n_img * R,), torch.int64), n_words=0, valid=False,
-                                filled=torch.cuda.Event())
+                                n_words=0, valid=False, filled=torch.cuda.Event())
+                if self.crop_cap:
+                    self.pre.update(crop_words=dv((self.crop_cap,), torch.int32),
+                                    crop_meta=dv((n_img * R, 4), torch.int32), crop_off=dv((n_img * R,), torch.int64))
+                else:
+                    self.pre.update(rle_chars=dv((self.rle_cap,), torch.uint8), rle_off=dv((n_img * R,), torch.int64),
+                                    rle_len=dv((n_img * R,), torch.int32), rle_hw=dv((n_img, 2), torch.int32))
                 if self.ragged:
                     self.pre["n_props"] = dv((n_img,), torch.int32)
                 self.copy_stream2 = torch.cuda.Stream(device=self.dev)
         self.h2d_bytes = sum(t.numel() * t.element_size() for t in (self.hi_rois, self.hi_labels))
         if self.ragged:
             self.h2d_bytes += self.hi_n_props.numel() * 4
-        if not self.crop_cap:
+        if self.hi_masks is not None:
             self.h2d_bytes += self.hi_masks.numel() * 4
         self.d2h_bytes = sum(t.numel() * t.element_size() for t in results + (self.ho_checksum,))
         # the sampling hop: pseudo-GT counts down, one double per pseudo GT up (self.last_uniform_bytes, set by run())
@@ -549,12 +582,13 @@ class CIMHeadStep:
         self.h2d_ev = torch.cuda.Event()
         self._h2d_pending = False
         self._pending = False
+        self._bad_rle = 0
         self.results_host = None
 
     def wait_inputs_consumed(self):
         """Block until the last stage_host_inputs() has finished READING the pinned input buffers (hi_rois, hi_labels,
-        hi_masks / hi_crop_*, hi_n_props).  The copies are asynchronous: refill those buffers for the following step only after
-        this returns (set_host_crops() calls it itself)."""
+        hi_masks / hi_crop_* / hi_rle_*, hi_n_props).  The copies are asynchronous: refill those buffers for the following
+        step only after this returns (set_host_crops() and set_host_rle() call it themselves)."""
         if getattr(self, "_h2d_pending", False):
             self.h2d_ev.synchronize()
             self._h2d_pending = False
@@ -570,6 +604,25 @@ class CIMHeadStep:
         self.hi_crop_off.copy_(crops.off)
         self.n_crop_words = n
         self.mask_hw = (crops.height, crops.width)
+
+    def set_host_rle(self, rle):
+        """Copy a MaskRLE (CPU; mask_ops.batch_rle_host) of the n_img * R proposal masks into the pinned input buffers
+        (alloc_host_io(rle_capacity_bytes=...)).  Its canvas must be the step's: height * width == 32 * mask_words and
+        width == 16 * mask_kb_per_row."""
+        self.wait_inputs_consumed()
+        n, rows = rle.chars.numel(), self.n_img * self.R
+        if n > self.rle_cap:
+            raise ValueError(f"{n} RLE characters exceed the capacity {self.rle_cap}")
+        if rle.off.numel() != rows or rle.len.numel() != rows or tuple(rle.hw.shape) != (self.n_img, 2):
+            raise ValueError(f"the RLE batch must have {rows} rows and {self.n_img} image sizes")
+        if rle.height * rle.width != 32 * self.words or rle.width != 16 * self.kb_per_row:
+            raise ValueError(f"the RLE canvas {rle.height} x {rle.width} is not the step's tiled mask canvas")
+        self.hi_rle_chars[:n].copy_(rle.chars)
+        self.hi_rle_off.copy_(rle.off)
+        self.hi_rle_len.copy_(rle.len)
+        self.hi_rle_hw.copy_(rle.hw)
+        self.n_rle_chars = n
+        self.mask_hw = (rle.height, rle.width)
 
     def stage_host_inputs(self, defer_kernels=False, direct=False):
         """Enqueue the host->device copy of the CURRENT contents of hi_rois / hi_labels / hi_masks
@@ -591,7 +644,16 @@ class CIMHeadStep:
             with torch.cuda.stream(self.copy_stream):
                 if after is not None:
                     self.copy_stream.wait_event(after)
-                if self.crop_cap:
+                if self.rle_cap:
+                    # RLE strings -> tiled bit masks + their metadata, the same sparse update as the crops'
+                    rc = self.L.cim_mask_unpack_rle_tiled_meta_sparse(
+                        _lib.ptr(buf["rle_chars"]), buf["n_chars"], _lib.ptr(buf["rle_off"]), _lib.ptr(buf["rle_len"]),
+                        _lib.ptr(buf["rle_hw"]), _lib.ptr(buf["masks"]), _lib.ptr(buf["prev_rects"]),
+                        _lib.ptr(buf["meta"]), buf["meta"].numel(), self.n_img, self.R, self.mask_hw[0],
+                        self.mask_hw[1], self.words, _lib.ptr(buf["bad"]), C.c_void_p(self.copy_stream.cuda_stream))
+                    _lib.check(rc, "cim_mask_unpack_rle_tiled_meta_sparse")
+                    buf["meta_done"] = True
+                elif self.crop_cap:
                     fused = bool(self.kb_per_row) and self.use_meta and \
                         self.words * 32 == self.mask_hw[0] * self.mask_hw[1]
                     if fused:
@@ -619,7 +681,8 @@ class CIMHeadStep:
                 buf["ready"].record(self.copy_stream)
 
         def h2d(dst, stream):
-            """pinned input buffers -> dst (a device input buffer or the pre-stage); returns the crop word count"""
+            """pinned input buffers -> dst (a device input buffer or the pre-stage); returns the crop word / RLE
+            character count"""
             if self.compact:
                 dst["counts"] = self.hi_n_props.numpy().copy()        # this step's host counts travel with it
                 dst["N"] = int(dst["counts"].sum())
@@ -636,6 +699,13 @@ class CIMHeadStep:
                 dst["crop_meta"].copy_(self.hi_crop_meta, non_blocking=True)
                 dst["crop_off"].copy_(self.hi_crop_off, non_blocking=True)
                 self.last_mask_h2d_bytes = n * 4 + self.hi_crop_meta.numel() * 4 + self.hi_crop_off.numel() * 8
+            elif self.rle_cap:
+                n = self.n_rle_chars
+                dst["rle_chars"][:n].copy_(self.hi_rle_chars[:n], non_blocking=True)
+                for key in ("rle_off", "rle_len", "rle_hw"):
+                    dst[key].copy_(getattr(self, "hi_" + key), non_blocking=True)
+                self.last_mask_h2d_bytes = n + sum(getattr(self, "hi_" + k).numel() * getattr(self, "hi_" + k).element_size()
+                                                   for k in ("rle_off", "rle_len", "rle_hw"))
             else:
                 dst["masks"].copy_(self.hi_masks, non_blocking=True)
                 dst["meta_done"] = False
@@ -653,13 +723,16 @@ class CIMHeadStep:
                 # the input of this buffer's step arrived a step ago: device-to-device
                 self.copy_stream.wait_event(pre["filled"])
                 n = pre["n_words"]
-                for key in ("rois", "labels", "crop_meta", "crop_off") + (("n_props",) if self.ragged else ()):
+                wire = ("crop_meta", "crop_off") if self.crop_cap else ("rle_off", "rle_len", "rle_hw")
+                for key in ("rois", "labels") + wire + (("n_props",) if self.ragged else ()):
                     buf[key].copy_(pre[key], non_blocking=True)
                 if self.compact:
                     buf["counts"], buf["N"] = pre["counts"], pre["N"]
-                buf["crop_words"][:n].copy_(pre["crop_words"][:n], non_blocking=True)
+                big = "crop_words" if self.crop_cap else "rle_chars"
+                buf[big][:n].copy_(pre[big][:n], non_blocking=True)
+                buf["n_chars"] = n
             else:
-                h2d(buf, self.copy_stream)
+                buf["n_chars"] = h2d(buf, self.copy_stream)
         if pre is not None:
             # ... and the pinned buffers (the input of the step after that one) go to the pre-stage on their own stream,
             # so that a slow copy never sits in front of the unpack kernel
@@ -684,11 +757,20 @@ class CIMHeadStep:
         self.results_host = {"valid": self.ho_valid.numpy().copy(), "checksum": self.ho_checksum.numpy().copy()}
         if self.head_grads:
             self.results_host["losses"] = self.ho_losses.numpy().copy()
+        if self.rle_cap:
+            self._bad_rle = self.results_host["bad_rle"] = int(self.ho_bad[0])
         self._pending = False
+
+    def _raise_bad_rle(self):
+        """The RLE wire: raise for the malformed strings of the step whose results were collected last."""
+        n, self._bad_rle = self._bad_rle, 0
+        if n:
+            raise ValueError(f"{n} malformed RLE string(s) among the step's proposal masks: those masks were empty")
 
     def flush_results(self):
         """With lag_results: wait for the results of the last run_host() call (self.results_host)."""
         self._collect_results()
+        self._raise_bad_rle()
         return self.results_host
 
     def next_step_rows(self):
@@ -729,6 +811,8 @@ class CIMHeadStep:
                  n_props=buf["counts"] if compact else buf.get("n_props"), feat_hw=feat_hw, compact=compact,
                  mid_hook=lambda: ((finish_stage(self.ev_premine) if finish_stage else None),
                                    (self._collect_results() if lag_results else None)))
+        if self.rle_cap:
+            self.d_bad.copy_(buf["bad"])                       # read before the buffer's next unpack overwrites it
         buf["free"].record(cur_stream)
         # two sparse checksums of the RoIAlign outputs ride along with the losses (a few hundred elements each, summed
         # straight into the result buffer).  roi_out is the first thing the next step overwrites, so its checksum stays on
@@ -749,6 +833,8 @@ class CIMHeadStep:
                 self.ho_weights.copy_(self.loss_weights, non_blocking=True)
             self.ho_valid.copy_(self.valid, non_blocking=True)
             self.ho_checksum.copy_(self.d_checksum, non_blocking=True)
+            if self.rle_cap:
+                self.ho_bad.copy_(self.d_bad, non_blocking=True)
             self.res_ev.record(self.res_stream)
         self._res_guard = True
         self._pending = True
@@ -758,4 +844,5 @@ class CIMHeadStep:
             self._slot ^= 1
         else:
             self._staged = False
+        self._raise_bad_rle()
         return self

@@ -286,6 +286,22 @@ int cim_mask_unpack_crops_tiled_meta(const uint32_t *crop_words, const int32_t *
 int cim_mask_unpack_crops_tiled_meta_sparse(const uint32_t *crop_words, const int32_t *crop_meta, const int64_t *crop_off,
                                             uint32_t *packed, int32_t *prev_rects, void *meta, size_t meta_bytes, int n_img,
                                             int n, int H, int W, int64_t words, cim_stream_t stream);
+/* The same sparse update fed with COCO compressed RLE strings instead of crops (pycocotools' rleFrString + rleDecode):
+ *   row m of the n_img * n rows has the string chars[off[m], off[m] + len[m]) (off int64, len int32); len 0 = a row of
+ *   zeros (padding rows).  mask_hw [n_img][2] int32 (may be NULL = the canvas): image b's native (h, w), clamped to
+ *   [1, H] x [1, W]; its masks sit at the top left of the canvas, string pixel p = (x, y) = (p / h, p % h).
+ *   A string is malformed when a character lies outside [48, 111], its last character still has the continuation bit
+ *   0x20, a count (after the delta decoding and rleFrString's (uint) cast) lies outside [0, h*w], the counts do not sum
+ *   to h*w, or off + len > n_chars (or either is negative).  Its row becomes a row of zeros with an empty rectangle and
+ *   empty metadata, and is counted in *bad (int32, zeroed by the call; may be NULL).  Nothing outside a row is written.
+ *   Output bit for bit what cim_mask_unpack_crops_tiled_meta_sparse writes for the crops of the same masks; prev_rects
+ *   = the tight box of the ones rounded out to 32-pixel words in x, the crops' units, whichever wire filled the row.
+ *   Conditions as there (words * 32 == H * W, H % 8 == 0, W % 16 == 0), and H * W <= 2^31 - 1, W <= 8192,
+ *   ceil(words / 128) <= 2048 (CIM_ERR_SHAPE otherwise).  One CTA per row, no global atomics on the masks, deterministic. */
+int cim_mask_unpack_rle_tiled_meta_sparse(const uint8_t *chars, int64_t n_chars, const int64_t *off, const int32_t *len,
+                                          const int32_t *mask_hw, uint32_t *packed, int32_t *prev_rects, void *meta,
+                                          size_t meta_bytes, int n_img, int n, int H, int W, int64_t words,
+                                          int32_t *bad, cim_stream_t stream);
 int cim_mask_meta(const uint32_t *packed, int n_img, int n, int64_t words, int kb_per_row, void *meta,
                   size_t meta_bytes, cim_stream_t stream);
 int cim_mask_overlap_meta(const uint32_t *packed, const void *meta, int n_img, int n, int64_t words, int kb_per_row,
